@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: mesh-nodes/s through the deformer forward+backward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): batched 2D 30x30 meshes, batch 256 per GPU, 4 Euler layers,
 hidden 8, fp32, L1 mesh loss -- one STEP is one full training pass over one batch: feature
@@ -116,7 +116,13 @@ class ClockSampler:
 
     def stop(self):
         if self.proc is not None:
+            # reap the sampler: bench.py must not leave an nvidia-smi process (or its zombie) behind
             self.proc.terminate()
+            try:
+                self.proc.wait(timeout=5)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
         sm, smax, reasons = [], [], set()
         names = ("hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap")
         lo = (self.t0 or 0) - 0.05
@@ -451,7 +457,13 @@ def main():
                          "through other ranks' GPUs (NVLink); proposals are timed on the real loop and the direct loop "
                          "stays unless one of them is at least 3%% faster (DESIGN section 15)")
     ap.add_argument("--skip-configs", action="store_true", help="do not time the other BASELINE configs (cfg 1, 3, 4, 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy: loss, x_phys (the deformed "
+                         "mesh of its batch), params and grads (the flat parameter vector after its Adam update and the "
+                         "gradient it applied); inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA training step (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -566,6 +578,13 @@ def main():
     barrier()
     clocks.mark(False)
     trainer.check_peer()
+    # what the last timed step handed back, written before anything below runs more steps on the same buffers
+    if args.dump_outputs and rank == 0:
+        last = trainer.slots[plan[-1][-1] if graph_mode else (K - 1) % R]
+        outputs = {"loss": last.loss, "x_phys": last.x_phys, "params": trainer.flat, "grads": trainer.gflat}
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.detach().cpu().numpy())
     ms_stream_events = ev0.elapsed_time(ev1)
     ms_total = trainer.epoch_elapsed_ms(plan[0]) if in_graph_events else ms_stream_events
     eager_launches = lib.gad_launch_count() - launches0
