@@ -36,7 +36,10 @@ namespace {
 using namespace fem2d;
 
 constexpr int FEM2D_THREADS = 512;
-constexpr int MAX_HITS = 12;
+// An evaluation point on a vertex lies in every cell of the vertex's star, so the point pass must keep D hits: the
+// launch check bounds D by MAX_HITS.  f2_load<1> packs 2 bits per star cell into one 32-bit mask: D <= 16.
+constexpr int MAX_HITS = 16;
+static_assert(2 * MAX_HITS <= 32, "f2_load<1>: the star-cell mask has 2 bits per cell in 32 bits");
 constexpr int MAX_GAUSS = 16;
 constexpr int MAX_ROWS_PER_THREAD = 8;     // CG keeps r / x / Ap of its rows in registers: N <= 8 * 512 (template R)
 __host__ __device__ inline int f2_rows_per_thread(int N) {
@@ -753,8 +756,8 @@ int f2_launch(const F2Args& a, int B, bool backward, cudaStream_t st) {
     const size_t bytes = f2_smem_bytes(a.N, a.T, a.D);
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "fem2d: a mesh of %d nodes / %d cells needs %zu B of shared memory", a.N, a.T,
                   bytes);
-    GAD_CHECK_ARG(a.G <= MAX_GAUSS && a.D <= 16, "fem2d: at most %d Gaussians and 16 cells per node (got %d, %d)", MAX_GAUSS,
-                  a.G, a.D);
+    GAD_CHECK_ARG(a.G <= MAX_GAUSS && a.D <= MAX_HITS, "fem2d: at most %d Gaussians and %d cells per node (got %d, %d)",
+                  MAX_GAUSS, MAX_HITS, a.G, a.D);
     GAD_CHECK_ARG(a.N <= MAX_ROWS_PER_THREAD * FEM2D_THREADS && a.N <= 65535 && a.T <= 65535,
                   "fem2d: %d nodes / %d cells exceed the kernel's limits (%d nodes, 16-bit indices)", a.N, a.T,
                   MAX_ROWS_PER_THREAD * FEM2D_THREADS);
