@@ -92,6 +92,8 @@ SIGNATURES = {
     "gad_deform_bwd_ell": (_i, [_p, _p, _i64, _p, _i, _i, _i, _p, _p, _i, _i, _p, _p, _i, _p, _i, _p, _p, _p, _p, _sz, _p]),
     "gad_deform_bwd_ell_rk4": (_i, [_p, _p, _i64, _p, _i, _i, _i, _p, _p, _i, _i, _p, _p, _i, _p, _i, _p, _p, _p, _sz, _p]),
     "gad_ell_rk4_bwd_supported": (_i, [_i, _i, _i]),
+    "gad_train_step_ell_rk4": (_i, [C.POINTER(TrainDesc), _p]),
+    "gad_ell_rk4_train_supported": (_i, [_i, _i, _i]),
     "gad_deform_train_ell": (_i, [_p, _p, _i64, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _i, _i,
                                   _f, _f, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "gad_train_step_ell": (_i, [C.POINTER(TrainDesc), _p]),

@@ -434,32 +434,31 @@ extern "C" int gad_deform_train_ell(const void* ell_in, const void* ell_out, int
     return reduce_partials(CE, T, Lw, L, ws, gMu, g_tau, loss_scale, loss, st);
 }
 
-extern "C" int gad_train_step_ell(const gad_train_desc* d, void* stream) {
-    GAD_CHECK_ARG(d, "gad_train_step_ell: null descriptor");
+// One training step of gad_train_step_ell / gad_train_step_ell_rk4 (`who` names the entry point in errors).
+static int train_step(const gad_train_desc* d, int method, const char* who, void* stream) {
+    GAD_CHECK_ARG(d, "%s: null descriptor", who);
     GAD_CHECK_ARG(d->ell_in && d->ell_out && d->x_comp && d->target && d->Mu && d->tau && d->states &&
                       d->gMu && d->loss && d->workspace && d->counter,
-                  "gad_train_step_ell: null pointer");
-    {
-        const int32_t* tile_ptr = d->tile_ptr;
-        const int64_t N = d->N;
-        const int T = d->T, max_tile_nodes = d->max_tile_nodes;
-        GAD_UNIFORM_TILES_OK("gad_train_step_ell");
-    }
+                  "%s: null pointer", who);
+    GAD_CHECK_ARG(d->tile_ptr || (d->max_tile_nodes > 0 &&
+                                  (int64_t)d->T == (d->N + d->max_tile_nodes - 1) / d->max_tile_nodes),
+                  "%s: tile_ptr == NULL means T = ceil(N / max_tile_nodes) equal tiles (N=%lld T=%d tile=%d)", who,
+                  (long long)d->N, d->T, d->max_tile_nodes);
     GAD_CHECK_ARG(d->N > 0 && d->T > 0 && d->L > 0 && d->dim >= 1 && d->dim <= d->CE && (d->Lw == 1 || d->Lw == d->L),
-                  "gad_train_step_ell: N=%lld T=%d L=%d dim=%d CE=%d Lw=%d", (long long)d->N, d->T, d->L, d->dim, d->CE,
-                  d->Lw);
-    GAD_CHECK_ARG(d->dim + (d->f ? 1 : 0) + (d->uu ? 1 : 0) <= d->CE, "gad_train_step_ell: input features exceed CE=%d",
-                  d->CE);
-    GAD_CHECK_ARG(d->loss_kind == 0 || d->loss_kind == 1, "gad_train_step_ell: unknown loss kind %d", d->loss_kind);
-    GAD_CHECK_ARG(d->tail == 1 || d->tail == 2, "gad_train_step_ell: tail must be 1 or 2 (got %d)", d->tail);
+                  "%s: N=%lld T=%d L=%d dim=%d CE=%d Lw=%d", who, (long long)d->N, d->T, d->L, d->dim, d->CE, d->Lw);
+    GAD_CHECK_ARG(d->dim + (d->f ? 1 : 0) + (d->uu ? 1 : 0) <= d->CE, "%s: input features exceed CE=%d", who, d->CE);
+    GAD_CHECK_ARG(d->loss_kind == 0 || d->loss_kind == 1, "%s: unknown loss kind %d", who, d->loss_kind);
+    GAD_CHECK_ARG(d->tail == 1 || d->tail == 2, "%s: tail must be 1 or 2 (got %d)", who, d->tail);
     GAD_CHECK_ARG(d->Wq && d->bq && d->Wk && d->gWq && d->gbq && d->gWk && d->gbk && d->C > 0,
-                  "gad_train_step_ell: the tail needs the Linear parameters and their gradient buffers");
+                  "%s: the tail needs the Linear parameters and their gradient buffers", who);
     GAD_CHECK_ARG(d->tail < 2 || (d->params && d->grads && d->exp_avg && d->exp_avg_sq && d->step && d->n_params > 0),
-                  "gad_train_step_ell: tail == 2 needs the flat parameter vector and the Adam state");
-    GAD_CHECK_ARG(d->workspace_bytes >= ws_floats(d->CE, d->T, d->L) * sizeof(float),
-                  "gad_train_step_ell: workspace too small");
+                  "%s: tail == 2 needs the flat parameter vector and the Adam state", who);
+    GAD_CHECK_ARG(d->workspace_bytes >= ws_floats(d->CE, d->T, d->L) * sizeof(float), "%s: workspace too small", who);
+    GAD_CHECK_ARG(method == GAD_METHOD_EULER || d->g_tau == nullptr,
+                  "%s: the step sizes get no gradient through RK4 (g_tau must be NULL)", who);
+    const int kind = method == GAD_METHOD_RK4 ? KIND_TRAIN_RK4 : KIND_BWD;
     Plan p;
-    int rc = make_plan(d->CE, KIND_BWD, d->max_tile_nodes, d->max_deg, &p);
+    int rc = make_plan(d->CE, kind, d->max_tile_nodes, d->max_deg, &p);
     if (rc) return rc;
     const int NACC = d->CE * d->CE + d->CE + 1;
     float* ws = reinterpret_cast<float*>(d->workspace);
@@ -529,7 +528,7 @@ extern "C" int gad_train_step_ell(const gad_train_desc* d, void* stream) {
     // needs Wq / bq / Wk to be views of `params` (tail 2) and its scratch plan to fit the CTA.
     auto within = [](const float* q, const float* base, long long n) { return q >= base && q < base + n; };
     const long long np = d->tail >= 2 ? d->n_params : 0;
-    const Layout lay = make_layout(d->CE, KIND_BWD, d->max_tile_nodes, p.ells != 0, (p.threads + 31) / 32);
+    const Layout lay = make_layout(d->CE, kind, d->max_tile_nodes, p.ells != 0, (p.threads + 31) / 32);
     const TailPlan tplan = plan_tail(d->CE, d->Lw, d->L, d->C, a.tau_partials && a.g_tau, true, np, d->T, (p.threads + 31) / 32,
                                      lay.bar);
     bool fused_tail = tplan.ok;
@@ -545,16 +544,16 @@ extern "C" int gad_train_step_ell(const gad_train_desc* d, void* stream) {
     const bool exchange = d->world > 1 && d->peers;
     if (exchange) {
         GAD_CHECK_ARG(d->tail == 2 && d->peer_seq && d->rank >= 0 && d->rank < d->world && d->world <= GAD_MAX_PEERS,
-                      "gad_train_step_ell: the peer exchange needs tail == 2, a sequence counter and rank < world <= %d",
+                      "%s: the peer exchange needs tail == 2, a sequence counter and rank < world <= %d", who,
                       GAD_MAX_PEERS);
-        GAD_CHECK_ARG(fused_tail, "gad_train_step_ell: the peer exchange needs the in-kernel tail (flat parameter views, "
-                                  "scratch of %u B)", lay.bar);
+        GAD_CHECK_ARG(fused_tail, "%s: the peer exchange needs the in-kernel tail (flat parameter views, scratch of %u B)",
+                      who, lay.bar);
     }
-    if (fused_tail) return dispatch(d->CE, p, 2, a, GAD_METHOD_EULER, st);
+    if (fused_tail) return dispatch(d->CE, p, 2, a, method, st);
     // generic path: the same step as separate launches
     a.tail = 0;
     a.pdl = 0;
-    if ((rc = dispatch(d->CE, p, 2, a, GAD_METHOD_EULER, st))) return rc;
+    if ((rc = dispatch(d->CE, p, 2, a, method, st))) return rc;
     if ((rc = reduce_partials(d->CE, d->T, d->Lw, d->L, ws, d->gMu, d->g_tau, d->loss_scale, d->loss, st))) return rc;
     if ((rc = gad_weight_grads(d->Wq, d->bq, d->Wk, d->gMu, d->Lw, d->C, d->CE, d->inv_temp, d->gWq, d->gbq, d->gWk, d->gbk,
                                stream)))
@@ -566,4 +565,19 @@ extern "C" int gad_train_step_ell(const gad_train_desc* d, void* stream) {
         if ((rc = gad_prepare_weights(d->Wq, d->bq, d->Wk, d->Lw, d->C, d->CE, d->inv_temp, d->Mu, stream))) return rc;
     }
     return GAD_OK;
+}
+
+extern "C" int gad_train_step_ell(const gad_train_desc* d, void* stream) {
+    return train_step(d, GAD_METHOD_EULER, "gad_train_step_ell", stream);
+}
+
+extern "C" int gad_train_step_ell_rk4(const gad_train_desc* d, void* stream) {
+    return train_step(d, GAD_METHOD_RK4, "gad_train_step_ell_rk4", stream);
+}
+
+extern "C" int gad_ell_rk4_train_supported(int CE, int max_tile_nodes, int max_deg) {
+    Plan p;
+    if (CE != 2 && CE != 4) return 0;
+    if (max_deg > ELL_SLOTS || max_tile_nodes <= 0 || (long long)max_tile_nodes * CE * 4 > 0x10000) return 0;
+    return make_plan(CE, KIND_TRAIN_RK4, max_tile_nodes, max_deg, &p) == GAD_OK ? 1 : 0;
 }

@@ -39,7 +39,8 @@ namespace ell {
 #define GAD_ELL_MINB 1
 #endif
 
-enum Kind { KIND_FWD = 0, KIND_FWD_RK4 = 1, KIND_BWD = 2, KIND_BWD_RK4 = 3 };
+// KIND_TRAIN_RK4: the rows of KIND_BWD_RK4, with the train tail's scratch rule of KIND_BWD.
+enum Kind { KIND_FWD = 0, KIND_FWD_RK4 = 1, KIND_BWD = 2, KIND_BWD_RK4 = 3, KIND_TRAIN_RK4 = 4 };
 
 constexpr size_t TAIL_SCRATCH_MIN = 24 * 1024;
 
@@ -63,9 +64,10 @@ __host__ __device__ inline Layout make_layout(int CE, int kind, int cap_nodes, b
         s.p = bump(rows);    // RK4: base state;   backward: p_i rows
         s.gs = bump(rows);   // RK4: accumulator;  backward: per-node gradient carry
     }
-    const bool bwd = (kind == KIND_BWD || kind == KIND_BWD_RK4);
+    const bool bwd = (kind == KIND_BWD || kind == KIND_BWD_RK4 || kind == KIND_TRAIN_RK4);
+    const bool rk4_rows = (kind == KIND_BWD_RK4 || kind == KIND_TRAIN_RK4);
     if (bwd) s.dl = bump((size_t)cap_nodes * 8);
-    if (kind == KIND_BWD_RK4) {
+    if (rk4_rows) {
         s.y2 = bump(rows);
         s.y3 = bump(rows);
         s.y4 = bump(rows);
@@ -78,7 +80,7 @@ __host__ __device__ inline Layout make_layout(int CE, int kind, int cap_nodes, b
     }
     s.mu = bump((size_t)(CE * CE + CE) * sizeof(float));
     if (bwd) s.red = bump((size_t)(CE * CE + CE + 1) * nwarps * sizeof(float));
-    if (kind == KIND_BWD && o < TAIL_SCRATCH_MIN) o = TAIL_SCRATCH_MIN;   // train tail: [0, bar) is its scratch
+    if ((kind == KIND_BWD || kind == KIND_TRAIN_RK4) && o < TAIL_SCRATCH_MIN) o = TAIL_SCRATCH_MIN;   // train tail: [0, bar) is its scratch
     s.bar = bump(16);
     s.total = (uint32_t)o;
     return s;
@@ -1152,13 +1154,18 @@ __device__ __forceinline__ void tail_finish(const Args& a, unsigned char* scratc
 // loss_type = mesh_loss): x_phys and its cotangent never leave the SM.  The layer states go to
 // `states` (L2-resident scratch) on the way up and are read back by the same thread on the way
 // down; ld.global.cg keeps those reads coherent.
-template <int CE, int W, bool ELLS>
+// METHOD == GAD_METHOD_RK4: classical RK4 steps (the forward of k_ell_fwd<..., GAD_METHOD_RK4>, same
+// expressions), the loss fused into stage 4 of the last step, then tile_backward_rk4.  The inputs are
+// staged into the Y2 rows (untouched until the backward recomputes the stages) and the target into DL;
+// the cotangent goes to the G rows, which tile_backward_rk4 reads as dL/dx^L.
+template <int CE, int W, bool ELLS, int METHOD>
 __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const Args a) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, nthr = blockDim.x;
-    const Layout lay = make_layout(CE, KIND_BWD, a.cap_nodes, ELLS, (nthr + 31) >> 5);
+    const Layout lay = make_layout(CE, METHOD == GAD_METHOD_RK4 ? KIND_TRAIN_RK4 : KIND_BWD, a.cap_nodes, ELLS,
+                                   (nthr + 31) >> 5);
     unsigned char* B0 = smem + lay.xa;
     unsigned char* B1 = smem + lay.xb;
     unsigned char* P = smem + lay.p;
@@ -1202,8 +1209,8 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
         const bool stage = a.dim <= 2 && (NT % 4 == 0) &&
                            ((reinterpret_cast<uintptr_t>(xc_g) | reinterpret_cast<uintptr_t>(tg_g) |
                              reinterpret_cast<uintptr_t>(f_g) | reinterpret_cast<uintptr_t>(uu_g)) & 15) == 0;
-        unsigned char* st_xc = P;
-        unsigned char* st_f = P + xc_bytes;
+        unsigned char* st_xc = (METHOD == GAD_METHOD_RK4) ? smem + lay.y2 : P;
+        unsigned char* st_f = st_xc + xc_bytes;
         unsigned char* st_uu = st_f + (a.f ? sc_bytes : 0u);
         const uint32_t tx = (ELLS ? 2u * (uint32_t)NT * 16u : 0u) +
                             (stage ? 2u * xc_bytes + (a.f ? sc_bytes : 0u) + (a.uu ? sc_bytes : 0u) : 0u);
@@ -1250,6 +1257,7 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
         EllView<ELLS> Ein{ELLS ? reinterpret_cast<const uint4*>(smem + lay.ein) : a.ell_in + e0};
         EllView<ELLS> Eout{ELLS ? reinterpret_cast<const uint4*>(smem + lay.eout) : a.ell_out + e0};
 
+        if constexpr (METHOD == GAD_METHOD_EULER) {
         // ---- forward (Euler), loss and cotangent fused into the last layer --------------------
         float loss_acc = 0.f;
         for (int l = 0; l < a.L; ++l) {
@@ -1315,6 +1323,87 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
         tr.mark();   // loss reduced
         tile_backward<CE, W, ELLS>(a, tile, n0, NT, Xc, Xn, P, DL, GS, Ein, Eout, Mu, red);
         tr.mark();   // backward + block reduction done
+        } else {
+        // ---- forward (RK4 steps), loss and cotangent fused into stage 4 of the last step ----------
+        unsigned char* XB = P;    // base state of the step
+        unsigned char* AC = GS;   // k-accumulator
+        unsigned char* G = smem + lay.g;
+        float loss_acc = 0.f;
+        for (int l = 0; l < a.L; ++l) {
+            if (a.Lw > 1 && l > 0) {
+                for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
+                __syncthreads();
+            }
+            const float h = __ldcg(a.tau + l);
+            const bool last = (l == a.L - 1);
+            float* st_out = last ? nullptr : a.states + (size_t)(l + 1) * state_stride;
+            const float cin[4] = {0.5f * h, 0.5f * h, h, 0.f};
+            const float wacc[4] = {1.f, 2.f, 2.f, 1.f};
+#pragma unroll
+            for (int s = 0; s < 4; ++s) {
+                for (int i = tid; i < NT; i += nthr) {
+                    const uint4 e = Ein.get(i);
+                    const Row<CE> y = lds_row<CE>(Xc, i * RB);
+                    if (l == 0 && s == 0) store_row<CE>(a.states, (int64_t)n0 + i, y);
+                    const Row<CE> k = ell_feval<CE, W>(Xc, e, y, Mu);
+                    Row<CE> base, acc, out;
+                    if (s == 0) {
+                        base = y;
+                        acc = k;
+                        sts_row<CE>(XB, i * RB, y);
+                    } else {
+                        base = lds_row<CE>(XB, i * RB);
+                        acc = lds_row<CE>(AC, i * RB);
+#pragma unroll
+                        for (int c = 0; c < CE; ++c) acc.v[c] = fmaf(wacc[s], k.v[c], acc.v[c]);
+                    }
+                    if (s < 3) {
+                        sts_row<CE>(AC, i * RB, acc);
+#pragma unroll
+                        for (int c = 0; c < CE; ++c) out.v[c] = fmaf(cin[s], k.v[c], base.v[c]);
+                        sts_row<CE>(Xn, i * RB, out);
+                    } else {
+#pragma unroll
+                        for (int c = 0; c < CE; ++c) out.v[c] = fmaf(h * (1.0f / 6.0f), acc.v[c], base.v[c]);
+                        if (!last) {
+                            sts_row<CE>(Xn, i * RB, out);
+                            store_row<CE>(st_out, (int64_t)n0 + i, out);
+                        } else {
+                            const int64_t gi = (int64_t)n0 + i;
+                            if (a.x_phys) store_dims<CE>(a.x_phys, gi, a.dim, out);
+                            const Row<CE> tg = stage ? load_dims<CE>(reinterpret_cast<const float*>(DL), i, a.dim)
+                                                     : load_dims<CE>(a.target, gi, a.dim);
+                            Row<CE> g;
+#pragma unroll
+                            for (int c = 0; c < CE; ++c) {
+                                const float d = (c < a.dim) ? out.v[c] - tg.v[c] : 0.f;
+                                if (a.loss_kind == 0) {
+                                    loss_acc += fabsf(d);
+                                    g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);   // torch sign()
+                                } else {
+                                    loss_acc = fmaf(d, d, loss_acc);
+                                    g.v[c] = 2.0f * a.grad_scale * d;
+                                }
+                            }
+                            sts_row<CE>(G, i * RB, g);
+                        }
+                    }
+                }
+                __syncthreads();
+                unsigned char* t = Xc;
+                Xc = Xn;
+                Xn = t;
+            }
+            tr.mark();   // 3 .. 2+L: forward steps
+        }
+        {
+            float one[1] = {loss_acc};
+            block_reduce<1>(one, red, a.loss_partials + tile);
+        }
+        tr.mark();   // loss reduced
+        tile_backward_rk4<CE, W, ELLS>(a, tile, n0, NT, smem, lay, Ein, Eout, Mu, red);
+        tr.mark();   // backward + block reduction done
+        }
     }
 
     // ---- tail: the last CTA to finish reduces the partials (fixed order -> deterministic), applies
@@ -1415,11 +1504,12 @@ int launch_bwd_rk4_t(const Args& a, int threads, cudaStream_t st) {
     return GAD_OK;
 }
 
-template <int CE, int W, bool ELLS>
-int launch_train_t(const Args& a_in, int threads, cudaStream_t st) {
+template <int CE, int W, bool ELLS, int METHOD>
+int launch_train_m(const Args& a_in, int threads, cudaStream_t st) {
     int grid = 0, rc;
-    const size_t bytes = make_layout(CE, KIND_BWD, a_in.cap_nodes, ELLS, (threads + 31) / 32).total;
-    if ((rc = prepare_launch(k_ell_train<CE, W, ELLS>, threads, bytes, a_in.T + 1, &grid))) return rc;
+    const int kind = METHOD == GAD_METHOD_RK4 ? KIND_TRAIN_RK4 : KIND_BWD;
+    const size_t bytes = make_layout(CE, kind, a_in.cap_nodes, ELLS, (threads + 31) / 32).total;
+    if ((rc = prepare_launch(k_ell_train<CE, W, ELLS, METHOD>, threads, bytes, a_in.T + 1, &grid))) return rc;
     Args a = a_in;
     // grid == T + 1: every tile has its own CTA and one more fits -> that one is the reducer
     static const bool allow_reducer = !(getenv("GAD_TAIL_CTA") && atoi(getenv("GAD_TAIL_CTA")) == 0);
@@ -1438,16 +1528,22 @@ int launch_train_t(const Args& a_in, int threads, cudaStream_t st) {
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_ell_train<CE, W, ELLS>, a));
+        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_ell_train<CE, W, ELLS, METHOD>, a));
         count_launch(1);
         return GAD_OK;
     }
-    k_ell_train<CE, W, ELLS><<<grid, threads, bytes, st>>>(a);
+    k_ell_train<CE, W, ELLS, METHOD><<<grid, threads, bytes, st>>>(a);
     GAD_LAUNCH_CHECK();
     return GAD_OK;
 }
 
-// which: 0 forward, 1 backward, 2 train, 3 backward through RK4 steps
+template <int CE, int W, bool ELLS>
+int launch_train_t(const Args& a, int method, int threads, cudaStream_t st) {
+    if (method == GAD_METHOD_RK4) return launch_train_m<CE, W, ELLS, GAD_METHOD_RK4>(a, threads, st);
+    return launch_train_m<CE, W, ELLS, GAD_METHOD_EULER>(a, threads, st);
+}
+
+// which: 0 forward, 1 backward, 2 train (Euler or RK4 by `method`), 3 backward through RK4 steps
 #define GAD_ELL_INSTANTIATE(CE_, W_)                                                                         \
     int ell_launch_c##CE_##w##W_(int which, const Args& a, int method, int ells, int threads, cudaStream_t st) { \
         if (which == 3)                                                                                      \
@@ -1457,7 +1553,8 @@ int launch_train_t(const Args& a_in, int threads, cudaStream_t st) {
                         : launch_fwd_t<CE_, W_, false>(a, method, threads, st);                              \
         if (which == 1)                                                                                      \
             return ells ? launch_bwd_t<CE_, W_, true>(a, threads, st) : launch_bwd_t<CE_, W_, false>(a, threads, st); \
-        return ells ? launch_train_t<CE_, W_, true>(a, threads, st) : launch_train_t<CE_, W_, false>(a, threads, st); \
+        return ells ? launch_train_t<CE_, W_, true>(a, method, threads, st)                                 \
+                    : launch_train_t<CE_, W_, false>(a, method, threads, st);                               \
     }
 
 #define GAD_ELL_DECLARE(CE_, W_) \

@@ -241,6 +241,23 @@ def _tile_bias_grads(ws: torch.Tensor, T: int, Lw: int, L: int, CE: int) -> torc
     return part[:, :, CE * CE:CE * CE + CE].clone()
 
 
+def rk4_backward_resident(graph: MeshGraph, CE: int, force_stream: bool = False) -> bool:
+    """Which kernel runs the backward through RK4 steps on `graph`: True for the mesh-resident one
+    (csrc/ell_kernels.cuh: k_ell_bwd_rk4, gad_deform_bwd_ell_rk4), False for the streaming chain
+    (csrc/stream_ell.cu, gad_deform_bwd_wide_rk4; its wide rows are built here, so call this outside any capture).
+    Raises NotImplementedError when neither serves the graph.  The module path and DeformerTrainer both ask here."""
+    lib = _lib.load()
+    if (graph.tile_ptr is not None and not force_stream and use_ell(graph, CE)
+            and lib.gad_ell_rk4_bwd_supported(CE, graph.max_tile_nodes, graph.ell_deg)):
+        return True
+    if not graph.ensure_wide(CE):
+        raise NotImplementedError(
+            "backward through ode_method='rk4': meshes of at most ~1200 nodes run on the mesh-resident ELL kernel, "
+            "larger ones on the streaming ELL kernels, both for degree <= 7 and 2 or 4 live channels; this graph "
+            f"has max degree {max(graph.max_in_deg, graph.max_out_deg)}, CE = {CE}")
+    return False
+
+
 def deform_backward_rk4(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.Tensor, dim: int, Mu: torch.Tensor,
                         tau: torch.Tensor, want_gx0: bool = False, du: Optional[torch.Tensor] = None,
                         force_stream: bool = False):
@@ -256,17 +273,10 @@ def deform_backward_rk4(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.T
     dev = states.device
     gMu = torch.empty_like(Mu)
     g_x0 = torch.empty((N, CE), dtype=torch.float32, device=dev) if want_gx0 else None
-    resident = (graph.tile_ptr is not None and not force_stream and use_ell(graph, CE)
-                and lib.gad_ell_rk4_bwd_supported(CE, graph.max_tile_nodes, graph.ell_deg))
-    if not resident:
+    if not rk4_backward_resident(graph, CE, force_stream):
         if du is not None:
             raise NotImplementedError("global CNN features reach the kernels as a per-tile bias offset: meshes that fit "
                                       "a CTA only (backward through ode_method='rk4' on the streaming kernels has none)")
-        if not graph.ensure_wide(CE):
-            raise NotImplementedError(
-                "backward through ode_method='rk4': meshes of at most ~1200 nodes run on the mesh-resident ELL kernel, "
-                "larger ones on the streaming ELL kernels, both for degree <= 7 and 2 or 4 live channels; this graph "
-                f"has max degree {max(graph.max_in_deg, graph.max_out_deg)}, CE = {CE}")
         ws_bytes = lib.gad_deform_bwd_wide_rk4_workspace_bytes(N, CE)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         with _on_device(dev):

@@ -14,6 +14,11 @@ partials in a fixed order, applies the chain rule to the Linear parameters, take
 and refolds (M, u) for the next step.  With more than one rank the kernel stops after the chain
 rule, NCCL all-reduces the flat gradient, and Adam + refold follow as two tiny kernels.
 
+`ode_method='rk4'` trains the same way through `gad_train_step_ell_rk4` (k_ell_train with RK4 steps) where a
+tile fits its nine rows per node (`gad_ell_rk4_train_supported`).  Larger tiles and meshes beyond one CTA run the
+launch chain: forward, mesh loss, the RK4 backward of `functional.rk4_backward_resident`'s choice, weight
+gradients, Adam.  The step sizes get no gradient through RK4, so `learn_step` is refused.
+
 Sharding (SURVEY 8e): a batch is a disjoint union of meshes, so ranks take contiguous shards of
 whole meshes with no data-path collective; the only exchange is the all-reduce of the flat
 gradient (144 + L floats).  The mesh loss is a mean over ALL nodes of the global batch
@@ -84,9 +89,8 @@ class DeformerTrainer:
         self.CE = model.CE
         self.dim = model.dim
         self.method = GF.METHODS[opt.get("ode_method", "euler")]
-        if self.method != GF.METHOD_EULER:
-            raise NotImplementedError("DeformerTrainer fuses the Euler step; ode_method='rk4' trains through GNN.forward + "
-                                      "autograd (hand-written RK4 backward kernel, csrc/ell_kernels.cuh: k_ell_bwd_rk4)")
+        if self.method == GF.METHOD_RK4 and opt["learn_step"]:
+            raise NotImplementedError("learn_step with ode_method='rk4': the step sizes get no gradient through RK4")
         self._flatten_parameters()
         self.slots: List[_Slot] = []
         self.graphs: Dict[int, torch.cuda.CUDAGraph] = {}
@@ -240,7 +244,18 @@ class DeformerTrainer:
             if streaming:
                 s.graph.ensure_wide(self.CE)     # wide rows for the streaming ELL kernels, built outside any capture
             s.prefer_stream = None
-            if T == 0 and not self.opt.get("gad_no_cluster", False) and s.graph.ensure_cluster(self.CE):
+            s.rk4_fused = s.rk4_resident = False
+            if self.method == GF.METHOD_RK4:
+                g = s.graph
+                s.rk4_fused = bool(T and GF.use_ell(g, self.CE)
+                                   and lib.gad_ell_rk4_train_supported(self.CE, g.max_tile_nodes, g.ell_deg))
+                if not self._fused_ell(s):
+                    # launch chain: the RK4 backward kernel is chosen (and wide rows built) here, outside any capture
+                    s.rk4_resident = GF.rk4_backward_resident(g, self.CE, self.opt.get("gad_force_stream", False))
+                    s.bwd_ws_bytes = max(s.bwd_ws_bytes, lib.gad_deform_bwd_wide_rk4_workspace_bytes(N, self.CE))
+                    s.bwd_ws = torch.empty(s.bwd_ws_bytes, dtype=torch.uint8, device=dev)
+            if (T == 0 and self.method == GF.METHOD_EULER and not self.opt.get("gad_no_cluster", False)
+                    and s.graph.ensure_cluster(self.CE)):
                 s.prefer_stream = bool(s.graph.stream_train_preferred(self.CE))   # decided outside any capture
                 need = lib.gad_cluster_workspace_bytes(self.CE, len(s.graph.mesh_sizes), s.graph.cl_C, self.L)
                 if need > s.bwd_ws_bytes:
@@ -343,7 +358,7 @@ class DeformerTrainer:
         CE, L, Lw, C_, dim = self.CE, self.L, self.Lw, self.C, self.dim
         tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
         inv_temp = self.model.inv_temp
-        ell = tiles and GF.use_ell(g, CE) and not self.opt.get("gad_no_fused_train", False)
+        ell = self._fused_ell(s)
         cluster = (not ell) and self._cluster(s)
         if ell or cluster:
             # ONE launch per step (csrc/ell_kernels.cuh: k_ell_train): pack + forward + loss + backward per
@@ -353,6 +368,9 @@ class DeformerTrainer:
             if stage in ("all", "pre") and cluster:
                 chk(lib.gad_train_step_cluster(C.byref(self._train_desc(s, 2 if single else 1)), g.cl_C, stream_ptr),
                     "gad_train_step_cluster")
+            elif stage in ("all", "pre") and self.method == GF.METHOD_RK4:
+                chk(lib.gad_train_step_ell_rk4(C.byref(self._train_desc(s, 2 if single else 1)), stream_ptr),
+                    "gad_train_step_ell_rk4")
             elif stage in ("all", "pre"):
                 chk(lib.gad_train_step_ell(C.byref(self._train_desc(s, 2 if single else 1)), stream_ptr),
                     "gad_train_step_ell")
@@ -385,7 +403,16 @@ class DeformerTrainer:
                                   P(s.loss_ws),
                                   stream_ptr),
                 "gad_mesh_loss")
-            if wide:
+            if self.method == GF.METHOD_RK4 and s.rk4_resident:
+                chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
+                                               g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), None, Lw,
+                                               P(self.tau), L, P(self.gMu), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
+                    "gad_deform_bwd_ell_rk4")
+            elif self.method == GF.METHOD_RK4:
+                chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
+                                                dim, CE, P(self.Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
+                                                s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
+            elif wide:
                 chk(lib.gad_deform_bwd_wide(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out), dim, CE,
                                             P(self.Mu), Lw, P(self.tau), L, P(self.gMu), P(self.gtau), None, P(s.bwd_ws),
                                             s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide")
@@ -413,11 +440,18 @@ class DeformerTrainer:
         else:
             dp.allreduce_flat(self.gflat, group=self.pg)
 
-    def _cluster(self, s: _Slot) -> bool:
-        """Meshes too large for one CTA run on the cluster-resident kernel (csrc/cl_kernels.cu)."""
+    def _fused_ell(self, s: _Slot) -> bool:
+        """The step of this slot is the one-launch kernel k_ell_train (gad_train_step_ell / _rk4)."""
         g = s.graph
-        if not (g.tile_ptr is None and g.cl_in is not None and not self.opt.get("gad_no_cluster", False)
-                and not self.opt.get("gad_force_stream", False)):
+        tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
+        return bool(tiles and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
+                    and (self.method == GF.METHOD_EULER or s.rk4_fused))
+
+    def _cluster(self, s: _Slot) -> bool:
+        """Meshes too large for one CTA run on the cluster-resident kernel (csrc/cl_kernels.cu, Euler only)."""
+        g = s.graph
+        if not (self.method == GF.METHOD_EULER and g.tile_ptr is None and g.cl_in is not None
+                and not self.opt.get("gad_no_cluster", False) and not self.opt.get("gad_force_stream", False)):
             return False
         if s.prefer_stream is None:      # one or two very large meshes: the streaming chain uses all SMs
             s.prefer_stream = bool(g.stream_train_preferred(self.CE))
@@ -429,9 +463,7 @@ class DeformerTrainer:
         return self._one_launch_local(s) and (self.world == 1 or s.peer_route)
 
     def _one_launch_local(self, s: _Slot) -> bool:
-        g = s.graph
-        tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
-        return bool(tiles and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)) or self._cluster(s)
+        return self._fused_ell(s) or self._cluster(s)
 
     def close(self):
         """Drop the captured graphs and the peer mappings (call on every rank, after the last step)."""

@@ -245,6 +245,16 @@ int gad_deform_bwd_ell_rk4(const void* ell_in, const void* ell_out, int64_t N, c
                            int CE, const float* Mu, const float* du, int Lw, const float* tau, int L, float* gMu,
                            float* g_x0, void* workspace, size_t workspace_bytes, void* stream);
 int gad_ell_rk4_bwd_supported(int CE, int max_tile_nodes, int max_deg);
+/* One whole training step through classical RK4 steps in one launch: gad_train_step_ell's contract and descriptor
+ * (declared below) with the forward of gad_deform_fwd_ell* (method = GAD_METHOD_RK4) and the backward of
+ * gad_deform_bwd_ell_rk4 in the kernel; the loss and its cotangent are fused into stage 4 of the last step, and the
+ * tail (reduction, chain rule, peer all-reduce, Adam, refold) is gad_train_step_ell's.  desc->g_tau must be NULL: the
+ * step sizes get no gradient through RK4.  gad_ell_rk4_train_supported: 1 when a tile of that size fits the kernel's
+ * shared memory (nine rows, the loss row and both ELL rows per node: 184 B at CE = 4); otherwise train through
+ * gad_deform_fwd* + gad_mesh_loss + gad_deform_bwd_ell_rk4 / gad_deform_bwd_wide_rk4. */
+struct gad_train_desc;
+int gad_train_step_ell_rk4(const struct gad_train_desc* desc, void* stream);
+int gad_ell_rk4_train_supported(int CE, int max_tile_nodes, int max_deg);
 int gad_deform_train_ell(const void* ell_in, const void* ell_out, int64_t N, const int32_t* tile_ptr, int T,
                          int max_tile_nodes, int max_deg, const float* x_comp, const float* f,
                          const float* uu, const float* f_scale, const float* uu_scale, const float* target,
