@@ -447,11 +447,17 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_fwd(const Ar
 // ============================================================================================
 // On entry (all visible to the CTA): X = x^{L-1} rows, GS = dL/dx^L rows, Mu = weights of layer
 // L-1.  acc: per-thread (G_M, G_u[, g_tau]) accumulators, zero on entry.
-template <int CE, int W, bool ELLS>
+// FUSED_LAST (k_ell_train): the caller has already run phase A of layer L-1 inside its last forward
+// layer (ell_feval_bwd_dst) and synchronised the CTA: GO / P / DL / GS hold that pass's rows, and
+// acc_in / gtau_in its accumulators; the loop starts at phase B of layer L-1.  Then phase A also skips
+// what nothing reads: g_tau terms without a g_tau column, and M t and the row stores of a layer that
+// is followed by no source pass.
+template <int CE, int W, bool ELLS, bool FUSED_LAST = false>
 __device__ __forceinline__ void tile_backward(const Args& a, int tile, int n0, int NT, unsigned char* X,
                                               unsigned char* GO, unsigned char* P, unsigned char* DL,
                                               unsigned char* GS, const EllView<ELLS>& Ein,
-                                              const EllView<ELLS>& Eout, float* Mu, float* red) {
+                                              const EllView<ELLS>& Eout, float* Mu, float* red,
+                                              const float* acc_in = nullptr, float gtau_in = 0.f) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
     constexpr int NACC = MUSZ + 1;
@@ -459,9 +465,10 @@ __device__ __forceinline__ void tile_backward(const Args& a, int tile, int n0, i
     const bool per_layer = (a.Lw > 1);
     const int slots = per_layer ? a.L : 1;
     const size_t state_stride = (size_t)a.N * CE;
+    const bool need_gtau = !FUSED_LAST || per_layer || a.tau_partials != nullptr;
     float acc[NACC];
 #pragma unroll
-    for (int k = 0; k < NACC; ++k) acc[k] = 0.f;
+    for (int k = 0; k < NACC; ++k) acc[k] = FUSED_LAST ? acc_in[k] : 0.f;
 
     for (int l = a.L - 1; l >= 0; --l) {
         if (per_layer && l < a.L - 1) {
@@ -469,9 +476,11 @@ __device__ __forceinline__ void tile_backward(const Args& a, int tile, int n0, i
             __syncthreads();
         }
         const float b = a.tau[l];
-        float gtau = 0.f;
+        const bool fused = FUSED_LAST && l == a.L - 1;
+        float gtau = fused ? gtau_in : 0.f;
         // ---- phase A: destination pass ------------------------------------------------------
-        {
+        if (!fused) {
+            const bool store = !FUSED_LAST || (l > 0) || (a.g_x0 != nullptr);   // a source pass reads the rows
             uint4 e_nx = (tid < NT) ? Ein.get(tid) : make_uint4(0, 0, 0, 0);
             for (int i = tid; i < NT; i += nthr) {
                 const uint4 e = e_nx;
@@ -484,27 +493,31 @@ __device__ __forceinline__ void tile_backward(const Args& a, int tile, int n0, i
                 Row<CE> p, t, o;
                 float D, lse;
                 ell_bwd_dst<CE, W>(X, e, xi, go, Mu, p, D, lse, t, o);
+                if (need_gtau) {
 #pragma unroll
-                for (int c = 0; c < CE; ++c) gtau = fmaf(gp.v[c], o.v[c] - xi.v[c], gtau);
+                    for (int c = 0; c < CE; ++c) gtau = fmaf(gp.v[c], o.v[c] - xi.v[c], gtau);
+                }
 #pragma unroll
                 for (int aa = 0; aa < CE; ++aa)
 #pragma unroll
                     for (int bb = 0; bb < CE; ++bb) acc[aa * CE + bb] = fmaf(xi.v[aa], t.v[bb], acc[aa * CE + bb]);
 #pragma unroll
                 for (int bb = 0; bb < CE; ++bb) acc[CE * CE + bb] += t.v[bb];
-                const Row<CE> Mt = apply_M<CE>(Mu, t);
-                Row<CE> gs;
+                if (store) {
+                    const Row<CE> Mt = apply_M<CE>(Mu, t);
+                    Row<CE> gs;
 #pragma unroll
-                for (int c = 0; c < CE; ++c) gs.v[c] = fmaf(1.0f - b, gp.v[c], Mt.v[c]);   // Euler: a = 1
-                sts_row<CE>(P, i * RB, p);
-                *reinterpret_cast<float2*>(DL + (size_t)i * 8) = make_float2(D, lse);
-                sts_row<CE>(GO, i * RB, go);
-                sts_row<CE>(GS, i * RB, gs);
+                    for (int c = 0; c < CE; ++c) gs.v[c] = fmaf(1.0f - b, gp.v[c], Mt.v[c]);   // Euler: a = 1
+                    sts_row<CE>(P, i * RB, p);
+                    *reinterpret_cast<float2*>(DL + (size_t)i * 8) = make_float2(D, lse);
+                    sts_row<CE>(GO, i * RB, go);
+                    sts_row<CE>(GS, i * RB, gs);
+                }
             }
         }
         const bool need_src = (l > 0) || (a.g_x0 != nullptr);
         if (need_src) {
-            __syncthreads();   // P, DL, GO visible; every gather of X done
+            if (!fused) __syncthreads();   // P, DL, GO visible; every gather of X done
             // ---- phase B: source pass -------------------------------------------------------
             const float* xprev_g = (l > 0) ? a.states + (size_t)(l - 1) * state_stride : nullptr;
             uint4 e_nx = (tid < NT) ? Eout.get(tid) : make_uint4(0, 0, 0, 0);
@@ -1239,6 +1252,14 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
         unsigned char* Xc = B0;
         unsigned char* Xn = B1;
         assemble_rows<CE>(a, n0, NT, stage, st_xc, st_f, st_uu, Xc, nullptr);   // x^0 reaches `states` from the first layer's loop, after the wait
+        if (METHOD == GAD_METHOD_EULER && a.dim == 1 && stage) {
+            // The Euler last layer overwrites the DL row of node i (8 bytes) with (D, lse) right after reading
+            // node i's target.  A staged 1-D target is 4 bytes per node, so that row holds the targets of nodes
+            // 2i and 2i+1, which other threads may not have read yet: move each target into its node's GS row
+            // (unused until then) before the barrier.  At dim 2 the DL row of node i is node i's target.
+            for (int i = tid; i < NT; i += nthr)
+                reinterpret_cast<float*>(GS + i * RB)[0] = reinterpret_cast<const float*>(DL)[i];
+        }
         __syncthreads();
         // previous step done (weights refolded, its reads of `states` finished): from here on this
         // step may read Mu / tau and write global memory
@@ -1258,16 +1279,15 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
         EllView<ELLS> Eout{ELLS ? reinterpret_cast<const uint4*>(smem + lay.eout) : a.ell_out + e0};
 
         if constexpr (METHOD == GAD_METHOD_EULER) {
-        // ---- forward (Euler), loss and cotangent fused into the last layer --------------------
-        float loss_acc = 0.f;
-        for (int l = 0; l < a.L; ++l) {
+        // ---- forward (Euler); the last layer also computes the loss, its cotangent and phase A
+        // (destination pass) of the backward of that layer, from the same gathered rows
+        for (int l = 0; l < a.L - 1; ++l) {
             if (a.Lw > 1 && l > 0) {
                 for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
                 __syncthreads();
             }
             const float h = __ldcg(a.tau + l);
-            const bool last = (l == a.L - 1);
-            float* st_out = last ? nullptr : a.states + (size_t)(l + 1) * state_stride;
+            float* st_out = a.states + (size_t)(l + 1) * state_stride;
             float Mr[MUSZ];   // (M, u) in registers for the whole layer: no broadcast loads per node
 #pragma unroll
             for (int t = 0; t < MUSZ; ++t) Mr[t] = Mu[t];
@@ -1281,48 +1301,112 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
                 Row<CE> xn;
 #pragma unroll
                 for (int c = 0; c < CE; ++c) xn.v[c] = fmaf(h, k.v[c], y.v[c]);
-                if (!last) {
-                    sts_row<CE>(Xn, i * RB, xn);
-                    store_row<CE>(st_out, (int64_t)n0 + i, xn);
-                } else {
-                    const int64_t gi = (int64_t)n0 + i;
-                    if (a.x_phys) store_dims<CE>(a.x_phys, gi, a.dim, xn);
-                    const Row<CE> tg = stage ? load_dims<CE>(reinterpret_cast<const float*>(DL), i, a.dim)
-                                             : load_dims<CE>(a.target, gi, a.dim);
-                    Row<CE> g;
-#pragma unroll
-                    for (int c = 0; c < CE; ++c) {
-                        const float d = (c < a.dim) ? xn.v[c] - tg.v[c] : 0.f;
-                        if (a.loss_kind == 0) {
-                            loss_acc += fabsf(d);
-                            g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);   // torch sign()
-                        } else {
-                            loss_acc = fmaf(d, d, loss_acc);
-                            g.v[c] = 2.0f * a.grad_scale * d;
-                        }
-                    }
-                    sts_row<CE>(GS, i * RB, g);
-                }
+                sts_row<CE>(Xn, i * RB, xn);
+                store_row<CE>(st_out, (int64_t)n0 + i, xn);
             }
             __syncthreads();
             tr.mark();   // 3 .. 2+L: forward layers
-            if (!last) {
-                unsigned char* t = Xc;
-                Xc = Xn;
-                Xn = t;
-            }
-        }
-        // Xc = x^{L-1} (never overwritten by the last layer), Xn = free -> GO
-        if (a.Lw > 1) {
-            // weights of layer L-1 are already in Mu
+            unsigned char* t = Xc;
+            Xc = Xn;
+            Xn = t;
         }
         {
+            // last layer, l = L-1: Xc = x^{L-1} (kept for the backward), Xn is free and takes the GO rows
+            const int l = a.L - 1;
+            if (a.Lw > 1 && l > 0) {
+                for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
+                __syncthreads();
+            }
+            const float h = __ldcg(a.tau + l);
+            const bool src = (l > 0) || (a.g_x0 != nullptr);   // a source pass follows: the rows below are read
+            const bool need_gtau = (a.Lw > 1) || (a.tau_partials != nullptr);
+            const unsigned char* TG = (a.dim == 1) ? GS : DL;   // staged target of node i, see the feature assembly
+            const uint32_t tg_rb = (a.dim == 1) ? RB : 8u;
+            constexpr int NACC = MUSZ + 1;
+            float acc[NACC];
+#pragma unroll
+            for (int k = 0; k < NACC; ++k) acc[k] = 0.f;
+            float gtau = 0.f, loss_acc = 0.f;
+            if (l == 0)   // L = 1: x^0 reaches `states` here
+                for (int i = tid; i < NT; i += nthr) store_row<CE>(a.states, (int64_t)n0 + i, lds_row<CE>(Xc, i * RB));
+            uint4 e_nx = (tid < NT) ? Ein.get(tid) : make_uint4(0, 0, 0, 0);
+            for (int i = tid; i < NT; i += nthr) {
+                const uint4 e = e_nx;
+                if (i + nthr < NT) e_nx = Ein.get(i + nthr);
+                const Row<CE> y = lds_row<CE>(Xc, i * RB);
+                const int64_t gi = (int64_t)n0 + i;
+                // x^L = y + h k -> x_phys, loss term and cotangent dL/dx^L of this node
+                auto cot = [&](const Row<CE>& k) {
+                    Row<CE> xn;
+#pragma unroll
+                    for (int c = 0; c < CE; ++c) xn.v[c] = fmaf(h, k.v[c], y.v[c]);
+                    auto term = [&](float d) {   // adds d's loss term, returns its cotangent entry
+                        if (a.loss_kind == 0) {
+                            loss_acc += fabsf(d);
+                            return (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);   // torch sign()
+                        }
+                        loss_acc = fmaf(d, d, loss_acc);
+                        return 2.0f * a.grad_scale * d;
+                    };
+                    Row<CE> g = zero_row<CE>();
+                    if (a.dim == 2) {
+                        // 2-D meshes: float2 rows, no per-channel tests; the channels beyond dim have d = 0, whose
+                        // loss term (+0) and cotangent (0) the general form below would add
+                        if (a.x_phys) *reinterpret_cast<float2*>(a.x_phys + gi * 2) = make_float2(xn.v[0], xn.v[1]);
+                        const float2 tg = stage ? *reinterpret_cast<const float2*>(DL + (size_t)i * 8)
+                                                : *reinterpret_cast<const float2*>(a.target + gi * 2);
+                        g.v[0] = term(xn.v[0] - tg.x);
+                        g.v[1] = term(xn.v[1] - tg.y);
+                    } else {
+                        if (a.x_phys) store_dims<CE>(a.x_phys, gi, a.dim, xn);
+                        const Row<CE> tg = stage ? load_dims<CE>(reinterpret_cast<const float*>(TG + i * tg_rb), 0, a.dim)
+                                                 : load_dims<CE>(a.target, gi, a.dim);
+#pragma unroll
+                        for (int c = 0; c < CE; ++c) g.v[c] = term((c < a.dim) ? xn.v[c] - tg.v[c] : 0.f);
+                    }
+                    return g;
+                };
+                const Row<CE> p = project<CE>(Mu, y);
+                if (src) sts_row<CE>(P, i * RB, p);
+                Row<CE> gp, t, o;
+                float D, lse;
+                ell_feval_bwd_dst<CE, W>(Xc, e, y, p, h, cot, gp, D, lse, t, o);
+                // the rest of tile_backward's phase A at xi = y, b = h
+                if (need_gtau) {
+#pragma unroll
+                    for (int c = 0; c < CE; ++c) gtau = fmaf(gp.v[c], o.v[c] - y.v[c], gtau);
+                }
+#pragma unroll
+                for (int aa = 0; aa < CE; ++aa)
+#pragma unroll
+                    for (int bb = 0; bb < CE; ++bb) acc[aa * CE + bb] = fmaf(y.v[aa], t.v[bb], acc[aa * CE + bb]);
+#pragma unroll
+                for (int bb = 0; bb < CE; ++bb) acc[CE * CE + bb] += t.v[bb];
+                if (src) {
+                    const Row<CE> Mt = apply_M<CE>(Mu, t);
+                    Row<CE> go, gs;
+#pragma unroll
+                    for (int c = 0; c < CE; ++c) {
+                        go.v[c] = h * gp.v[c];
+                        gs.v[c] = fmaf(1.0f - h, gp.v[c], Mt.v[c]);   // Euler: a = 1
+                    }
+                    // at dim 2 the DL row of node i held node i's staged target, read above by this thread only
+                    *reinterpret_cast<float2*>(DL + (size_t)i * 8) = make_float2(D, lse);
+                    sts_row<CE>(Xn, i * RB, go);
+                    sts_row<CE>(GS, i * RB, gs);
+                }
+            }
+            // the tile's loss: warp sums before the barrier that ends the layer, the cross-warp sum after it
             float one[1] = {loss_acc};
-            block_reduce<1>(one, red, a.loss_partials + tile);
+            block_reduce_warps<1>(one, red);
+            __syncthreads();
+            tr.mark();   // 2+L: last forward layer + phase A of its backward
+            block_reduce_finish<1>(red, a.loss_partials + tile);
+            if (!src) __syncthreads();   // the block reduction that follows at once reuses `red`
+            tr.mark();   // loss reduced
+            tile_backward<CE, W, ELLS, true>(a, tile, n0, NT, Xc, Xn, P, DL, GS, Ein, Eout, Mu, red, acc, gtau);
+            tr.mark();   // backward + block reduction done
         }
-        tr.mark();   // loss reduced
-        tile_backward<CE, W, ELLS>(a, tile, n0, NT, Xc, Xn, P, DL, GS, Ein, Eout, Mu, red);
-        tr.mark();   // backward + block reduction done
         } else {
         // ---- forward (RK4 steps), loss and cotangent fused into stage 4 of the last step ----------
         unsigned char* XB = P;    // base state of the step

@@ -142,6 +142,58 @@ __device__ __forceinline__ void ell_bwd_dst(const unsigned char* __restrict__ Xb
     }
 }
 
+// ---- last forward layer fused with the destination pass of its backward ------------------------
+// One gather of the row serves both.  p = project(Mu, y) comes from the caller (which can store it
+// before the gathers: fewer live registers).  k = F(y) as ell_feval; gp = cot(k) = dL/dx^L at this node (the
+// caller's node-local loss cotangent of x^L = y + b k); then, with go = b * gp, the outputs of ell_bwd_dst
+// at xi = y from the same registers (w_q, m, Z, rZ).  Every term is ell_feval's / ell_bwd_dst's
+// expression, so the bits equal those of the two separate passes.
+template <int CE, int W, typename Cot>
+__device__ __forceinline__ void ell_feval_bwd_dst(const unsigned char* __restrict__ Xb, const uint4& ell,
+                                                  const Row<CE>& y, const Row<CE>& p, float b, Cot cot, Row<CE>& gp,
+                                                  float& D, float& lse, Row<CE>& t, Row<CE>& o) {
+    const bool any = ell_valid(ell) != 0;
+    Row<CE> xj[W];
+    float s[W];
+    float m = -3.0e38f;
+#pragma unroll
+    for (int q = 0; q < W; ++q) {
+        xj[q] = lds_row<CE>(Xb, ell_off(ell, q));
+        const float d = dot<CE>(p, xj[q]);
+        s[q] = ell_has(ell, q) ? d : -CUDART_INF_F;
+        m = fmaxf(m, s[q]);
+    }
+    float Z = 0.f;
+    o = zero_row<CE>();
+#pragma unroll
+    for (int q = 0; q < W; ++q) {
+        s[q] = ex2_approx(s[q] - m);   // w_q
+        Z += s[q];
+#pragma unroll
+        for (int c = 0; c < CE; ++c) o.v[c] = fmaf(s[q], xj[q].v[c], o.v[c]);
+    }
+    const float rZ = any ? rcp_refined(Z) : 0.f;
+    Row<CE> k;
+#pragma unroll
+    for (int c = 0; c < CE; ++c) k.v[c] = fmaf(o.v[c], rZ, -y.v[c]);
+    gp = cot(k);
+    Row<CE> go;
+#pragma unroll
+    for (int c = 0; c < CE; ++c) go.v[c] = b * gp.v[c];
+#pragma unroll
+    for (int c = 0; c < CE; ++c) o.v[c] *= rZ;
+    D = dot<CE>(go, o);
+    lse = any ? m + lg2_approx(Z) : 0.f;
+    const float scale = rZ * LN2_F;
+    t = zero_row<CE>();
+#pragma unroll
+    for (int q = 0; q < W; ++q) {
+        const float ds = (s[q] * scale) * (dot<CE>(go, xj[q]) - D);
+#pragma unroll
+        for (int c = 0; c < CE; ++c) t.v[c] = fmaf(ds, xj[q].v[c], t.v[c]);
+    }
+}
+
 // ---- backward, source pass ---------------------------------------------------------------------
 // Contributions of the out-edges (j -> i) of node j:  sum_e alpha_e (go_i + c_e p_i),
 // c_e = ln2 (<go_i, x_j> - D_i),  alpha_e = 2^(<p_i, x_j> - lse_i).

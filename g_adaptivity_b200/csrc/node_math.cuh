@@ -347,10 +347,10 @@ __device__ __forceinline__ Row<CE> node_bwd_src(const float* __restrict__ P, con
 }
 
 // Deterministic block-wide sum of NACC per-thread accumulators into out[0..NACC).
-// red must hold NACC * (blockDim/32) floats.
+// red must hold NACC * (blockDim/32) floats.  The two halves are also called on their own by a
+// caller that already has a barrier between them (and keeps `red` untouched until the second is done).
 template <int NACC>
-__device__ __forceinline__ void block_reduce(float (&acc)[NACC], float* __restrict__ red,
-                                             float* __restrict__ out) {
+__device__ __forceinline__ void block_reduce_warps(const float (&acc)[NACC], float* __restrict__ red) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = (blockDim.x + 31) >> 5;
 #pragma unroll
     for (int k = 0; k < NACC; ++k) {
@@ -359,12 +359,24 @@ __device__ __forceinline__ void block_reduce(float (&acc)[NACC], float* __restri
         for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
         if (lane == 0) red[k * nwarp + warp] = v;
     }
-    __syncthreads();
+}
+
+template <int NACC>
+__device__ __forceinline__ void block_reduce_finish(const float* __restrict__ red, float* __restrict__ out) {
+    const int nwarp = (blockDim.x + 31) >> 5;
     for (int k = threadIdx.x; k < NACC; k += blockDim.x) {
         double s = 0.0;   // the sums cancel heavily (signed gradient terms): keep the cross-warp step exact
         for (int w = 0; w < nwarp; ++w) s += (double)red[k * nwarp + w];
         out[k] = (float)s;
     }
+}
+
+template <int NACC>
+__device__ __forceinline__ void block_reduce(float (&acc)[NACC], float* __restrict__ red,
+                                             float* __restrict__ out) {
+    block_reduce_warps<NACC>(acc, red);
+    __syncthreads();
+    block_reduce_finish<NACC>(red, out);
     __syncthreads();
 }
 
