@@ -379,22 +379,7 @@ class GNN(nn.Module):
         lib_c = GF.fold_scale(self.inv_temp, int(opt["hidden_dim"]))
         sizes = self._mesh_sizes(data)
         B, N1 = len(sizes), int(sizes[0])
-        gather = self.__dict__.get("_cnn_gather")
-        if gather is None or gather.numel() != N1 or gather.device != dev:
-            if self.dim == 2:
-                mapping = getattr(self.dataset, "mapping_tensor", None)
-                if opt.get("data_type") == "randg_mix":
-                    mapping = getattr(data, "mapping_tensor", mapping)
-                if mapping is None:
-                    raise ValueError("global CNN features on 2-D meshes need dataset.mapping_tensor (src/GNN.py:245)")
-                n = int(round(N1 ** 0.5))
-                # reshape_fd_tensor_to_grid (utils_data.py:125-141): gather by the mapping, reshape [n, n], transpose,
-                # flip rows -- as ONE index map applied by the kernel's load: grid[r, c] = u[mapping[c * n + n - 1 - r]]
-                r, c = torch.meshgrid(torch.arange(n), torch.arange(n), indexing="ij")
-                gather = torch.as_tensor(mapping).reshape(-1)[(c * n + (n - 1 - r)).reshape(-1)].to(dev, torch.int32)
-            else:
-                gather = torch.arange(N1, dtype=torch.int32, device=dev)
-            self.__dict__["_cnn_gather"] = gather
+        gather = self._cnn_grid_map(data, N1, dev)
         feats = []
         if opt["gnn_inc_glob_feat_f"]:
             src = data.f_tensor.to(dev, non_blocking=True) if f is None else f
@@ -414,6 +399,27 @@ class GNN(nn.Module):
         if self.live < self.CE:
             du = torch.nn.functional.pad(du, (0, self.CE - self.live))
         return du.contiguous()
+
+    def _cnn_grid_map(self, data, N1: int, dev) -> torch.Tensor:
+        """int32 [N1]: the node of a mesh whose value sits in each cell of the CNN's grid (cached)."""
+        opt = self.opt
+        gather = self.__dict__.get("_cnn_gather")
+        if gather is None or gather.numel() != N1 or gather.device != dev:
+            if self.dim == 2:
+                mapping = getattr(self.dataset, "mapping_tensor", None)
+                if opt.get("data_type") == "randg_mix":
+                    mapping = getattr(data, "mapping_tensor", mapping)
+                if mapping is None:
+                    raise ValueError("global CNN features on 2-D meshes need dataset.mapping_tensor (src/GNN.py:245)")
+                n = int(round(N1 ** 0.5))
+                # reshape_fd_tensor_to_grid (utils_data.py:125-141): gather by the mapping, reshape [n, n], transpose,
+                # flip rows -- as ONE index map applied by the kernel's load: grid[r, c] = u[mapping[c * n + n - 1 - r]]
+                r, c = torch.meshgrid(torch.arange(n), torch.arange(n), indexing="ij")
+                gather = torch.as_tensor(mapping).reshape(-1)[(c * n + (n - 1 - r)).reshape(-1)].to(dev, torch.int32)
+            else:
+                gather = torch.arange(N1, dtype=torch.int32, device=dev)
+            self.__dict__["_cnn_gather"] = gather
+        return gather
 
     def _fem2d_topology(self, dev, num_nodes: int):
         """Triangulation tables of `dataset.mesh` for the batched 2-D FEM kernels, built once per model.

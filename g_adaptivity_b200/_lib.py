@@ -122,6 +122,9 @@ SIGNATURES = {
     "gad_cnn_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
     "gad_cnn_fwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_p), _p, _p, _sz, _p]),
     "gad_cnn_bwd": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, C.POINTER(_p), C.POINTER(_p), _p, _p, _p, _sz, _p]),
+    "gad_glob_bias_fwd": (_i, [_p, _p, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _f, _p, _p]),
+    "gad_glob_bias_bwd": (_i, [_p, _p, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _f, _p, _sz, _p, _p, _p, _p, _p]),
+    "gad_absmax": (_i, [_p, _i64, _p, _p]),
     "gad_host_alloc": (_i, [_sz, _i, C.POINTER(_p)]),
     "gad_host_free": (_i, [_p]),
     "gad_pipeline_run": (_i, [C.POINTER(PipelineSlot), _i, C.POINTER(_p), _i, _i64, _p, _p, _p]),

@@ -19,6 +19,10 @@ tile fits its nine rows per node (`gad_ell_rk4_train_supported`).  Larger tiles 
 launch chain: forward, mesh loss, the RK4 backward of `functional.rk4_backward_resident`'s choice, weight
 gradients, Adam.  The step sizes get no gradient through RK4, so `learn_step` is refused.
 
+Global CNN features (`gnn_inc_glob_feat_f / _uu` with channels that survive the encoder) train as a chain of library
+kernels: CNN forward, the per-mesh bias offset du (csrc/glob_train.cu), the mesh-resident forward and backward with du,
+the adjoint of du, CNN backward into the flat gradient, Adam over Linear and CNN parameters (`_issue_glob`).
+
 Sharding (SURVEY 8e): a batch is a disjoint union of meshes, so ranks take contiguous shards of
 whole meshes with no data-path collective; the only exchange is the all-reduce of the flat
 gradient (144 + L floats).  The mesh loss is a mean over ALL nodes of the global batch
@@ -40,6 +44,11 @@ import torch.distributed as dist
 from . import _lib, dp
 from . import functional as GF
 from .GNN import GNN
+
+
+def _ptr_array(tensors):
+    """Host array of device pointers (the per-layer weight / bias arguments of gad_cnn_fwd / gad_cnn_bwd)."""
+    return (C.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors])
 
 
 class _Slot:
@@ -65,9 +74,6 @@ class DeformerTrainer:
                 f"DeformerTrainer fuses the mesh loss (loss_type='mesh_loss', src/run_GNN.py:105-107); opt['loss_type']="
                 f"{opt['loss_type']!r} trains through GNN.forward + autograd instead.  Pass loss_fn='l1' / 'mse' explicitly "
                 "to train the mesh loss on such a preset")
-        if getattr(model, "n_glob_used", 0) or opt.get("gnn_inc_glob_feat_f") or opt.get("gnn_inc_glob_feat_uu"):
-            raise NotImplementedError("DeformerTrainer: global CNN features are trained through GNN.forward + autograd "
-                                      "(the fused step does not update the CNN's parameters)")
         if opt.get("softmax_temp_type") == "learnable_a":
             raise NotImplementedError("DeformerTrainer: the learnable temperature is trained through GNN.forward + autograd")
         if opt.get("gnn_normalize", False):
@@ -91,6 +97,9 @@ class DeformerTrainer:
         self.method = GF.METHODS[opt.get("ode_method", "euler")]
         if self.method == GF.METHOD_RK4 and opt["learn_step"]:
             raise NotImplementedError("learn_step with ode_method='rk4': the step sizes get no gradient through RK4")
+        # global CNN channels that survive the encoder's truncation; with none the model is a plain deformer and its
+        # CNNs are never run (GNN.forward skips them too, so torch.optim.Adam never touches their parameters)
+        self.n_g = int(getattr(model, "n_glob_used", 0))
         self._flatten_parameters()
         self.slots: List[_Slot] = []
         self.graphs: Dict[int, torch.cuda.CUDAGraph] = {}
@@ -118,12 +127,22 @@ class DeformerTrainer:
 
     # ------------------------------------------------------------------------------------
     def _flatten_parameters(self):
-        """flat = [Wq (Lw,C,C) | bq (Lw,C) | Wk (Lw,C,C) | bk (Lw,C) | steps (L, if learn_step)]."""
+        """flat = [Wq (Lw,C,C) | bq (Lw,C) | Wk (Lw,C,C) | bk (Lw,C) | steps (L, if learn_step) | CNN f | CNN uu], the
+        parameters of each global feature extractor in gad_cnn_bwd's order (w_0, b_0, w_1, ...), when n_g > 0."""
         m, Lw, C = self.model, self.Lw, self.C
         convs = [m.conv_layers[0]] if self.opt["share_conv"] else list(m.conv_layers)
         nW, nb = Lw * C * C, Lw * C
         nsteps = self.L if self.opt["learn_step"] else 0
-        n = 2 * nW + 2 * nb + nsteps
+        cnn_specs, before = [], 0
+        for name in (("f", "uu") if self.n_g else ()):
+            ext = getattr(m, f"global_feature_extractor_cnn_{name}", None)
+            if ext is None:
+                continue
+            # an extractor whose outputs the encoder truncates away still trains (zero gradient, weight decay), as the
+            # module's cat + slice gives it; it is never run
+            cnn_specs.append((name, ext, [p for c in ext.convs for p in (c.weight, c.bias)], self.n_g > before))
+            before += ext.out_channels
+        n = 2 * nW + 2 * nb + nsteps + sum(p.numel() for _, _, ps, _ in cnn_specs for p in ps)
         flat = torch.empty(n, dtype=torch.float32, device=self.dev)
         gflat = torch.zeros(n, dtype=torch.float32, device=self.dev)
         o = 0
@@ -148,6 +167,21 @@ class DeformerTrainer:
             else:
                 self.tau = torch.full((self.L,), float(self.opt["time_step"]), dtype=torch.float32, device=self.dev)
                 self.gtau = None
+            o += nsteps
+            self.cnn = []
+            for name, ext, ps, used in cnn_specs:
+                o0, ws, bs = o, [], []
+                for p in ps:
+                    k = p.numel()
+                    view = flat[o:o + k]
+                    view.copy_(p.detach().to(self.dev).reshape(-1))
+                    p.data = view.view(p.shape)
+                    p.grad = gflat[o:o + k].view(p.shape)
+                    (ws if p.dim() > 1 else bs).append(view)
+                    o += k
+                self.cnn.append({"name": name, "used": used, "g": gflat[o0:o], "Cm": ext.mid_channels,
+                                 "Co": ext.out_channels, "L": len(ext.convs),
+                                 "wp": _ptr_array(ws), "bp": _ptr_array(bs)})
         self.flat, self.gflat = flat, gflat
         self.exp_avg = torch.zeros_like(flat)
         self.exp_avg_sq = torch.zeros_like(flat)
@@ -210,16 +244,27 @@ class DeformerTrainer:
         m, dev, lib = self.model, self.dev, self.lib
         s = _Slot()
         with torch.cuda.device(dev):
-            s.graph = m._graph(data, dev, allow_uniform=True)      # the trainer never reads attention weights
+            tile_nodes = None
+            if self.n_g:          # the module's planning: one mesh per tile, so the bias offset is per tile
+                sizes = m._mesh_sizes(data)
+                if any(n != sizes[0] for n in sizes):
+                    raise NotImplementedError("global CNN features need meshes of equal size in a batch")
+                tile_nodes = int(sizes[0])
+            s.graph = m._graph(data, dev, allow_uniform=True, tile_nodes=tile_nodes)   # the trainer never reads attention weights
             N = s.graph.N
             s.N = N
+            s.glob = bool(self.n_g)
+            if s.glob:
+                self._check_glob_graph(s.graph)
             f32 = dict(dtype=torch.float32, device=dev)
             xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
             # node inputs of a step live in ONE device buffer [target | f | uu | x_comp] (segments padded to
             # 16 bytes, the TMA staging granularity), so that a packed host batch travels in one copy.  x_comp
             # comes last: datasets on one shared mesh (`randg`, src/data.py:143: every sample has the same
             # computational mesh) send it once, and a step's copy is the [target | f | uu] prefix only.
-            has_f, has_uu = bool(self.opt["gnn_inc_feat_f"]), bool(self.opt["gnn_inc_feat_uu"])
+            # the global feature extractors read f / uu from the same buffer
+            has_f = bool(self.opt["gnn_inc_feat_f"]) or any(r["name"] == "f" and r["used"] for r in self.cnn)
+            has_uu = bool(self.opt["gnn_inc_feat_uu"]) or any(r["name"] == "uu" and r["used"] for r in self.cnn)
             seg = [N * self.dim, N if has_f else 0, N if has_uu else 0, N * self.dim]
             offs, o = [], 0
             for n in seg:
@@ -261,6 +306,8 @@ class DeformerTrainer:
                 if need > s.bwd_ws_bytes:
                     s.bwd_ws_bytes = need
                     s.bwd_ws = torch.zeros(need, dtype=torch.uint8, device=dev)
+            if s.glob:
+                self._add_glob_buffers(s, data)
             s.fwd_ws_bytes = lib.gad_deform_workspace_bytes(N, self.CE, self.method) if streaming else 0
             s.fwd_ws = torch.empty(max(s.fwd_ws_bytes, 16), dtype=torch.uint8, device=dev)
             s.h2d_bytes = 0
@@ -286,6 +333,32 @@ class DeformerTrainer:
         sid = len(self.slots) - 1
         self.load_inputs(sid, data)
         return sid
+
+    def _check_glob_graph(self, g):
+        """A batch with global CNN features runs on the mesh-resident ELL kernels, one mesh per tile (GNN.forward's
+        planning); anything else raises as the module path does."""
+        if (self.opt.get("gad_force_stream", False) or not GF.use_ell(g, self.CE) or g.mesh_sizes is None
+                or g.T != len(g.mesh_sizes)):
+            raise NotImplementedError("global CNN features (per-mesh bias offset) run on the mesh-resident ELL kernels only")
+        if self.method == GF.METHOD_RK4 and not GF.rk4_backward_resident(g, self.CE):
+            raise NotImplementedError("global CNN features reach the kernels as a per-tile bias offset: meshes that fit "
+                                      "a CTA only (backward through ode_method='rk4' on the streaming kernels has none)")
+
+    def _add_glob_buffers(self, s: "_Slot", data):
+        """CNN grid map, workspace, per-mesh CNN outputs / cotangents and the bias offset of a slot."""
+        f32 = dict(dtype=torch.float32, device=self.dev)
+        B, N1 = len(s.graph.mesh_sizes), int(s.graph.mesh_sizes[0])
+        s.B = B
+        s.cnn_hw = (int(round(N1 ** 0.5)),) * 2 if self.dim == 2 else (1, N1)
+        s.cnn_gather = self.model._cnn_grid_map(data, N1, self.dev)
+        used = [r for r in self.cnn if r["used"]]
+        s.cnn_ws_bytes = max(self.lib.gad_cnn_workspace_bytes(B, s.cnn_hw[0], s.cnn_hw[1], r["Cm"], r["Co"], r["L"])
+                             for r in used)
+        s.cnn_ws = torch.empty(s.cnn_ws_bytes, dtype=torch.uint8, device=self.dev)
+        s.cnn_scale = {r["name"]: torch.zeros(1, **f32) for r in used}
+        s.cnn_out = {r["name"]: torch.zeros((B, r["Co"]), **f32) for r in used}
+        s.cnn_gout = {r["name"]: torch.zeros((B, r["Co"]), **f32) for r in used}
+        s.du = torch.zeros((B, self.Lw, self.CE), **f32)
 
     def _host_buffer(self, numel: int, write_combined: bool) -> torch.Tensor:
         """Pinned fp32 host buffer.  Write-combined pages come from the library (`gad_host_alloc`); the tensor is a view
@@ -353,6 +426,8 @@ class DeformerTrainer:
     # ------------------------------------------------------------------------------------
     def _issue(self, s: _Slot, stream_ptr: int, with_optimizer: bool = True, stage: str = "all"):
         """Enqueue the kernels of one training step on `stream_ptr` (captured or eager)."""
+        if s.glob:
+            return self._issue_glob(s, stream_ptr, with_optimizer, stage)
         lib, P, chk = self.lib, _lib.ptr, _lib.check
         g = s.graph
         CE, L, Lw, C_, dim = self.CE, self.L, self.Lw, self.C, self.dim
@@ -430,6 +505,65 @@ class DeformerTrainer:
                                   self.lr, b1, b2, self.eps, self.wd, 1.0, P(self.step_count), stream_ptr),
                 "gad_adam_step")
 
+    def _issue_glob(self, s: _Slot, stream_ptr: int, with_optimizer: bool, stage: str):
+        """The step of a slot with global CNN features: CNN forward -> bias offset du -> deformer forward with du ->
+        mesh loss -> deformer backward with du -> weight gradients -> adjoint of du (CNN cotangents and the du terms of
+        gWq / gWk) -> CNN backward into the flat gradient -> [all-reduce] -> Adam over the whole flat vector."""
+        lib, P, chk = self.lib, _lib.ptr, _lib.check
+        g, m = s.graph, self.model
+        CE, L, Lw, C_, dim, B = self.CE, self.L, self.Lw, self.C, self.dim, s.B
+        inv_temp = m.inv_temp
+        used = [r for r in self.cnn if r["used"]]
+        src = {"f": s.f, "uu": s.uu}
+        H, W = s.cnn_hw
+        g_f, g_uu = s.cnn_out.get("f"), s.cnn_out.get("uu")
+        glob = (B, used[0]["Co"], self.n_g, P(self.Wq), P(self.Wk), Lw, C_, m.z_dim, m.live, CE, inv_temp)
+        if stage in ("all", "pre"):
+            chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
+                "gad_prepare_weights")
+            for r in used:
+                u, scale = src[r["name"]], s.cnn_scale[r["name"]]
+                chk(lib.gad_absmax(P(u), u.numel(), P(scale), stream_ptr), "gad_absmax")
+                if self.world > 1 and self.loopback is None:       # the CNN normalises by the max over the GLOBAL batch
+                    dist.all_reduce(scale, op=dist.ReduceOp.MAX, group=self.pg)
+                chk(lib.gad_cnn_fwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"], r["bp"],
+                                    P(s.cnn_out[r["name"]]), P(s.cnn_ws), s.cnn_ws_bytes, stream_ptr), "gad_cnn_fwd")
+            chk(lib.gad_glob_bias_fwd(P(g_f), P(g_uu), *glob, P(s.du), stream_ptr), "gad_glob_bias_fwd")
+            # node features as GNN.forward feeds them (identity encoder: channels beyond CE are dropped)
+            f = s.f if self.opt["gnn_inc_feat_f"] and dim < CE else None
+            uu = s.uu if self.opt["gnn_inc_feat_uu"] and dim + (1 if f is not None else 0) < CE else None
+            chk(lib.gad_deform_fwd_ell_raw(P(g.ell_in), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes, g.ell_deg,
+                                           P(s.x_comp), P(f), P(uu), None, None, dim, CE, P(self.Mu), P(s.du), Lw,
+                                           P(self.tau), L, self.method, P(s.x_phys), P(s.states), stream_ptr),
+                "gad_deform_fwd_ell_raw")
+            chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, 0 if self.loss_kind == "l1" else 1,
+                                  dp.local_grad_scale(s.N * dim, s.count_global, world=self.world), P(s.loss), P(s.g_out),
+                                  P(s.loss_ws), stream_ptr), "gad_mesh_loss")
+            if self.method == GF.METHOD_RK4:
+                chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
+                                               g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), P(s.du), Lw,
+                                               P(self.tau), L, P(self.gMu), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
+                    "gad_deform_bwd_ell_rk4")
+            else:
+                chk(lib.gad_deform_bwd_ell(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
+                                           g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), P(s.du), Lw, P(self.tau),
+                                           L, P(self.gMu), P(self.gtau), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
+                    "gad_deform_bwd_ell")
+            chk(lib.gad_weight_grads(P(self.Wq), P(self.bq), P(self.Wk), P(self.gMu), Lw, C_, CE, inv_temp, P(self.gWq),
+                                     P(self.gbq), P(self.gWk), P(self.gbk), stream_ptr), "gad_weight_grads")
+            chk(lib.gad_glob_bias_bwd(P(g_f), P(g_uu), *glob, P(s.bwd_ws), s.bwd_ws_bytes, P(s.cnn_gout.get("f")),
+                                      P(s.cnn_gout.get("uu")), P(self.gWq), P(self.gWk), stream_ptr), "gad_glob_bias_bwd")
+            for r in used:
+                u, scale = src[r["name"]], s.cnn_scale[r["name"]]
+                chk(lib.gad_cnn_bwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"], r["bp"],
+                                    P(s.cnn_gout[r["name"]]), P(r["g"]), P(s.cnn_ws), s.cnn_ws_bytes, stream_ptr),
+                    "gad_cnn_bwd")
+        if stage in ("all", "post") and with_optimizer:
+            b1, b2 = self.betas
+            chk(lib.gad_adam_step(P(self.flat), P(self.gflat), P(self.exp_avg), P(self.exp_avg_sq), self.flat.numel(),
+                                  self.lr, b1, b2, self.eps, self.wd, 1.0, P(self.step_count), stream_ptr),
+                "gad_adam_step")
+
     def _allreduce(self, s: Optional[_Slot] = None):
         """NCCL all-reduce of the flat gradient -- unless the train kernel of this slot does the
         exchange itself over peer memory (fused_dp on the one-launch path)."""
@@ -444,13 +578,13 @@ class DeformerTrainer:
         """The step of this slot is the one-launch kernel k_ell_train (gad_train_step_ell / _rk4)."""
         g = s.graph
         tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
-        return bool(tiles and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
+        return bool(tiles and not s.glob and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
                     and (self.method == GF.METHOD_EULER or s.rk4_fused))
 
     def _cluster(self, s: _Slot) -> bool:
         """Meshes too large for one CTA run on the cluster-resident kernel (csrc/cl_kernels.cu, Euler only)."""
         g = s.graph
-        if not (self.method == GF.METHOD_EULER and g.tile_ptr is None and g.cl_in is not None
+        if not (self.method == GF.METHOD_EULER and not s.glob and g.tile_ptr is None and g.cl_in is not None
                 and not self.opt.get("gad_no_cluster", False) and not self.opt.get("gad_force_stream", False)):
             return False
         if s.prefer_stream is None:      # one or two very large meshes: the streaming chain uses all SMs
@@ -692,7 +826,8 @@ class DeformerTrainer:
         cs, ms = self._copy_stream, self.stream
         packed = all(torch.is_tensor(b) and (b.is_pinned() or getattr(b, "_gad_pinned", False)) and b.dtype == torch.float32
                      for b in host_batches)
-        pure = all(self._one_launch(s) for s in self.slots)      # the step's graph holds library kernels only
+        # the step's graph holds library kernels only (a slot with global features, single GPU: a chain of them)
+        pure = all(self._one_launch(s) or (s.glob and self.world == 1) for s in self.slots)
         if native is None:
             native = self.use_graph and packed and pure
         if native:

@@ -472,6 +472,22 @@ int gad_cnn_fwd(const float* u, const int32_t* gather, const float* scale, int B
 int gad_cnn_bwd(const float* u, const int32_t* gather, const float* scale, int B, int H, int W, int Cm, int Co, int L,
                 const float* const* weights, const float* const* biases, const float* g_out, float* g_params,
                 void* workspace, size_t workspace_bytes, void* stream);
+/* The CNN outputs as the per-mesh bias offset `du` of the deformer kernels, and its adjoint (training with global
+ * features).  g = cat[g_f | g_uu][:, :n_g] (g_f / g_uu [B, Co], either may be NULL) are the global channels the identity
+ * encoder keeps, z0 the node-varying input channels before them, c = log2(e) * inv_temp / sqrt(C):
+ *     du[b, lw, z] = c * sum_g (Wq[lw]^T Wk[lw])[z0 + g, z] * g[b, g]   for z < live, 0 for live <= z < CE.
+ * gad_glob_bias_bwd reads G_b = d loss / d du_b from `workspace`, the workspace of the deformer's backward
+ * (gad_deform_bwd_ell / gad_deform_bwd_ell_rk4 on one mesh per tile, T = B), writes d loss / d g into g_out_f / g_out_uu
+ * [B, Co] (zero for outputs beyond n_g; the input of gad_cnn_bwd) and ADDS the du terms to gWq / gWk [Lw, C, C].  The
+ * sums over meshes run in fp64 in mesh order.  Limits: n_g <= 32 and at most Co per given output, z0 + n_g <= C,
+ * live <= CE <= 8, Lw <= 16. */
+int gad_glob_bias_fwd(const float* g_f, const float* g_uu, int B, int Co, int n_g, const float* Wq, const float* Wk, int Lw,
+                      int C, int z0, int live, int CE, float inv_temp, float* du, void* stream);
+int gad_glob_bias_bwd(const float* g_f, const float* g_uu, int B, int Co, int n_g, const float* Wq, const float* Wk, int Lw,
+                      int C, int z0, int live, int CE, float inv_temp, const void* workspace, size_t workspace_bytes,
+                      float* g_out_f, float* g_out_uu, float* gWq, float* gWk, void* stream);
+/* out[0] = max |u[i]| over n values (the CNN's normalisation, `scale` of gad_cnn_fwd), on the device. */
+int gad_absmax(const float* u, int64_t n, float* out, void* stream);
 
 /* ---- host side of the end-to-end training loop ------------------------------------------------------
  * The reference's `for data in loader: ... loss.backward(); optimizer.step()` (src/run_GNN.py:95-131) with
