@@ -345,24 +345,63 @@ class GNN(nn.Module):
             # src/GNN.py:307-342 (dim == 1): per mesh torch_FEM_1D on its relocated points -> one batched launch.
             # Returns (coeffs_batched [B*(n-2), 1], x_phys_batched [N], sol_batched [B*Q]) like the reference.
             from . import fem1d
-            B = len(graph.mesh_sizes) if graph.mesh_sizes is not None else int(data.batch.max().item()) + 1
-            n = int(x_phys.shape[0]) // B
-            if graph.mesh_sizes is not None and any(m != n for m in graph.mesh_sizes):
-                raise NotImplementedError("pde_loss needs meshes of equal size in a batch")
-            # the Gaussian parameters of a batch object do not change between epochs: converted once per object
-            # (the entry keeps the dict alive, so its id cannot be recycled while it is cached)
-            cache = self.__dict__.setdefault("_pde_cache", {})
-            hit = cache.get(id(data.pde_params))
-            if hit is None or hit[0] is not data.pde_params or hit[1].shape[0] != B:
-                if len(cache) >= 64:
-                    cache.clear()
-                hit = (data.pde_params,) + fem1d._pde_params_to_tensors(data.pde_params, B, dev)
-                cache[id(data.pde_params)] = hit
-            centers, scales = hit[1], hit[2]
+            B, n = self._pde_batch_shape(data, graph, int(x_phys.shape[0]))
+            centers, scales = self._pde_gaussians(data, B, dev)
+            (quad,), _ = self._pde_eval_points(dev)
             xp = x_phys.squeeze(-1)
-            coeffs, sol = fem1d.fem1d_solve(xp, centers, scales, self.quad_points, n, int(opt.get("load_quad_points", 101)))
+            coeffs, sol = fem1d.fem1d_solve(xp, centers, scales, quad, n, int(opt.get("load_quad_points", 101)))
             return coeffs, xp, sol
         return x_phys
+
+    # ------------------------------------------------------------------------------------
+    # set-up of loss_type='pde_loss', shared by the module's FEM tail and DeformerTrainer's pde slots
+    @staticmethod
+    def _pde_batch_shape(data, graph, num_nodes: int):
+        """(B, nodes per mesh) of a pde_loss batch; the batched FEM kernels need meshes of one size."""
+        B = len(graph.mesh_sizes) if graph.mesh_sizes is not None else int(data.batch.max().item()) + 1
+        n = num_nodes // B
+        if graph.mesh_sizes is not None and any(m != n for m in graph.mesh_sizes):
+            raise NotImplementedError("pde_loss needs meshes of equal size in a batch")
+        return B, n
+
+    def _pde_gaussians(self, data, B: int, dev):
+        """(centers, scales) of `data.pde_params` as the FEM kernels take them: 1-D fp32 [B, G], 2-D fp64 [B, G, 2].
+        The Gaussian parameters of a batch object do not change between epochs: converted once per object (the entry
+        keeps the dict alive, so its id cannot be recycled while it is cached)."""
+        cache = self.__dict__.setdefault("_pde_cache", {})
+        hit = cache.get(id(data.pde_params))
+        if hit is None or hit[0] is not data.pde_params or hit[1].shape[0] != B:
+            if len(cache) >= 64:
+                cache.clear()
+            hit = (data.pde_params,) + self._pde_params_to_tensors(data.pde_params, B, dev)
+            cache[id(data.pde_params)] = hit
+        return hit[1], hit[2]
+
+    def _pde_params_to_tensors(self, pde_params, B: int, dev) -> tuple:
+        """`pde_params` -> (centers, scales) in the FEM kernels' layout and precision, uncached."""
+        from . import fem1d, fem2d
+        to_tensors = fem2d.pde_params_to_tensors if self.dim == 2 else fem1d._pde_params_to_tensors
+        return to_tensors(pde_params, B, dev)
+
+    def _pde_eval_points(self, dev):
+        """Where the FEM solution is evaluated, and the order the loss reads it in (cached on the device):
+        1-D ((quad [Q],), None); 2-D ((X [Q*Q], Y [Q*Q]), order [Q*Q] int64).  2-D `order` is
+        argsort(mapping_tensor_fine): `reshape_grid_to_fd_tensor(sol.view(-1).unsqueeze(-1), mapping_tensor_fine)`
+        (utils_data.py:143-159) is `sol.view(-1)[order]` for this call shape."""
+        ev = self.__dict__.get("_pde_eval")
+        if ev is None or ev[0][0].device != dev:
+            if self.dim == 2:
+                X, Y = self.quad_points
+                mapping = getattr(self.dataset, "mapping_tensor_fine", None)
+                if mapping is None:
+                    raise ValueError("loss_type='pde_loss' on 2-D meshes needs dataset.mapping_tensor_fine (src/GNN.py:333)")
+                _, order = torch.sort(torch.as_tensor(mapping).reshape(-1))           # utils_data.py:154
+                ev = ((X.reshape(-1).to(dev, torch.float32).contiguous(), Y.reshape(-1).to(dev, torch.float32).contiguous()),
+                      order.to(dev))
+            else:
+                ev = ((self.quad_points.to(dev, torch.float32).contiguous(),), None)
+            self.__dict__["_pde_eval"] = ev
+        return ev
 
     # ------------------------------------------------------------------------------------
     def _global_bias_offsets(self, data, graph, f, uu, f_scale, uu_scale, dev):
@@ -450,33 +489,13 @@ class GNN(nn.Module):
         `sol.view(-1)[argsort(mapping_tensor_fine)]`).  Here: ONE batched launch (csrc/fem2d.cu) + one gather.
         Returns (coeffs [B*n*n, 1], x_phys [B*n*n, 2], sol [B*Q*Q]) like the reference."""
         from . import fem2d
-        opt = self.opt
-        B = len(graph.mesh_sizes) if graph.mesh_sizes is not None else int(data.batch.max().item()) + 1
-        Nm = int(x_phys.shape[0]) // B
-        if graph.mesh_sizes is not None and any(m != Nm for m in graph.mesh_sizes):
-            raise NotImplementedError("pde_loss needs meshes of equal size in a batch")
+        B, Nm = self._pde_batch_shape(data, graph, int(x_phys.shape[0]))
         topo = self._fem2d_topology(dev, Nm)
-        cache = self.__dict__.setdefault("_pde_cache", {})
-        hit = cache.get(id(data.pde_params))
-        if hit is None or hit[0] is not data.pde_params or hit[1].shape[0] != B:
-            if len(cache) >= 64:
-                cache.clear()
-            hit = (data.pde_params,) + fem2d.pde_params_to_tensors(data.pde_params, B, dev)
-            cache[id(data.pde_params)] = hit
-        centers, scales = hit[1], hit[2]
-        ev = self.__dict__.get("_fem2d_eval")
-        if ev is None or ev[0].device != dev:
-            X, Y = self.quad_points
-            mapping = getattr(self.dataset, "mapping_tensor_fine", None)
-            if mapping is None:
-                raise ValueError("loss_type='pde_loss' on 2-D meshes needs dataset.mapping_tensor_fine (src/GNN.py:333)")
-            _, order = torch.sort(torch.as_tensor(mapping).reshape(-1))           # utils_data.py:154
-            ev = (X.reshape(-1).to(dev, torch.float32).contiguous(), Y.reshape(-1).to(dev, torch.float32).contiguous(),
-                  order.to(dev))
-            self.__dict__["_fem2d_eval"] = ev
-        sol, coeffs, _ = fem2d.fem2d_solve(x_phys.view(B, Nm, 2), topo, centers, scales, ev[0], ev[1],
-                                           int(opt.get("load_quad_points", 101)))
-        sol_fd = sol.index_select(1, ev[2])
+        centers, scales = self._pde_gaussians(data, B, dev)
+        (ex, ey), order = self._pde_eval_points(dev)
+        sol, coeffs, _ = fem2d.fem2d_solve(x_phys.view(B, Nm, 2), topo, centers, scales, ex, ey,
+                                           int(self.opt.get("load_quad_points", 101)))
+        sol_fd = sol.index_select(1, order)
         return coeffs.reshape(B * Nm, 1), x_phys, sol_fd.reshape(-1)
 
     def inference_session(self, data) -> "InferenceSession":

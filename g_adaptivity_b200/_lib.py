@@ -108,6 +108,8 @@ SIGNATURES = {
     "gad_conv_bwd": (_i, [_p, _p, _p, _p, _i64, _i64, _p, _p, _i, _p, _p, _p, _p, _sz, _p]),
     "gad_mesh_loss": (_i, [_p, _p, _i64, _i, _f, _p, _p, _p, _p]),
     "gad_mesh_loss_workspace_bytes": (_sz, [_i64]),
+    "gad_pde_loss": (_i, [_p, _p, _p, _i, _i, _f, _p, _p, _p, _p]),
+    "gad_pde_loss_workspace_bytes": (_sz, [_i, _i]),
     "gad_adam_step": (_i, [_p, _p, _p, _p, _i64, _f, _f, _f, _f, _f, _f, _p, _p]),
     "gad_fem1d_fwd": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _p]),
     "gad_fem1d_bwd": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p]),

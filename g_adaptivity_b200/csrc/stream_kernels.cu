@@ -197,22 +197,46 @@ __global__ void k_reduce_partials(const float* __restrict__ partials, int rows, 
 }
 
 // ---- mesh loss + cotangent (run_GNN.py:80-84,103-106) ---------------------------------------
-__global__ void __launch_bounds__(TB) k_loss(const float* __restrict__ out, const float* __restrict__ target,
-                                             int64_t count, int kind, float grad_scale, float* __restrict__ g_out,
-                                             float* __restrict__ partials) {
+// Per-block partial sums of |d| or d^2, d = out[j] - target[i], and the cotangent at out[j].  Without an index map
+// j = i.  With one (kOrder, the pde loss) entry i = b * Q + q of `target` pairs with j = b * Q + order[q]: the FEM
+// solution stays in evaluation-grid order and the target is in the fine mesh's node order (src/GNN.py:333).
+template <bool kOrder>
+__device__ __forceinline__ void loss_partials(const float* __restrict__ out, const float* __restrict__ target,
+                                              int64_t count, int kind, float grad_scale, float* __restrict__ g_out,
+                                              float* __restrict__ partials, const int32_t* __restrict__ order,
+                                              int64_t Q) {
     __shared__ float red[TB / 32];
     float acc[1] = {0.f};
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x) {
-        const float d = out[i] - target[i];
+        int64_t j = i;
+        if (kOrder) {
+            const int64_t b = i / Q;
+            j = b * Q + order[i - b * Q];
+        }
+        const float d = out[j] - target[i];
         if (kind == 0) {
             acc[0] += fabsf(d);
-            if (g_out) g_out[i] = (d > 0.f ? grad_scale : (d < 0.f ? -grad_scale : 0.f));
+            if (g_out) g_out[j] = (d > 0.f ? grad_scale : (d < 0.f ? -grad_scale : 0.f));
         } else {
             acc[0] = fmaf(d, d, acc[0]);
-            if (g_out) g_out[i] = 2.f * d * grad_scale;
+            if (g_out) g_out[j] = 2.f * d * grad_scale;
         }
     }
     block_reduce<1>(acc, red, partials + blockIdx.x);
+}
+
+__global__ void __launch_bounds__(TB) k_loss(const float* __restrict__ out, const float* __restrict__ target,
+                                             int64_t count, int kind, float grad_scale, float* __restrict__ g_out,
+                                             float* __restrict__ partials) {
+    loss_partials<false>(out, target, count, kind, grad_scale, g_out, partials, nullptr, 1);
+}
+
+// squared error through the index map (gad_pde_loss)
+__global__ void __launch_bounds__(TB) k_loss_ordered(const float* __restrict__ out, const int32_t* __restrict__ order,
+                                                     const float* __restrict__ target, int64_t count, int64_t Q,
+                                                     float grad_scale, float* __restrict__ g_out,
+                                                     float* __restrict__ partials) {
+    loss_partials<true>(out, target, count, 1, grad_scale, g_out, partials, order, Q);
 }
 
 __global__ void k_loss_final(const float* __restrict__ partials, int rows, float inv_count, float* __restrict__ loss) {
@@ -422,6 +446,33 @@ extern "C" int gad_mesh_loss(const float* out, const float* target, int64_t coun
     const int G = (int)(want < (int64_t)sm_count() * 8 ? want : (int64_t)sm_count() * 8);
     float* partials = reinterpret_cast<float*>(workspace);
     k_loss<<<G, TB, 0, st>>>(out, target, count, kind, grad_scale, g_out, partials);
+    GAD_LAUNCH_CHECK();
+    k_loss_final<<<1, 32, 0, st>>>(partials, G, 1.0f / (float)count, loss);
+    GAD_LAUNCH_CHECK();
+    return GAD_OK;
+}
+
+extern "C" size_t gad_pde_loss_workspace_bytes(int B, int Q) {
+    return gad_mesh_loss_workspace_bytes((int64_t)B * Q);
+}
+
+extern "C" int gad_pde_loss(const float* sol, const int32_t* order, const float* target, int B, int Q, float grad_scale,
+                            float* loss, float* g_sol, void* workspace, void* stream) {
+    GAD_CHECK_ARG(sol && target && loss && workspace, "gad_pde_loss: sol, target, loss and workspace must not be NULL");
+    GAD_CHECK_ARG(B > 0 && Q > 0, "gad_pde_loss: B=%d and Q=%d must be positive", B, Q);
+    GAD_CHECK_ARG(isfinite(grad_scale), "gad_pde_loss: grad_scale must be finite");
+    cudaStream_t st = as_stream(stream);
+    const int64_t count = (int64_t)B * Q;
+    const int64_t want = (count + TB - 1) / TB;
+    const int G = (int)(want < (int64_t)sm_count() * 8 ? want : (int64_t)sm_count() * 8);
+    float* partials = reinterpret_cast<float*>(workspace);
+    // the shared squared-error branch writes 2 * d * s; with s = grad_scale / 2 (exact: a power-of-two scaling) that
+    // is d * grad_scale rounded once, i.e. what torch's mse_loss backward writes with grad_scale = 2 / numel
+    const float half = 0.5f * grad_scale;
+    if (order)
+        k_loss_ordered<<<G, TB, 0, st>>>(sol, order, target, count, Q, half, g_sol, partials);
+    else
+        k_loss<<<G, TB, 0, st>>>(sol, target, count, 1, half, g_sol, partials);
     GAD_LAUNCH_CHECK();
     k_loss_final<<<1, 32, 0, st>>>(partials, G, 1.0f / (float)count, loss);
     GAD_LAUNCH_CHECK();

@@ -21,7 +21,16 @@ gradients, Adam.  The step sizes get no gradient through RK4, so `learn_step` is
 
 Global CNN features (`gnn_inc_glob_feat_f / _uu` with channels that survive the encoder) train as a chain of library
 kernels: CNN forward, the per-mesh bias offset du (csrc/glob_train.cu), the mesh-resident forward and backward with du,
-the adjoint of du, CNN backward into the flat gradient, Adam over Linear and CNN parameters (`_issue_glob`).
+the adjoint of du, CNN backward into the flat gradient, Adam over Linear and CNN parameters (`_issue_chain`).
+
+`loss_type='pde_loss'` (the reference's Poisson preset, src/run_GNN.py:109-110: mse(FEM solution on the deformed mesh,
+u_true_fine)) trains through the same chain with the loss stage FEM forward (gad_fem1d_fwd / gad_fem2d_fwd) ->
+gad_pde_loss -> FEM backward, the kernels GNN.forward + autograd run for that loss, so a step reproduces the module
+path's gradient bit for bit (in 2-D up to the last bit of the FEM backward, whose fp64 shared-memory atomics leave the
+order of its sums open).  u_true_fine and the Gaussians of the right-hand side are segments of the slot's input
+buffer.  Such slots need meshes of equal size on the mesh-resident ELL kernels and what the FEM kernels accept (2-D: up to
+38 x 38, at most 16 Gaussians and 16 cells per vertex); `add_batch` raises otherwise.  An explicit `loss_fn` trains
+the mesh loss instead.
 
 Sharding (SURVEY 8e): a batch is a disjoint union of meshes, so ranks take contiguous shards of
 whole meshes with no data-path collective; the only exchange is the all-reduce of the flat
@@ -36,6 +45,7 @@ kernels, the all-reduce and Adam all work on contiguous memory and `model.state_
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Dict, List, Optional
 
 import torch
@@ -69,11 +79,14 @@ class DeformerTrainer:
         self.betas, self.eps = betas, eps
         # Options GNN.forward and the reference training loop honour but this fused step does not implement
         # raise instead of silently training something else (src/run_GNN.py:80-88,109-131; src/GNN.py:231-237).
-        if loss_fn is None and opt.get("loss_type", "mesh_loss") != "mesh_loss":
+        loss_type = opt.get("loss_type", "mesh_loss")
+        if loss_fn is None and loss_type not in ("mesh_loss", "pde_loss"):
             raise NotImplementedError(
-                f"DeformerTrainer fuses the mesh loss (loss_type='mesh_loss', src/run_GNN.py:105-107); opt['loss_type']="
+                f"DeformerTrainer trains the mesh loss and the pde loss (src/run_GNN.py:105-110); opt['loss_type']="
                 f"{opt['loss_type']!r} trains through GNN.forward + autograd instead.  Pass loss_fn='l1' / 'mse' explicitly "
                 "to train the mesh loss on such a preset")
+        # loss_type='pde_loss': mse(FEM solution on the deformed mesh, u_true_fine), unless loss_fn asks for the mesh loss
+        self.pde = loss_fn is None and loss_type == "pde_loss"
         if opt.get("softmax_temp_type") == "learnable_a":
             raise NotImplementedError("DeformerTrainer: the learnable temperature is trained through GNN.forward + autograd")
         if opt.get("gnn_normalize", False):
@@ -82,8 +95,8 @@ class DeformerTrainer:
         if opt.get("gnn_dont_train", False):
             raise NotImplementedError("DeformerTrainer: gnn_dont_train=True skips the optimizer step (src/run_GNN.py:122-131); "
                                       "evaluate with GNN.forward instead")
-        self.loss_kind = (opt.get("loss_fn", "l1") if loss_fn is None else loss_fn)
-        if self.loss_kind not in ("l1", "mse"):
+        self.loss_kind = "pde" if self.pde else (opt.get("loss_fn", "l1") if loss_fn is None else loss_fn)
+        if not self.pde and self.loss_kind not in ("l1", "mse"):
             raise NotImplementedError(f"DeformerTrainer: loss_fn={self.loss_kind!r} (the reference has 'l1' and 'mse', "
                                       "src/run_GNN.py:80-84)")
         self.pg = process_group
@@ -254,33 +267,46 @@ class DeformerTrainer:
             N = s.graph.N
             s.N = N
             s.glob = bool(self.n_g)
+            s.pde = self.pde
+            s.du = None
             if s.glob:
                 self._check_glob_graph(s.graph)
+            if s.pde:
+                self._pde_setup(s, data)
             f32 = dict(dtype=torch.float32, device=dev)
-            xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
             # node inputs of a step live in ONE device buffer [target | f | uu | x_comp] (segments padded to
             # 16 bytes, the TMA staging granularity), so that a packed host batch travels in one copy.  x_comp
             # comes last: datasets on one shared mesh (`randg`, src/data.py:143: every sample has the same
             # computational mesh) send it once, and a step's copy is the [target | f | uu] prefix only.
-            # the global feature extractors read f / uu from the same buffer
+            # the global feature extractors read f / uu from the same buffer.  A pde slot's target is u_true_fine,
+            # followed by the Gaussians of the right-hand side: [u_true_fine | centers | scales | f | uu | x_comp].
             has_f = bool(self.opt["gnn_inc_feat_f"]) or any(r["name"] == "f" and r["used"] for r in self.cnn)
             has_uu = bool(self.opt["gnn_inc_feat_uu"]) or any(r["name"] == "uu" and r["used"] for r in self.cnn)
-            seg = [N * self.dim, N if has_f else 0, N if has_uu else 0, N * self.dim]
+            segs = [("target", (N, self.dim), torch.float32)]
+            if s.pde:
+                segs = [("target", (s.B * s.Q,), torch.float32), ("centers", s.gauss_shape, s.gauss_dtype),
+                        ("scales", s.gauss_shape, s.gauss_dtype)]
+            segs += [("f", (N if has_f else 0,), torch.float32), ("uu", (N if has_uu else 0,), torch.float32),
+                     ("x_comp", (N, self.dim), torch.float32)]
+            seg = [math.prod(shape) * (2 if dt == torch.float64 else 1) for _, shape, dt in segs]     # fp32 words
             offs, o = [], 0
             for n in seg:
                 offs.append(o)
                 o += (n + 3) // 4 * 4
             s.in_offs, s.in_sizes = offs, seg
             s.inbuf = torch.zeros(o, **f32)
-            s.target = s.inbuf[offs[0]:offs[0] + seg[0]].view(N, self.dim)
-            s.f = s.inbuf[offs[1]:offs[1] + seg[1]] if has_f else None
-            s.uu = s.inbuf[offs[2]:offs[2] + seg[2]] if has_uu else None
-            s.x_comp = s.inbuf[offs[3]:offs[3] + seg[3]].view(N, self.dim)
+            # typed views of the segments, in buffer order (host parts of a batch: _input_parts)
+            s.in_views = [s.inbuf[off:off + n].view(dt).view(shape)
+                          for off, n, (_, shape, dt) in zip(offs, seg, segs)]
+            views = {name: (v if n else None) for (name, _, _), n, v in zip(segs, seg, s.in_views)}
+            s.target, s.f, s.uu, s.x_comp = views["target"], views["f"], views["uu"], views["x_comp"]
+            s.centers, s.scales = views.get("centers"), views.get("scales")
             s.states = torch.empty((self.L, N, self.CE), **f32)
             s.x_phys = torch.empty((N, self.dim), **f32)
             s.g_out = torch.empty((N, self.dim), **f32)
             s.loss = torch.zeros(1, **f32)
-            s.loss_ws = torch.empty(lib.gad_mesh_loss_workspace_bytes(N * self.dim), dtype=torch.uint8, device=dev)
+            ws = lib.gad_pde_loss_workspace_bytes(s.B, s.Q) if s.pde else lib.gad_mesh_loss_workspace_bytes(N * self.dim)
+            s.loss_ws = torch.empty(ws, dtype=torch.uint8, device=dev)
             T = s.graph.T if s.graph.tile_ptr is not None else 0
             s.bwd_ws_bytes = max(lib.gad_deform_bwd_workspace_bytes(N, self.CE, T, self.L),
                                  lib.gad_ell_workspace_bytes(self.CE, T, self.L))
@@ -310,7 +336,10 @@ class DeformerTrainer:
                 self._add_glob_buffers(s, data)
             s.fwd_ws_bytes = lib.gad_deform_workspace_bytes(N, self.CE, self.method) if streaming else 0
             s.fwd_ws = torch.empty(max(s.fwd_ws_bytes, 16), dtype=torch.uint8, device=dev)
-            s.h2d_bytes = 0
+            with torch.cuda.stream(self.stream):
+                s.h2d_bytes = self._copy_inputs(s, data)
+            if s.pde:
+                self._pde_check(s)
             # Data parallel: add_batch is COLLECTIVE (every rank adds its shard of the same global batch, in the
             # same order).  Two things are agreed here, once per slot and outside any capture:
             #  * the mean of the loss is over the nodes of the GLOBAL batch (F.l1_loss on the whole batch,
@@ -318,21 +347,21 @@ class DeformerTrainer:
             #  * the gradient route.  Whether a rank can run the one-launch kernel (whose tail all-reduces over
             #    peer memory) depends on ITS shard (degree, mesh sizes, policy); a rank spinning in the peer
             #    exchange while another calls NCCL would hang both, so the route is the MIN over the ranks.
-            s.count_global = N * self.dim
+            #  A pde slot's mean is over the B * Q solution values of the global batch.
+            count = s.B * s.Q if s.pde else N * self.dim
+            s.count_global = count
             s.peer_route = False
             if self.loopback is not None:
-                s.count_global, s.peer_route = N * self.dim * self.world, bool(self._one_launch_local(s))
+                s.count_global, s.peer_route = count * self.world, bool(self._one_launch_local(s))
             elif self.world > 1:
                 mine = 1 if (self.fused_dp and self._one_launch_local(s)) else 0
-                t = torch.tensor([N * self.dim, 1 - mine], dtype=torch.int64, device=dev)
+                t = torch.tensor([count, 1 - mine], dtype=torch.int64, device=dev)
                 dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.pg)
                 t = t.cpu()
                 s.count_global = int(t[0])
                 s.peer_route = bool(int(t[1]) == 0)
         self.slots.append(s)
-        sid = len(self.slots) - 1
-        self.load_inputs(sid, data)
-        return sid
+        return len(self.slots) - 1
 
     def _check_glob_graph(self, g):
         """A batch with global CNN features runs on the mesh-resident ELL kernels, one mesh per tile (GNN.forward's
@@ -343,6 +372,42 @@ class DeformerTrainer:
         if self.method == GF.METHOD_RK4 and not GF.rk4_backward_resident(g, self.CE):
             raise NotImplementedError("global CNN features reach the kernels as a per-tile bias offset: meshes that fit "
                                       "a CTA only (backward through ode_method='rk4' on the streaming kernels has none)")
+
+    def _pde_setup(self, s: "_Slot", data):
+        """Refusals, FEM tables and buffers of a pde slot (loss_type='pde_loss'), from the helpers GNN.forward uses."""
+        m, g, dev = self.model, s.graph, self.dev
+        if self.opt.get("gad_force_stream", False) or not GF.use_ell(g, self.CE):
+            raise NotImplementedError("pde_loss training runs on the mesh-resident ELL kernels (meshes that fit a CTA, "
+                                      "bounded degree); train this batch through GNN.forward + autograd")
+        s.B, s.Nm = m._pde_batch_shape(data, g, s.N)
+        if getattr(data, "u_true_fine_tensor", None) is None or getattr(data, "pde_params", None) is None:
+            raise ValueError("loss_type='pde_loss' needs data.u_true_fine_tensor and data.pde_params (src/run_GNN.py:109-110)")
+        s.topo = m._fem2d_topology(dev, s.Nm) if self.dim == 2 else None
+        s.eval_pts, order = m._pde_eval_points(dev)
+        s.order = None if order is None else order.to(torch.int32)
+        s.Q = int(s.eval_pts[0].numel())
+        if data.u_true_fine_tensor.numel() != s.B * s.Q:
+            raise ValueError(f"u_true_fine_tensor has {data.u_true_fine_tensor.numel()} entries; the FEM solution of "
+                             f"{s.B} meshes at {s.Q} evaluation points has {s.B * s.Q}")
+        centers, _ = m._pde_params_to_tensors(data.pde_params, s.B, "cpu")
+        s.gauss_shape, s.gauss_dtype, s.G = tuple(centers.shape), centers.dtype, int(centers.shape[1])
+        s.K = int(self.opt.get("load_quad_points", 101))
+        s.count_global = s.B * s.Q
+        f32 = dict(dtype=torch.float32, device=dev)
+        s.sol = torch.zeros((s.B, s.Q), **f32)
+        s.g_sol = torch.zeros((s.B, s.Q), **f32)
+        if self.dim == 2:
+            s.coeffs = torch.zeros((s.B, s.Nm), **f32)
+            s.u64 = torch.zeros((s.B, s.Nm), dtype=torch.float64, device=dev)
+            s.cg_iters = torch.zeros(s.B, dtype=torch.int32, device=dev)
+
+    def _pde_check(self, s: "_Slot"):
+        """Run the loss stage of a pde slot once, eagerly, on the computational meshes: the FEM kernels refuse what
+        they cannot solve (2-D meshes beyond 38 x 38, more than 16 Gaussians, a vertex in more than 16 cells) here,
+        before any capture, rather than inside a CUDA graph."""
+        with torch.cuda.stream(self.stream):
+            self._issue_pde_loss(s, self.stream.cuda_stream, coords=s.x_comp)
+        self.stream.synchronize()
 
     def _add_glob_buffers(self, s: "_Slot", data):
         """CNN grid map, workspace, per-mesh CNN outputs / cotangents and the bias offset of a slot."""
@@ -374,25 +439,33 @@ class DeformerTrainer:
         buf._gad_pinned = True
         return buf
 
+    def _input_parts(self, s: "_Slot", data, with_x_comp: bool = True) -> list:
+        """Host tensors of `data` for the slot's input segments, in buffer order (None: the segment is not sent)."""
+        xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
+        if s.pde:
+            first = [data.u_true_fine_tensor, *self.model._pde_params_to_tensors(data.pde_params, s.B, "cpu")]
+        else:
+            first = [data.x_phys if data.x_phys.dim() == 2 else data.x_phys.unsqueeze(-1)]
+        return first + [data.f_tensor if s.f is not None else None, data.uu_tensor if s.uu is not None else None,
+                        xc if with_x_comp else None]
+
     def pack_host(self, sid: int, data, with_x_comp: bool = True, write_combined: bool = False) -> torch.Tensor:
         """One pinned host buffer holding `data`'s node inputs in the layout of slot `sid`
-        ([target | f | uu | x_comp]): `load_inputs` / `run_from_host` then move a batch host -> device
-        with a single copy.  `with_x_comp=False` packs the per-sample prefix [target | f | uu] only, for
-        datasets whose samples share one computational mesh (the slot keeps the x_comp it was given by
-        `add_batch`; the caller asserts that it does not change -- checked here against the slot).
-        `write_combined=True`: write-combined pinned pages (written once here, read only by the device)."""
+        ([target | f | uu | x_comp]; a pde slot's target is [u_true_fine | centers | scales]): `load_inputs` /
+        `run_from_host` then move a batch host -> device with a single copy.  `with_x_comp=False` packs the
+        per-sample prefix (everything but x_comp) only, for datasets whose samples share one computational mesh
+        (the slot keeps the x_comp it was given by `add_batch`; the caller asserts that it does not change -- checked
+        here against the slot).  `write_combined=True`: write-combined pinned pages (written once here, read only by
+        the device)."""
         s = self.slots[sid]
         xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
-        tg = data.x_phys if data.x_phys.dim() == 2 else data.x_phys.unsqueeze(-1)
         if not with_x_comp and not torch.equal(xc.to(torch.float32).cpu(), s.x_comp.cpu()):
             raise ValueError("pack_host(with_x_comp=False): this batch's x_comp differs from the slot's resident one")
-        n_total = s.inbuf.numel() if with_x_comp else s.in_offs[3]
+        n_total = s.inbuf.numel() if with_x_comp else s.in_offs[-1]
         buf = self._host_buffer(n_total, write_combined)
-        parts = [tg, data.f_tensor if s.f is not None else None, data.uu_tensor if s.uu is not None else None,
-                 xc if with_x_comp else None]
-        for off, n, t in zip(s.in_offs, s.in_sizes, parts):
+        for off, n, view, t in zip(s.in_offs, s.in_sizes, s.in_views, self._input_parts(s, data, with_x_comp)):
             if t is not None and n:
-                buf[off:off + n].copy_(t.reshape(-1))
+                buf[off:off + n].view(view.dtype).copy_(t.reshape(-1))
         return buf
 
     def _copy_inputs(self, s: "_Slot", data, skip_x_comp: bool = False) -> int:
@@ -401,16 +474,11 @@ class DeformerTrainer:
         if torch.is_tensor(data):                       # packed (pack_host): one copy (whole buffer or its prefix)
             s.inbuf[:data.numel()].copy_(data, non_blocking=True)
             return data.numel() * 4
-        xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
-        tg = data.x_phys if data.x_phys.dim() == 2 else data.x_phys.unsqueeze(-1)
         nbytes = 0
-        if not skip_x_comp:
-            s.x_comp.copy_(xc, non_blocking=True); nbytes += xc.numel() * 4
-        s.target.copy_(tg, non_blocking=True); nbytes += tg.numel() * 4
-        if s.f is not None:
-            s.f.copy_(data.f_tensor, non_blocking=True); nbytes += data.f_tensor.numel() * 4
-        if s.uu is not None:
-            s.uu.copy_(data.uu_tensor, non_blocking=True); nbytes += data.uu_tensor.numel() * 4
+        for n, view, t in zip(s.in_sizes, s.in_views, self._input_parts(s, data, with_x_comp=not skip_x_comp)):
+            if t is not None and n:
+                view.copy_(t.reshape(view.shape), non_blocking=True)
+                nbytes += t.numel() * t.element_size()
         return nbytes
 
     def load_inputs(self, sid: int, data, non_blocking: bool = True):
@@ -426,8 +494,8 @@ class DeformerTrainer:
     # ------------------------------------------------------------------------------------
     def _issue(self, s: _Slot, stream_ptr: int, with_optimizer: bool = True, stage: str = "all"):
         """Enqueue the kernels of one training step on `stream_ptr` (captured or eager)."""
-        if s.glob:
-            return self._issue_glob(s, stream_ptr, with_optimizer, stage)
+        if s.glob or s.pde:
+            return self._issue_chain(s, stream_ptr, with_optimizer, stage)
         lib, P, chk = self.lib, _lib.ptr, _lib.check
         g = s.graph
         CE, L, Lw, C_, dim = self.CE, self.L, self.Lw, self.C, self.dim
@@ -505,30 +573,37 @@ class DeformerTrainer:
                                   self.lr, b1, b2, self.eps, self.wd, 1.0, P(self.step_count), stream_ptr),
                 "gad_adam_step")
 
-    def _issue_glob(self, s: _Slot, stream_ptr: int, with_optimizer: bool, stage: str):
-        """The step of a slot with global CNN features: CNN forward -> bias offset du -> deformer forward with du ->
-        mesh loss -> deformer backward with du -> weight gradients -> adjoint of du (CNN cotangents and the du terms of
-        gWq / gWk) -> CNN backward into the flat gradient -> [all-reduce] -> Adam over the whole flat vector."""
+    def _issue_chain(self, s: _Slot, stream_ptr: int, with_optimizer: bool, stage: str):
+        """The step of a slot that is not on the one-launch kernel, as a chain of library kernels on the mesh-resident
+        ELL graph (a slot with global CNN features, or a pde slot):  [CNN forward -> bias offset du] -> deformer
+        forward [with du] -> loss stage (mesh loss; or FEM forward -> pde loss -> FEM backward) -> deformer backward ->
+        weight gradients -> [adjoint of du (CNN cotangents and the du terms of gWq / gWk) -> CNN backward into the
+        flat gradient] -> [all-reduce] -> Adam over the whole flat vector.  These are the kernels GNN.forward +
+        autograd run for the same batch."""
         lib, P, chk = self.lib, _lib.ptr, _lib.check
         g, m = s.graph, self.model
-        CE, L, Lw, C_, dim, B = self.CE, self.L, self.Lw, self.C, self.dim, s.B
+        CE, L, Lw, C_, dim = self.CE, self.L, self.Lw, self.C, self.dim
         inv_temp = m.inv_temp
-        used = [r for r in self.cnn if r["used"]]
-        src = {"f": s.f, "uu": s.uu}
-        H, W = s.cnn_hw
-        g_f, g_uu = s.cnn_out.get("f"), s.cnn_out.get("uu")
-        glob = (B, used[0]["Co"], self.n_g, P(self.Wq), P(self.Wk), Lw, C_, m.z_dim, m.live, CE, inv_temp)
+        if s.glob:
+            B = s.B
+            used = [r for r in self.cnn if r["used"]]
+            src = {"f": s.f, "uu": s.uu}
+            H, W = s.cnn_hw
+            g_f, g_uu = s.cnn_out.get("f"), s.cnn_out.get("uu")
+            glob = (B, used[0]["Co"], self.n_g, P(self.Wq), P(self.Wk), Lw, C_, m.z_dim, m.live, CE, inv_temp)
         if stage in ("all", "pre"):
             chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
                 "gad_prepare_weights")
-            for r in used:
-                u, scale = src[r["name"]], s.cnn_scale[r["name"]]
-                chk(lib.gad_absmax(P(u), u.numel(), P(scale), stream_ptr), "gad_absmax")
-                if self.world > 1 and self.loopback is None:       # the CNN normalises by the max over the GLOBAL batch
-                    dist.all_reduce(scale, op=dist.ReduceOp.MAX, group=self.pg)
-                chk(lib.gad_cnn_fwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"], r["bp"],
-                                    P(s.cnn_out[r["name"]]), P(s.cnn_ws), s.cnn_ws_bytes, stream_ptr), "gad_cnn_fwd")
-            chk(lib.gad_glob_bias_fwd(P(g_f), P(g_uu), *glob, P(s.du), stream_ptr), "gad_glob_bias_fwd")
+            if s.glob:
+                for r in used:
+                    u, scale = src[r["name"]], s.cnn_scale[r["name"]]
+                    chk(lib.gad_absmax(P(u), u.numel(), P(scale), stream_ptr), "gad_absmax")
+                    if self.world > 1 and self.loopback is None:       # the CNN normalises by the max over the GLOBAL batch
+                        dist.all_reduce(scale, op=dist.ReduceOp.MAX, group=self.pg)
+                    chk(lib.gad_cnn_fwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"],
+                                        r["bp"], P(s.cnn_out[r["name"]]), P(s.cnn_ws), s.cnn_ws_bytes, stream_ptr),
+                        "gad_cnn_fwd")
+                chk(lib.gad_glob_bias_fwd(P(g_f), P(g_uu), *glob, P(s.du), stream_ptr), "gad_glob_bias_fwd")
             # node features as GNN.forward feeds them (identity encoder: channels beyond CE are dropped)
             f = s.f if self.opt["gnn_inc_feat_f"] and dim < CE else None
             uu = s.uu if self.opt["gnn_inc_feat_uu"] and dim + (1 if f is not None else 0) < CE else None
@@ -536,10 +611,17 @@ class DeformerTrainer:
                                            P(s.x_comp), P(f), P(uu), None, None, dim, CE, P(self.Mu), P(s.du), Lw,
                                            P(self.tau), L, self.method, P(s.x_phys), P(s.states), stream_ptr),
                 "gad_deform_fwd_ell_raw")
-            chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, 0 if self.loss_kind == "l1" else 1,
-                                  dp.local_grad_scale(s.N * dim, s.count_global, world=self.world), P(s.loss), P(s.g_out),
-                                  P(s.loss_ws), stream_ptr), "gad_mesh_loss")
-            if self.method == GF.METHOD_RK4:
+            if s.pde:
+                self._issue_pde_loss(s, stream_ptr)
+            else:
+                chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, 0 if self.loss_kind == "l1" else 1,
+                                      dp.local_grad_scale(s.N * dim, s.count_global, world=self.world), P(s.loss),
+                                      P(s.g_out), P(s.loss_ws), stream_ptr), "gad_mesh_loss")
+            if self.method == GF.METHOD_RK4 and not s.rk4_resident:
+                chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
+                                                dim, CE, P(self.Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
+                                                s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
+            elif self.method == GF.METHOD_RK4:
                 chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
                                                g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), P(s.du), Lw,
                                                P(self.tau), L, P(self.gMu), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
@@ -551,18 +633,42 @@ class DeformerTrainer:
                     "gad_deform_bwd_ell")
             chk(lib.gad_weight_grads(P(self.Wq), P(self.bq), P(self.Wk), P(self.gMu), Lw, C_, CE, inv_temp, P(self.gWq),
                                      P(self.gbq), P(self.gWk), P(self.gbk), stream_ptr), "gad_weight_grads")
-            chk(lib.gad_glob_bias_bwd(P(g_f), P(g_uu), *glob, P(s.bwd_ws), s.bwd_ws_bytes, P(s.cnn_gout.get("f")),
-                                      P(s.cnn_gout.get("uu")), P(self.gWq), P(self.gWk), stream_ptr), "gad_glob_bias_bwd")
-            for r in used:
-                u, scale = src[r["name"]], s.cnn_scale[r["name"]]
-                chk(lib.gad_cnn_bwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"], r["bp"],
-                                    P(s.cnn_gout[r["name"]]), P(r["g"]), P(s.cnn_ws), s.cnn_ws_bytes, stream_ptr),
-                    "gad_cnn_bwd")
+            if s.glob:
+                chk(lib.gad_glob_bias_bwd(P(g_f), P(g_uu), *glob, P(s.bwd_ws), s.bwd_ws_bytes, P(s.cnn_gout.get("f")),
+                                          P(s.cnn_gout.get("uu")), P(self.gWq), P(self.gWk), stream_ptr),
+                    "gad_glob_bias_bwd")
+                for r in used:
+                    u, scale = src[r["name"]], s.cnn_scale[r["name"]]
+                    chk(lib.gad_cnn_bwd(P(u), P(s.cnn_gather), P(scale), B, H, W, r["Cm"], r["Co"], r["L"], r["wp"],
+                                        r["bp"], P(s.cnn_gout[r["name"]]), P(r["g"]), P(s.cnn_ws), s.cnn_ws_bytes,
+                                        stream_ptr), "gad_cnn_bwd")
         if stage in ("all", "post") and with_optimizer:
             b1, b2 = self.betas
             chk(lib.gad_adam_step(P(self.flat), P(self.gflat), P(self.exp_avg), P(self.exp_avg_sq), self.flat.numel(),
                                   self.lr, b1, b2, self.eps, self.wd, 1.0, P(self.step_count), stream_ptr),
                 "gad_adam_step")
+
+    def _issue_pde_loss(self, s: _Slot, stream_ptr: int, coords: Optional[torch.Tensor] = None):
+        """Loss stage of a pde slot: FEM forward on the deformed meshes (`coords`, default the slot's x_phys) -> mean
+        squared error of the solution against u_true_fine and its cotangent (gad_pde_loss) -> FEM backward into the
+        cotangent of x_phys, s.g_out.  The kernels GNN.forward + autograd run for mse(sol, u_true_fine)."""
+        lib, P, chk = self.lib, _lib.ptr, _lib.check
+        x = s.x_phys if coords is None else coords
+        grad_scale = 2.0 / float(s.count_global)         # torch's mse_loss backward over the global batch
+        if self.dim == 2:
+            t, (ex, ey) = s.topo, s.eval_pts
+            fem = (P(t.cells), t.T, P(t.is_bc), s.Nm, P(t.star_cell), P(t.star_loc), t.D, P(x), P(s.centers),
+                   P(s.scales), s.G, s.B, s.K, P(ex), P(ey), s.Q)
+            chk(lib.gad_fem2d_fwd(*fem, P(s.coeffs), P(s.sol), P(s.u64), P(s.cg_iters), stream_ptr), "gad_fem2d_fwd")
+            chk(lib.gad_pde_loss(P(s.sol), P(s.order), P(s.target), s.B, s.Q, grad_scale, P(s.loss), P(s.g_sol),
+                                 P(s.loss_ws), stream_ptr), "gad_pde_loss")
+            chk(lib.gad_fem2d_bwd(*fem, P(s.u64), P(s.g_sol), P(s.g_out), stream_ptr), "gad_fem2d_bwd")
+        else:
+            fem = (P(x), P(s.centers), P(s.scales), P(s.eval_pts[0]))
+            chk(lib.gad_fem1d_fwd(*fem, s.B, s.Nm, s.G, s.K, s.Q, P(s.sol), None, stream_ptr), "gad_fem1d_fwd")
+            chk(lib.gad_pde_loss(P(s.sol), None, P(s.target), s.B, s.Q, grad_scale, P(s.loss), P(s.g_sol),
+                                 P(s.loss_ws), stream_ptr), "gad_pde_loss")
+            chk(lib.gad_fem1d_bwd(*fem, P(s.g_sol), s.B, s.Nm, s.G, s.K, s.Q, P(s.g_out), stream_ptr), "gad_fem1d_bwd")
 
     def _allreduce(self, s: Optional[_Slot] = None):
         """NCCL all-reduce of the flat gradient -- unless the train kernel of this slot does the
@@ -578,13 +684,13 @@ class DeformerTrainer:
         """The step of this slot is the one-launch kernel k_ell_train (gad_train_step_ell / _rk4)."""
         g = s.graph
         tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
-        return bool(tiles and not s.glob and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
+        return bool(tiles and not (s.glob or s.pde) and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
                     and (self.method == GF.METHOD_EULER or s.rk4_fused))
 
     def _cluster(self, s: _Slot) -> bool:
         """Meshes too large for one CTA run on the cluster-resident kernel (csrc/cl_kernels.cu, Euler only)."""
         g = s.graph
-        if not (self.method == GF.METHOD_EULER and not s.glob and g.tile_ptr is None and g.cl_in is not None
+        if not (self.method == GF.METHOD_EULER and not (s.glob or s.pde) and g.tile_ptr is None and g.cl_in is not None
                 and not self.opt.get("gad_no_cluster", False) and not self.opt.get("gad_force_stream", False)):
             return False
         if s.prefer_stream is None:      # one or two very large meshes: the streaming chain uses all SMs
@@ -826,8 +932,9 @@ class DeformerTrainer:
         cs, ms = self._copy_stream, self.stream
         packed = all(torch.is_tensor(b) and (b.is_pinned() or getattr(b, "_gad_pinned", False)) and b.dtype == torch.float32
                      for b in host_batches)
-        # the step's graph holds library kernels only (a slot with global features, single GPU: a chain of them)
-        pure = all(self._one_launch(s) or (s.glob and self.world == 1) for s in self.slots)
+        # the step's graph holds library kernels only (a slot with global features or a pde slot, single GPU: a chain
+        # of them)
+        pure = all(self._one_launch(s) or ((s.glob or s.pde) and self.world == 1) for s in self.slots)
         if native is None:
             native = self.use_graph and packed and pure
         if native:

@@ -396,6 +396,16 @@ int gad_mesh_loss(const float* out, const float* target, int64_t count, int kind
                   float grad_scale, float* loss, float* g_out, void* workspace, void* stream);
 size_t gad_mesh_loss_workspace_bytes(int64_t count);
 
+/* ---- pde loss seam (loss_type='pde_loss', src/run_GNN.py:109-110): mse(sol[:, order].reshape(-1), target) ----
+ * sol [B, Q] (the FEM solution in evaluation-grid order, gad_fem1d_fwd / gad_fem2d_fwd), order [Q] a permutation of
+ * 0..Q-1 or NULL (identity), target [B*Q].  loss = mean over the B*Q entries of d^2 with
+ * d = sol[b, order[q]] - target[b*Q + q]; g_sol (may be NULL) receives the cotangent in sol's own order,
+ * g_sol[b, order[q]] = d * grad_scale.  grad_scale = 2 / (B*Q) is torch's mse_loss backward (bit for bit);
+ * data parallel, 2 / (sum of B*Q over the ranks).  Fixed-order reduction, no atomics. */
+int gad_pde_loss(const float* sol, const int32_t* order, const float* target, int B, int Q, float grad_scale,
+                 float* loss, float* g_sol, void* workspace, void* stream);
+size_t gad_pde_loss_workspace_bytes(int B, int Q);
+
 /* ---- optimiser step on the flat parameter vector (run_GNN.py:88,128,131: torch.optim.Adam) ----
  * torch.optim.Adam semantics (L2 weight decay added to the gradient, bias-corrected moments).
  * `step` is a DEVICE int64 counter incremented by the kernel, so the call is CUDA-graph replayable.
