@@ -127,6 +127,9 @@ SIGNATURES = {
     "gad_glob_bias_fwd": (_i, [_p, _p, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _f, _p, _p]),
     "gad_glob_bias_bwd": (_i, [_p, _p, _i, _i, _i, _p, _p, _i, _i, _i, _i, _i, _f, _p, _sz, _p, _p, _p, _p, _p]),
     "gad_absmax": (_i, [_p, _i64, _p, _p]),
+    "gad_batch_max": (_i, [_p, _i64, _p, _p]),
+    "gad_temp_fold": (_i, [_p, _p, _i, _i, _p, _p]),
+    "gad_temp_fold_bwd": (_i, [_p, _p, _p, _i, _i, _p, _p, _p]),
     "gad_host_alloc": (_i, [_sz, _i, C.POINTER(_p)]),
     "gad_host_free": (_i, [_p]),
     "gad_pipeline_run": (_i, [C.POINTER(PipelineSlot), _i, C.POINTER(_p), _i, _i64, _p, _p, _p]),

@@ -132,6 +132,61 @@ __global__ void k_absmax(const float* __restrict__ u, int64_t n, unsigned int* _
     if ((threadIdx.x & 31) == 0) atomicMax(out, __float_as_uint(m));
 }
 
+// NaN-propagating max, as torch.max: a NaN on either side wins
+__device__ __forceinline__ float nan_max(float a, float b) { return (a > b || a != a) ? a : b; }
+
+// signed max over n values (gnn_normalize: f / torch.max(f)).  `out` starts as 0xffffffff, a bit pattern below every
+// candidate in both orders used here: a non-negative float (sign bit clear) wins an integer max against any negative
+// one, and among negative floats the smaller unsigned bits are the larger value.  NaN enters as the positive quiet
+// NaN, which is above +inf as an integer.  The result does not depend on the order in which warps arrive.
+__global__ void k_batch_max(const float* __restrict__ x, int64_t n, unsigned int* __restrict__ out) {
+    float m = -INFINITY;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        m = nan_max(m, x[i]);
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, d));
+    if ((threadIdx.x & 31) == 0) {
+        const unsigned int bits = (m != m) ? 0x7fc00000u : __float_as_uint(m);
+        if (bits & 0x80000000u) atomicMin(out, bits);
+        else atomicMax(reinterpret_cast<int*>(out), (int)bits);
+    }
+}
+
+// learnable temperature: the logits of weight set l are divided by temp[l], i.e. its folded weights are scaled by
+// 1 / temp[l], rounded as functional.DeformFunction.forward does (an fp32 reciprocal, then a multiply)
+__global__ void k_temp_fold(const float* __restrict__ Mu, const float* __restrict__ temp, int Lw, int S,
+                            float* __restrict__ Mu_eff) {
+    for (int t = threadIdx.x; t < Lw * S; t += blockDim.x) {
+        const float inv = 1.0f / temp[t / S];
+        Mu_eff[t] = Mu[t] * inv;
+    }
+}
+
+// one CTA per weight set: g_temp[l] = -sum_j gMu[l, j] * Mu_eff[l, j] / temp[l] (fixed-order tree, no atomics) and
+// gMu_base[l] = gMu[l] / temp[l] (DeformFunction.backward)
+constexpr int TF_THREADS = 128;
+__global__ void __launch_bounds__(TF_THREADS) k_temp_fold_bwd(const float* __restrict__ gMu, const float* __restrict__ Mu_eff,
+                                                              const float* __restrict__ temp, int S,
+                                                              float* __restrict__ gMu_base, float* __restrict__ g_temp) {
+    __shared__ float red[TF_THREADS];
+    const int l = blockIdx.x;
+    const float t = temp[l];
+    const float* g = gMu + (size_t)l * S;
+    const float* mu = Mu_eff + (size_t)l * S;
+    float s = 0.f;
+    for (int j = threadIdx.x; j < S; j += TF_THREADS) {
+        s = fmaf(g[j], mu[j], s);
+        gMu_base[(size_t)l * S + j] = g[j] / t;
+    }
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = TF_THREADS / 2; w > 0; w >>= 1) {
+        if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) g_temp[l] = -red[0] / t;
+}
+
 int glob_fill(GlobArgs& a, const char* who, const float* g_f, const float* g_uu, int B, int Co, int n_g,
               const float* Wq, const float* Wk, int Lw, int C, int z0, int live, int CE, float inv_temp) {
     GAD_CHECK_ARG((g_f || g_uu) && Wq && Wk, "%s: null pointer", who);
@@ -191,6 +246,34 @@ extern "C" int gad_absmax(const float* u, int64_t n, float* out, void* stream) {
     const int64_t blocks = (n + 256 * 8 - 1) / (256 * 8);
     const int grid = (int)(blocks < 4LL * sm_count() ? blocks : 4LL * sm_count());
     k_absmax<<<grid, 256, 0, st>>>(u, n, reinterpret_cast<unsigned int*>(out));
+    GAD_LAUNCH_CHECK();
+    return GAD_OK;
+}
+
+extern "C" int gad_batch_max(const float* x, int64_t n, float* out, void* stream) {
+    GAD_CHECK_ARG(x && out && n > 0, "gad_batch_max: null pointer or empty input (n=%lld)", (long long)n);
+    cudaStream_t st = as_stream(stream);
+    GAD_CUDA(cudaMemsetAsync(out, 0xff, sizeof(float), st));
+    const int64_t blocks = (n + 256 * 8 - 1) / (256 * 8);
+    const int grid = (int)(blocks < 4LL * sm_count() ? blocks : 4LL * sm_count());
+    k_batch_max<<<grid, 256, 0, st>>>(x, n, reinterpret_cast<unsigned int*>(out));
+    GAD_LAUNCH_CHECK();
+    return GAD_OK;
+}
+
+extern "C" int gad_temp_fold(const float* Mu, const float* temp, int Lw, int CE, float* Mu_eff, void* stream) {
+    GAD_CHECK_ARG(Mu && temp && Mu_eff, "gad_temp_fold: null pointer");
+    GAD_CHECK_ARG(Lw > 0 && (CE == 2 || CE == 4 || CE == 8), "gad_temp_fold: Lw=%d CE=%d", Lw, CE);
+    k_temp_fold<<<1, 256, 0, as_stream(stream)>>>(Mu, temp, Lw, CE * CE + CE, Mu_eff);
+    GAD_LAUNCH_CHECK();
+    return GAD_OK;
+}
+
+extern "C" int gad_temp_fold_bwd(const float* gMu, const float* Mu_eff, const float* temp, int Lw, int CE,
+                                 float* gMu_base, float* g_temp, void* stream) {
+    GAD_CHECK_ARG(gMu && Mu_eff && temp && gMu_base && g_temp, "gad_temp_fold_bwd: null pointer");
+    GAD_CHECK_ARG(Lw > 0 && (CE == 2 || CE == 4 || CE == 8), "gad_temp_fold_bwd: Lw=%d CE=%d", Lw, CE);
+    k_temp_fold_bwd<<<Lw, TF_THREADS, 0, as_stream(stream)>>>(gMu, Mu_eff, temp, CE * CE + CE, gMu_base, g_temp);
     GAD_LAUNCH_CHECK();
     return GAD_OK;
 }

@@ -32,6 +32,18 @@ buffer.  Such slots need meshes of equal size on the mesh-resident ELL kernels a
 38 x 38, at most 16 Gaussians and 16 cells per vertex); `add_batch` raises otherwise.  An explicit `loss_fn` trains
 the mesh loss instead.
 
+`gnn_normalize=True` (f / torch.max(f), uu / torch.max(uu) over the batch, src/GNN.py:231-237) keeps the slot's route and
+puts gad_batch_max in front of it: every step recomputes the maxima of the resident f / uu (a batch copied into the
+slot is normalised by its own), MAX-all-reduced over the ranks, into the f_scale / uu_scale the kernels divide by.
+
+`softmax_temp_type='learnable_a'` (a trainable temperature per weight set, src/GRAND_plus.py:152-154,328-329) trains
+through the chain of library kernels: the temperatures join the flat vector after the steps, each step folds them into
+the weights (gad_temp_fold: Mu / temp) and takes their gradient from the deformer's (gad_temp_fold_bwd).  k_ell_train
+cannot: its tail refolds (M, u) with a constant temperature.  Such slots need the mesh-resident ELL kernels.
+
+Neither option is trained together with global CNN features, and gnn_dont_train is refused: those raise
+NotImplementedError and train through GNN.forward + autograd.
+
 Sharding (SURVEY 8e): a batch is a disjoint union of meshes, so ranks take contiguous shards of
 whole meshes with no data-path collective; the only exchange is the all-reduce of the flat
 gradient (144 + L floats).  The mesh loss is a mean over ALL nodes of the global batch
@@ -87,11 +99,13 @@ class DeformerTrainer:
                 "to train the mesh loss on such a preset")
         # loss_type='pde_loss': mse(FEM solution on the deformed mesh, u_true_fine), unless loss_fn asks for the mesh loss
         self.pde = loss_fn is None and loss_type == "pde_loss"
-        if opt.get("softmax_temp_type") == "learnable_a":
-            raise NotImplementedError("DeformerTrainer: the learnable temperature is trained through GNN.forward + autograd")
-        if opt.get("gnn_normalize", False):
-            raise NotImplementedError("DeformerTrainer: gnn_normalize=True (per-batch f / max f, src/GNN.py:231-237) is "
-                                      "only implemented on the GNN.forward path")
+        # softmax_temp_type='learnable_a': one trainable temperature per weight set (src/GRAND_plus.py:152-154,328-329)
+        self.learn_temp = opt.get("softmax_temp_type") == "learnable_a"
+        # gnn_normalize: f / torch.max(f) and uu / torch.max(uu) over the batch (src/GNN.py:231-237)
+        self.normalize = bool(opt.get("gnn_normalize", False))
+        if getattr(model, "n_glob_used", 0) and (self.learn_temp or self.normalize):
+            raise NotImplementedError("DeformerTrainer: global CNN features together with gnn_normalize=True or "
+                                      "softmax_temp_type='learnable_a' train through GNN.forward + autograd")
         if opt.get("gnn_dont_train", False):
             raise NotImplementedError("DeformerTrainer: gnn_dont_train=True skips the optimizer step (src/run_GNN.py:122-131); "
                                       "evaluate with GNN.forward instead")
@@ -140,12 +154,14 @@ class DeformerTrainer:
 
     # ------------------------------------------------------------------------------------
     def _flatten_parameters(self):
-        """flat = [Wq (Lw,C,C) | bq (Lw,C) | Wk (Lw,C,C) | bk (Lw,C) | steps (L, if learn_step) | CNN f | CNN uu], the
-        parameters of each global feature extractor in gad_cnn_bwd's order (w_0, b_0, w_1, ...), when n_g > 0."""
+        """flat = [Wq (Lw,C,C) | bq (Lw,C) | Wk (Lw,C,C) | bk (Lw,C) | steps (L, if learn_step) | temperatures (Lw, if
+        learnable_a) | CNN f | CNN uu], the parameters of each global feature extractor in gad_cnn_bwd's order (w_0,
+        b_0, w_1, ...), when n_g > 0."""
         m, Lw, C = self.model, self.Lw, self.C
         convs = [m.conv_layers[0]] if self.opt["share_conv"] else list(m.conv_layers)
         nW, nb = Lw * C * C, Lw * C
         nsteps = self.L if self.opt["learn_step"] else 0
+        ntemp = Lw if self.learn_temp else 0
         cnn_specs, before = [], 0
         for name in (("f", "uu") if self.n_g else ()):
             ext = getattr(m, f"global_feature_extractor_cnn_{name}", None)
@@ -155,7 +171,7 @@ class DeformerTrainer:
             # module's cat + slice gives it; it is never run
             cnn_specs.append((name, ext, [p for c in ext.convs for p in (c.weight, c.bias)], self.n_g > before))
             before += ext.out_channels
-        n = 2 * nW + 2 * nb + nsteps + sum(p.numel() for _, _, ps, _ in cnn_specs for p in ps)
+        n = 2 * nW + 2 * nb + nsteps + ntemp + sum(p.numel() for _, _, ps, _ in cnn_specs for p in ps)
         flat = torch.empty(n, dtype=torch.float32, device=self.dev)
         gflat = torch.zeros(n, dtype=torch.float32, device=self.dev)
         o = 0
@@ -181,6 +197,15 @@ class DeformerTrainer:
                 self.tau = torch.full((self.L,), float(self.opt["time_step"]), dtype=torch.float32, device=self.dev)
                 self.gtau = None
             o += nsteps
+            self.temp = self.gtemp = None
+            if ntemp:
+                self.temp, self.gtemp = flat[o:o + ntemp], gflat[o:o + ntemp]
+                for l, c in enumerate(convs):
+                    p = c.sm_temp_a
+                    self.temp[l:l + 1].copy_(p.detach().to(self.dev).reshape(1))
+                    p.data = self.temp[l:l + 1].view(p.shape)
+                    p.grad = self.gtemp[l:l + 1].view(p.shape)
+            o += ntemp
             self.cnn = []
             for name, ext, ps, used in cnn_specs:
                 o0, ws, bs = o, [], []
@@ -201,6 +226,9 @@ class DeformerTrainer:
         self.step_count = torch.zeros(1, dtype=torch.int64, device=self.dev)
         self.Mu = torch.empty((Lw, self.CE * self.CE + self.CE), dtype=torch.float32, device=self.dev)
         self.gMu = torch.empty_like(self.Mu)
+        # learnable temperature: the folded weights the deformer kernels run on (Mu / temp) and the cotangent of Mu
+        self.Mu_eff = torch.empty_like(self.Mu) if ntemp else None
+        self.gMu_base = torch.empty_like(self.Mu) if ntemp else None
 
     def broadcast_parameters(self, src: int = 0):
         dp.broadcast_flat(self.flat, src=src, group=self.pg)
@@ -229,7 +257,8 @@ class DeformerTrainer:
         else:
             d.ell_in, d.ell_out, d.tile_ptr, d.N = P(g.ell_in), P(g.ell_out), P(g.ell_tile_ptr), s.N
             d.T, d.max_tile_nodes, d.max_deg = g.T, g.max_tile_nodes, g.ell_deg
-        d.x_comp, d.f, d.uu, d.f_scale, d.uu_scale, d.target = P(s.x_comp), P(s.f), P(s.uu), None, None, P(s.target)
+        d.x_comp, d.f, d.uu, d.target = P(s.x_comp), P(s.f), P(s.uu), P(s.target)
+        d.f_scale, d.uu_scale = P(s.f_scale), P(s.uu_scale)
         d.dim, d.CE = self.dim, self.CE
         d.Mu, d.tau, d.Lw, d.L, d.C, d.inv_temp = P(self.Mu), P(self.tau), self.Lw, self.L, self.C, self.model.inv_temp
         d.loss_kind = 0 if self.loss_kind == "l1" else 1
@@ -243,7 +272,9 @@ class DeformerTrainer:
         d.n_params = self.flat.numel()
         d.lr, d.beta1, d.beta2, d.eps, d.weight_decay, d.adam_grad_scale = self.lr, b1, b2, self.eps, self.wd, 1.0
         d.step = P(self.step_count)
-        d.flags = 1 if (self.use_pdl and tail == 2) else 0      # GAD_TRAIN_PDL
+        # GAD_TRAIN_PDL.  Not on a normalised slot: the kernel reads f_scale / uu_scale while staging its inputs, before
+        # it waits on its predecessor, which there is gad_batch_max (or the all-reduce of its result)
+        d.flags = 1 if (self.use_pdl and tail == 2 and not s.norm) else 0
         d.peer_timeout_ms = 0
         if self.fused_dp and tail == 2:
             d.rank, d.world, d.peers, d.peer_seq = self.rank, self.world, P(self.peer.ptrs), P(self.peer.seq)
@@ -268,9 +299,16 @@ class DeformerTrainer:
             s.N = N
             s.glob = bool(self.n_g)
             s.pde = self.pde
+            s.temp = self.learn_temp
+            s.norm = self.normalize
+            s.chain = s.glob or s.pde or s.temp      # the step is _issue_chain's chain of library kernels
             s.du = None
             if s.glob:
                 self._check_glob_graph(s.graph)
+            if s.temp and (self.opt.get("gad_force_stream", False) or not GF.use_ell(s.graph, self.CE)):
+                # k_ell_train refolds (M, u) with a constant temperature in its tail; the chain runs on these kernels
+                raise NotImplementedError("softmax_temp_type='learnable_a' trains on the mesh-resident ELL kernels (meshes "
+                                          "that fit a CTA, bounded degree); train this batch through GNN.forward + autograd")
             if s.pde:
                 self._pde_setup(s, data)
             f32 = dict(dtype=torch.float32, device=dev)
@@ -301,6 +339,10 @@ class DeformerTrainer:
             views = {name: (v if n else None) for (name, _, _), n, v in zip(segs, seg, s.in_views)}
             s.target, s.f, s.uu, s.x_comp = views["target"], views["f"], views["uu"], views["x_comp"]
             s.centers, s.scales = views.get("centers"), views.get("scales")
+            # gnn_normalize: [max f, max uu] of the batch, recomputed by every step (gad_batch_max)
+            s.norm_max = torch.ones(2, **f32) if s.norm else None
+            s.f_scale = s.norm_max[0:1] if s.norm and s.f is not None else None
+            s.uu_scale = s.norm_max[1:2] if s.norm and s.uu is not None else None
             s.states = torch.empty((self.L, N, self.CE), **f32)
             s.x_phys = torch.empty((N, self.dim), **f32)
             s.g_out = torch.empty((N, self.dim), **f32)
@@ -494,7 +536,9 @@ class DeformerTrainer:
     # ------------------------------------------------------------------------------------
     def _issue(self, s: _Slot, stream_ptr: int, with_optimizer: bool = True, stage: str = "all"):
         """Enqueue the kernels of one training step on `stream_ptr` (captured or eager)."""
-        if s.glob or s.pde:
+        if s.norm and stage in ("all", "pre"):
+            self._issue_batch_max(s, stream_ptr)
+        if s.chain:
             return self._issue_chain(s, stream_ptr, with_optimizer, stage)
         lib, P, chk = self.lib, _lib.ptr, _lib.check
         g = s.graph
@@ -528,8 +572,8 @@ class DeformerTrainer:
         if stage in ("all", "pre"):
             chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
                 "gad_prepare_weights")
-            chk(lib.gad_pack_features(P(s.x_comp), P(s.f), P(s.uu), None, None, s.N, dim, CE, P(s.states), stream_ptr),
-                "gad_pack_features")
+            chk(lib.gad_pack_features(P(s.x_comp), P(s.f), P(s.uu), P(s.f_scale), P(s.uu_scale), s.N, dim, CE,
+                                      P(s.states), stream_ptr), "gad_pack_features")
             wide = (not tiles) and g.ensure_wide(CE)      # streaming ELL kernels (csrc/stream_ell.cu)
             if wide:
                 chk(lib.gad_deform_fwd_wide(P(g.wide_in), s.N, g.wide_deg, g.wide_reach, P(s.states), dim, CE, P(self.Mu), Lw, P(self.tau), L,
@@ -575,15 +619,17 @@ class DeformerTrainer:
 
     def _issue_chain(self, s: _Slot, stream_ptr: int, with_optimizer: bool, stage: str):
         """The step of a slot that is not on the one-launch kernel, as a chain of library kernels on the mesh-resident
-        ELL graph (a slot with global CNN features, or a pde slot):  [CNN forward -> bias offset du] -> deformer
-        forward [with du] -> loss stage (mesh loss; or FEM forward -> pde loss -> FEM backward) -> deformer backward ->
-        weight gradients -> [adjoint of du (CNN cotangents and the du terms of gWq / gWk) -> CNN backward into the
-        flat gradient] -> [all-reduce] -> Adam over the whole flat vector.  These are the kernels GNN.forward +
-        autograd run for the same batch."""
+        ELL graph (a slot with global CNN features, a pde slot, or a learnable temperature):  [CNN forward -> bias
+        offset du] -> [Mu / temp] -> deformer forward [with du] -> loss stage (mesh loss; or FEM forward -> pde loss ->
+        FEM backward) -> deformer backward -> [temperature gradient, cotangent of Mu] -> weight gradients -> [adjoint of
+        du (CNN cotangents and the du terms of gWq / gWk) -> CNN backward into the flat gradient] -> [all-reduce] ->
+        Adam over the whole flat vector.  These are the kernels GNN.forward + autograd run for the same batch."""
         lib, P, chk = self.lib, _lib.ptr, _lib.check
         g, m = s.graph, self.model
         CE, L, Lw, C_, dim = self.CE, self.L, self.Lw, self.C, self.dim
         inv_temp = m.inv_temp
+        Mu = self.Mu_eff if s.temp else self.Mu                    # the folded weights the deformer kernels run on
+        gMu_w = self.gMu_base if s.temp else self.gMu              # the cotangent gad_weight_grads takes
         if s.glob:
             B = s.B
             used = [r for r in self.cnn if r["used"]]
@@ -594,6 +640,8 @@ class DeformerTrainer:
         if stage in ("all", "pre"):
             chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
                 "gad_prepare_weights")
+            if s.temp:
+                chk(lib.gad_temp_fold(P(self.Mu), P(self.temp), Lw, CE, P(Mu), stream_ptr), "gad_temp_fold")
             if s.glob:
                 for r in used:
                     u, scale = src[r["name"]], s.cnn_scale[r["name"]]
@@ -608,8 +656,8 @@ class DeformerTrainer:
             f = s.f if self.opt["gnn_inc_feat_f"] and dim < CE else None
             uu = s.uu if self.opt["gnn_inc_feat_uu"] and dim + (1 if f is not None else 0) < CE else None
             chk(lib.gad_deform_fwd_ell_raw(P(g.ell_in), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes, g.ell_deg,
-                                           P(s.x_comp), P(f), P(uu), None, None, dim, CE, P(self.Mu), P(s.du), Lw,
-                                           P(self.tau), L, self.method, P(s.x_phys), P(s.states), stream_ptr),
+                                           P(s.x_comp), P(f), P(uu), P(s.f_scale), P(s.uu_scale), dim, CE, P(Mu),
+                                           P(s.du), Lw, P(self.tau), L, self.method, P(s.x_phys), P(s.states), stream_ptr),
                 "gad_deform_fwd_ell_raw")
             if s.pde:
                 self._issue_pde_loss(s, stream_ptr)
@@ -619,19 +667,22 @@ class DeformerTrainer:
                                       P(s.g_out), P(s.loss_ws), stream_ptr), "gad_mesh_loss")
             if self.method == GF.METHOD_RK4 and not s.rk4_resident:
                 chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
-                                                dim, CE, P(self.Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
+                                                dim, CE, P(Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
                                                 s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
             elif self.method == GF.METHOD_RK4:
                 chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
-                                               g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), P(s.du), Lw,
+                                               g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(Mu), P(s.du), Lw,
                                                P(self.tau), L, P(self.gMu), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
                     "gad_deform_bwd_ell_rk4")
             else:
                 chk(lib.gad_deform_bwd_ell(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
-                                           g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), P(s.du), Lw, P(self.tau),
+                                           g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(Mu), P(s.du), Lw, P(self.tau),
                                            L, P(self.gMu), P(self.gtau), None, P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr),
                     "gad_deform_bwd_ell")
-            chk(lib.gad_weight_grads(P(self.Wq), P(self.bq), P(self.Wk), P(self.gMu), Lw, C_, CE, inv_temp, P(self.gWq),
+            if s.temp:      # d loss / d temp into the flat gradient, and the cotangent of the base (M, u)
+                chk(lib.gad_temp_fold_bwd(P(self.gMu), P(Mu), P(self.temp), Lw, CE, P(gMu_w), P(self.gtemp), stream_ptr),
+                    "gad_temp_fold_bwd")
+            chk(lib.gad_weight_grads(P(self.Wq), P(self.bq), P(self.Wk), P(gMu_w), Lw, C_, CE, inv_temp, P(self.gWq),
                                      P(self.gbq), P(self.gWk), P(self.gbk), stream_ptr), "gad_weight_grads")
             if s.glob:
                 chk(lib.gad_glob_bias_bwd(P(g_f), P(g_uu), *glob, P(s.bwd_ws), s.bwd_ws_bytes, P(s.cnn_gout.get("f")),
@@ -647,6 +698,16 @@ class DeformerTrainer:
             chk(lib.gad_adam_step(P(self.flat), P(self.gflat), P(self.exp_avg), P(self.exp_avg_sq), self.flat.numel(),
                                   self.lr, b1, b2, self.eps, self.wd, 1.0, P(self.step_count), stream_ptr),
                 "gad_adam_step")
+
+    def _issue_batch_max(self, s: _Slot, stream_ptr: int):
+        """gnn_normalize: the maxima of the slot's resident f and uu into f_scale / uu_scale, the divisors the deformer
+        kernels apply (f / torch.max(f), src/GNN.py:231-237).  Inside the step, so that every batch copied into the slot
+        is normalised by its own maxima; with several ranks they are MAX-all-reduced to the global batch's."""
+        for u, out in ((s.f, s.f_scale), (s.uu, s.uu_scale)):
+            if out is not None:
+                _lib.check(self.lib.gad_batch_max(_lib.ptr(u), u.numel(), _lib.ptr(out), stream_ptr), "gad_batch_max")
+        if self.world > 1 and self.loopback is None:
+            dist.all_reduce(s.norm_max, op=dist.ReduceOp.MAX, group=self.pg)
 
     def _issue_pde_loss(self, s: _Slot, stream_ptr: int, coords: Optional[torch.Tensor] = None):
         """Loss stage of a pde slot: FEM forward on the deformed meshes (`coords`, default the slot's x_phys) -> mean
@@ -684,13 +745,13 @@ class DeformerTrainer:
         """The step of this slot is the one-launch kernel k_ell_train (gad_train_step_ell / _rk4)."""
         g = s.graph
         tiles = g.tile_ptr is not None and not self.opt.get("gad_force_stream", False)
-        return bool(tiles and not (s.glob or s.pde) and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
+        return bool(tiles and not s.chain and GF.use_ell(g, self.CE) and not self.opt.get("gad_no_fused_train", False)
                     and (self.method == GF.METHOD_EULER or s.rk4_fused))
 
     def _cluster(self, s: _Slot) -> bool:
         """Meshes too large for one CTA run on the cluster-resident kernel (csrc/cl_kernels.cu, Euler only)."""
         g = s.graph
-        if not (self.method == GF.METHOD_EULER and not (s.glob or s.pde) and g.tile_ptr is None and g.cl_in is not None
+        if not (self.method == GF.METHOD_EULER and not s.chain and g.tile_ptr is None and g.cl_in is not None
                 and not self.opt.get("gad_no_cluster", False) and not self.opt.get("gad_force_stream", False)):
             return False
         if s.prefer_stream is None:      # one or two very large meshes: the streaming chain uses all SMs
@@ -932,9 +993,10 @@ class DeformerTrainer:
         cs, ms = self._copy_stream, self.stream
         packed = all(torch.is_tensor(b) and (b.is_pinned() or getattr(b, "_gad_pinned", False)) and b.dtype == torch.float32
                      for b in host_batches)
-        # the step's graph holds library kernels only (a slot with global features or a pde slot, single GPU: a chain
-        # of them)
-        pure = all(self._one_launch(s) or ((s.glob or s.pde) and self.world == 1) for s in self.slots)
+        # the step's graph holds library kernels only (single GPU: a chain slot's chain of them; several ranks: no
+        # collective in the graph, so not a normalised slot, whose maxima are all-reduced)
+        pure = all((self._one_launch(s) and not (s.norm and self.world > 1 and self.loopback is None))
+                   or (s.chain and self.world == 1) for s in self.slots)
         if native is None:
             native = self.use_graph and packed and pure
         if native:

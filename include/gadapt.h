@@ -498,6 +498,17 @@ int gad_glob_bias_bwd(const float* g_f, const float* g_uu, int B, int Co, int n_
                       float* g_out_f, float* g_out_uu, float* gWq, float* gWk, void* stream);
 /* out[0] = max |u[i]| over n values (the CNN's normalisation, `scale` of gad_cnn_fwd), on the device. */
 int gad_absmax(const float* u, int64_t n, float* out, void* stream);
+/* out[0] = max x[i] over n > 0 values, equal to torch.max(x) with NaN propagating (gnn_normalize's f / max f, whose
+ * result feeds the f_scale / uu_scale arguments of the deformer kernels). */
+int gad_batch_max(const float* x, int64_t n, float* out, void* stream);
+/* Learnable softmax temperature (softmax_temp_type='learnable_a'): the logits of weight set l are divided by temp[l].
+ * gad_temp_fold: Mu_eff[l] = Mu[l] * (1 / temp[l]) for the Lw rows of CE*CE + CE folded weights (the fp32 reciprocal,
+ * then a multiply).  gad_temp_fold_bwd, from gMu = d loss / d Mu_eff:
+ *     g_temp[l] = -sum_j gMu[l, j] * Mu_eff[l, j] / temp[l]   (fixed-order sum, no atomics)
+ *     gMu_base[l] = gMu[l] / temp[l]                          (the input of gad_weight_grads). */
+int gad_temp_fold(const float* Mu, const float* temp, int Lw, int CE, float* Mu_eff, void* stream);
+int gad_temp_fold_bwd(const float* gMu, const float* Mu_eff, const float* temp, int Lw, int CE, float* gMu_base,
+                      float* g_temp, void* stream);
 
 /* ---- host side of the end-to-end training loop ------------------------------------------------------
  * The reference's `for data in loader: ... loss.backward(); optimizer.step()` (src/run_GNN.py:95-131) with
