@@ -288,6 +288,10 @@ class GNN(nn.Module):
                 raise NotImplementedError("global CNN features need meshes of equal size in a batch")
             tile_nodes = int(sizes[0])              # one mesh per tile: the bias offset is per tile
         graph = self._graph(data, dev, allow_uniform=not keep_alpha, tile_nodes=tile_nodes)
+        if tile_nodes is not None and graph.tile_ptr is not None and not GF.use_ell(graph, self.CE):
+            # a mesh too large for the mesh-resident ELL kernels: the graph a model without global features builds, which
+            # runs on the cluster / streaming kernels (they take the offset per mesh), not on CSR tiles
+            graph = self._graph(data, dev, allow_uniform=not keep_alpha)
         x_comp = data.x_comp.to(dev, non_blocking=True)
         f = data.f_tensor.to(dev, non_blocking=True) if opt["gnn_inc_feat_f"] else None
         uu = data.uu_tensor.to(dev, non_blocking=True) if opt["gnn_inc_feat_uu"] else None

@@ -80,10 +80,10 @@ SIGNATURES = {
                             _p, _sz, _p]),
     "gad_graph_build_wide": (_i, [_p, _p, _i64, _p, _p, _p]),
     "gad_deform_bwd_wide_rk4_workspace_bytes": (_sz, [_i64, _i]),
-    "gad_deform_bwd_wide_rk4": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _p, _i, _p, _i, _p, _p, _p, _sz, _p]),
+    "gad_deform_bwd_wide_rk4": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _p, _p, _i, _i, _p, _i, _p, _p, _p, _p, _sz, _p]),
     "gad_wide_persist_nodes": (_i64, [_i, _i, _i64]),
-    "gad_deform_fwd_wide": (_i, [_p, _i64, _i, _i64, _p, _i, _i, _p, _i, _p, _i, _i, _p, _p, _p, _sz, _p]),
-    "gad_deform_bwd_wide": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _p, _i, _p, _i, _p, _p, _p, _p, _sz, _p]),
+    "gad_deform_fwd_wide": (_i, [_p, _i64, _i, _i64, _p, _i, _i, _p, _p, _i, _i, _p, _i, _i, _p, _p, _p, _sz, _p]),
+    "gad_deform_bwd_wide": (_i, [_p, _p, _i64, _i, _p, _p, _i, _i, _p, _p, _i, _i, _p, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "gad_graph_build_ell": (_i, [_p, _p, _i64, _p, _i, _i, _i, _p, _p, _p]),
     "gad_ell_supported": (_i, [_i, _i, _i, _i]),
     "gad_ell_workspace_bytes": (_sz, [_i, _i, _i]),
@@ -98,8 +98,10 @@ SIGNATURES = {
                                   _f, _f, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "gad_train_step_ell": (_i, [C.POINTER(TrainDesc), _p]),
     "gad_cluster_plan": (_i, [_i, _i, _i, C.POINTER(_i), C.POINTER(_i)]),
-    "gad_deform_bwd_cluster": (_i, [_p, _p, _p, _i, _i, _i, _i, _i64, _p, _p, _i, _i, _p, _i, _p, _i, _p, _p, _p, _p, _sz, _p]),
-    "gad_deform_fwd_cluster": (_i, [_p, _p, _i, _i, _i, _i, _i64, _p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _i, _i, _p, _p, _p]),
+    "gad_deform_bwd_cluster": (_i, [_p, _p, _p, _i, _i, _i, _i, _i64, _p, _p, _i, _i, _p, _p, _i, _p, _i, _p, _p, _p, _p, _p,
+                                    _sz, _p]),
+    "gad_deform_fwd_cluster": (_i, [_p, _p, _i, _i, _i, _i, _i64, _p, _p, _p, _p, _p, _i, _i, _p, _p, _i, _p, _i, _i, _p, _p,
+                                    _p]),
     "gad_graph_build_cluster": (_i, [_p, _p, _p, _i, _i, _i, _i, _p, _p, _p]),
     "gad_cluster_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "gad_cluster_occupancy": (_i, [_i, _i, _i, _i, C.POINTER(_i)]),

@@ -118,9 +118,11 @@ __host__ __device__ inline Layout make_layout(int CE, int cap_nodes, int nwarps)
 
 // ---- backward of one slab (shared by the train and the backward kernels) ---------------------------------
 // On entry: X = x^{L-1} rows of the slab (buffer at cluster offset offX), GS = dL/dx^L rows, Mu = weights of
-// layer L-1; GO (offset offGO) is free.  Per-CTA partial rows go to a.partials[blockIdx.x].
-template <int CE, int W>
-__device__ __forceinline__ void cl_backward(const Args& a, const Layout& lay, int n0, int NT, unsigned char* X,
+// layer L-1 (with the bias offset of the mesh when DU: a.du, global CNN features); GO (offset offGO) is free.  Per-CTA
+// partial rows go to a.partials[blockIdx.x].  DU is a template flag so that the kernels without the offset compile to
+// what they were before it existed.
+template <int CE, int W, bool DU>
+__device__ __forceinline__ void cl_backward(const Args& a, const Layout& lay, int mesh, int n0, int NT, unsigned char* X,
                                             unsigned char* GO, uint32_t offX, uint32_t offGO, unsigned char* P,
                                             unsigned char* DL, unsigned char* GS, const uint4* __restrict__ Rin,
                                             const uint4* __restrict__ Rout, float* Mu, float* red,
@@ -138,7 +140,8 @@ __device__ __forceinline__ void cl_backward(const Args& a, const Layout& lay, in
     for (int k = 0; k < NACC; ++k) acc[k] = 0.f;
     for (int l = a.L - 1; l >= 0; --l) {
         if (per_layer && l < a.L - 1) {
-            for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
+            if constexpr (DU) ell::load_mu<CE>(a, Mu, l, mesh);
+            else for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
             __syncthreads();
         }
         const float b = __ldcg(a.tau + l);
@@ -421,7 +424,7 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_train(const Args a) {
     tr.mark();
 
     // ---- backward: Xc = x^{L-1}, Xn = free -> GO ---------------------------------------------------
-    cl_backward<CE, W>(a, lay, n0, NT, Xc, Xn, offXc, offXn, P, DL, GS, Rin, Rout, Mu, red, s_base);
+    cl_backward<CE, W, false>(a, lay, mesh, n0, NT, Xc, Xn, offXc, offXn, P, DL, GS, Rin, Rout, Mu, red, s_base);
     tr.mark();
     // no CTA may leave while a peer can still read its shared memory
     cluster_sync();
@@ -446,7 +449,8 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_train(const Args a) {
 }
 
 // ---- backward only (autograd of the module seam): from the saved layer inputs ---------------------------
-template <int CE, int W>
+// DU: a.du holds the per-mesh bias offset (global CNN features)
+template <int CE, int W, bool DU>
 __global__ void __launch_bounds__(MAXT, 1) k_cl_bwd(const Args a) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
@@ -475,9 +479,10 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_bwd(const Args a) {
         sts_row<CE>(GS, i * RB, ell::load_dims<CE>(a.g_xphys, (int64_t)n0 + i, a.dim));   // cotangent of x^L[:, :dim]
     }
     const int lw = (a.Lw > 1) ? a.L - 1 : 0;
-    for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)lw * MUSZ + t];
+    if constexpr (DU) ell::load_mu<CE>(a, Mu, lw, mesh);
+    else for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)lw * MUSZ + t];
     cluster_sync();
-    cl_backward<CE, W>(a, lay, n0, NT, X, GO, lay.xa, lay.xb, P, DL, GS, a.ell_in + 2 * (size_t)n0,
+    cl_backward<CE, W, DU>(a, lay, mesh, n0, NT, X, GO, lay.xa, lay.xb, P, DL, GS, a.ell_in + 2 * (size_t)n0,
                        a.ell_out + 2 * (size_t)n0, Mu, red, s_base);
     cluster_sync();   // nobody leaves while a peer may still read its shared memory
 }
@@ -487,6 +492,18 @@ __global__ void k_cl_reduce(const float* __restrict__ partials, int T, int slots
                             const float* __restrict__ tau_partials, int L, float* __restrict__ g_tau) {
     tail::reduce_partials(partials, T, slots, nacc, musz, gMu, tau_partials, L, g_tau, nullptr, 0.f, nullptr,
                           blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5));
+}
+
+// d loss / d du [M, Lw, CE] (global CNN features): G_u of the cluster's C per-CTA partial rows, summed in rank order
+__global__ void k_cl_du_reduce(const float* __restrict__ partials, int M, int C, int Lw, int slots, int nacc, int CE,
+                               float* __restrict__ g_du) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= M * Lw * CE) return;
+    const int z = k % CE, lw = (k / CE) % Lw, b = k / (CE * Lw);
+    const int slot = (slots > 1) ? lw : 0;
+    double s = 0.0;
+    for (int r = 0; r < C; ++r) s += (double)partials[((size_t)(b * C + r) * slots + slot) * nacc + CE * CE + z];
+    g_du[k] = (float)s;
 }
 
 // ---- forward only (module seam / inference): Euler layers or classical RK4 steps -------------------------
@@ -532,7 +549,7 @@ __device__ __forceinline__ Row<CE> cl_feval(const CRow& e, const Row<CE>& y, con
 // One cluster per mesh, the state resident in shared memory for ALL layers / RK4 steps of the call
 // (BASELINE config 4: a 200x200 mesh, 64 RK4 steps = 256 F-evaluations, is one launch of 16 CTAs
 // instead of 256 dependent launches).  Inputs are the raw features (src/GNN.py:225-239).
-template <int CE, int W, int METHOD>
+template <int CE, int W, int METHOD, bool DU>
 __global__ void __launch_bounds__(MAXT, 1) k_cl_fwd(const Args a) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
@@ -552,7 +569,8 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_fwd(const Args a) {
     const int n0 = m0 + (int)rank * S;
     const int NT = max(0, min(S, NM - (int)rank * S));
     if (tid < 16) s_base[tid] = (tid < (int)C) ? mapa(smem_u32(smem), (uint32_t)tid) : 0u;
-    for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[t];
+    if constexpr (DU) ell::load_mu<CE>(a, Mu, 0, mesh);
+    else for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[t];
     const size_t state_stride = (size_t)a.N * CE;
     const uint4* Rin = a.ell_in + 2 * (size_t)n0;
     ell::assemble_rows<CE>(a, n0, NT, false, nullptr, nullptr, nullptr, Xc, a.states);
@@ -561,7 +579,8 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_fwd(const Args a) {
     for (int l = 0; l < a.L; ++l) {
         if (a.Lw > 1 && l > 0) {
             __syncthreads();
-            for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
+            if constexpr (DU) ell::load_mu<CE>(a, Mu, l, mesh);
+            else for (int t = tid; t < MUSZ; t += nthr) Mu[t] = a.Mu[(size_t)l * MUSZ + t];
             __syncthreads();
         }
         const float h = a.tau[l];
@@ -884,11 +903,12 @@ namespace gad {
 namespace cl {
 template <int CE, int W, int METHOD>
 int launch_fwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
+    auto kern = a.du ? k_cl_fwd<CE, W, METHOD, true> : k_cl_fwd<CE, W, METHOD, false>;
     const size_t bytes = make_layout(CE, a.cap_nodes, (threads + 31) / 32).total;
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "cluster kernel: slab of %d nodes needs %zu B of shared memory",
                   a.cap_nodes, bytes);
-    GAD_CUDA(cudaFuncSetAttribute(k_cl_fwd<CE, W, METHOD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(k_cl_fwd<CE, W, METHOD>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3((unsigned)threads);
@@ -901,7 +921,7 @@ int launch_fwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    GAD_CUDA(cudaLaunchKernelEx(&cfg, k_cl_fwd<CE, W, METHOD>, a));
+    GAD_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
     count_launch(1);
     return GAD_OK;
 }
@@ -909,12 +929,13 @@ int launch_fwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
 }  // namespace gad
 
 /* Deformer forward from the raw inputs on cluster-resident meshes, ONE launch for all L layers / RK4
- * steps (gad_deform_fwd_ell_raw's contract with cluster rows, mesh_ptr [M + 1] and the cluster size). */
+ * steps (gad_deform_fwd_ell_raw's contract with cluster rows, mesh_ptr [M + 1] and the cluster size;
+ * du [M, Lw, CE] or NULL: per-mesh bias offset). */
 extern "C" int gad_deform_fwd_cluster(const void* crows_in, const int32_t* mesh_ptr, int M, int max_mesh_nodes,
                                       int max_deg, int cluster_size, int64_t N, const float* x_comp, const float* f,
                                       const float* uu, const float* f_scale, const float* uu_scale, int dim, int CE,
-                                      const float* Mu, int Lw, const float* tau, int L, int method, float* x_phys,
-                                      float* states, void* stream) {
+                                      const float* Mu, const float* du, int Lw, const float* tau, int L, int method,
+                                      float* x_phys, float* states, void* stream) {
     GAD_CHECK_ARG(crows_in && mesh_ptr && x_comp && Mu && tau && x_phys, "gad_deform_fwd_cluster: null pointer");
     GAD_CHECK_ARG(N > 0 && M > 0 && L > 0 && dim >= 1 && dim <= CE && (Lw == 1 || Lw == L) && (CE == 2 || CE == 4),
                   "gad_deform_fwd_cluster: N=%lld M=%d L=%d dim=%d CE=%d Lw=%d", (long long)N, M, L, dim, CE, Lw);
@@ -933,6 +954,7 @@ extern "C" int gad_deform_fwd_cluster(const void* crows_in, const int32_t* mesh_
     a.cap_nodes = S;
     a.N = N;
     a.Mu = Mu;
+    a.du = du;
     a.tau = tau;
     a.Lw = Lw;
     a.L = L;
@@ -962,11 +984,12 @@ namespace gad {
 namespace cl {
 template <int CE, int W>
 int launch_bwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
+    auto kern = a.du ? k_cl_bwd<CE, W, true> : k_cl_bwd<CE, W, false>;
     const size_t bytes = make_layout(CE, a.cap_nodes, (threads + 31) / 32).total;
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "cluster kernel: slab of %d nodes needs %zu B of shared memory",
                   a.cap_nodes, bytes);
-    GAD_CUDA(cudaFuncSetAttribute(k_cl_bwd<CE, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(k_cl_bwd<CE, W>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3((unsigned)threads);
@@ -979,7 +1002,7 @@ int launch_bwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    GAD_CUDA(cudaLaunchKernelEx(&cfg, k_cl_bwd<CE, W>, a));
+    GAD_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
     count_launch(1);
     return GAD_OK;
 }
@@ -987,17 +1010,19 @@ int launch_bwd_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
 }  // namespace gad
 
 /* Deformer backward on cluster-resident meshes (gad_deform_bwd_ell's contract over cluster rows):
- * cotangent g_xphys [N, dim] + saved states [L, N, CE] -> gMu, g_tau (may be NULL), g_x0 (may be NULL).
+ * cotangent g_xphys [N, dim] + saved states [L, N, CE] -> gMu, g_tau (may be NULL), g_x0 (may be NULL), and with the
+ * per-mesh bias offset du [M, Lw, CE] of the forward, g_du [M, Lw, CE] (may be NULL).
  * workspace: gad_cluster_workspace_bytes(CE, M, cluster_size, L). */
 extern "C" int gad_deform_bwd_cluster(const void* crows_in, const void* crows_out, const int32_t* mesh_ptr, int M,
                                       int max_mesh_nodes, int max_deg, int cluster_size, int64_t N, const float* states,
-                                      const float* g_xphys, int dim, int CE, const float* Mu, int Lw, const float* tau,
-                                      int L, float* gMu, float* g_tau, float* g_x0, void* workspace,
-                                      size_t workspace_bytes, void* stream) {
+                                      const float* g_xphys, int dim, int CE, const float* Mu, const float* du, int Lw,
+                                      const float* tau, int L, float* gMu, float* g_tau, float* g_x0, float* g_du,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
     GAD_CHECK_ARG(crows_in && crows_out && mesh_ptr && states && g_xphys && Mu && tau && gMu && workspace,
                   "gad_deform_bwd_cluster: null pointer");
     GAD_CHECK_ARG(N > 0 && M > 0 && L > 0 && dim >= 1 && dim <= CE && (Lw == 1 || Lw == L) && (CE == 2 || CE == 4),
                   "gad_deform_bwd_cluster: N=%lld M=%d L=%d dim=%d CE=%d Lw=%d", (long long)N, M, L, dim, CE, Lw);
+    GAD_CHECK_ARG(!g_du || du, "gad_deform_bwd_cluster: g_du needs the bias offset du of the forward");
     const int C = cluster_size;
     GAD_CHECK_ARG(C >= 2 && C <= 16 && (C & (C - 1)) == 0, "gad_deform_bwd_cluster: cluster size %d", C);
     const int grid = M * C;
@@ -1016,6 +1041,7 @@ extern "C" int gad_deform_bwd_cluster(const void* crows_in, const void* crows_ou
     a.cap_nodes = S;
     a.N = N;
     a.Mu = Mu;
+    a.du = du;
     a.tau = tau;
     a.Lw = Lw;
     a.L = L;
@@ -1038,5 +1064,10 @@ extern "C" int gad_deform_bwd_cluster(const void* crows_in, const void* crows_ou
     const int ncol = slots * NACC + L + 1;
     cl::k_cl_reduce<<<(ncol + 7) / 8, 256, 0, st>>>(a.partials, grid, slots, NACC, MUSZ, gMu, a.tau_partials, L, g_tau);
     GAD_LAUNCH_CHECK();
+    if (g_du) {
+        const int n = M * Lw * CE;
+        cl::k_cl_du_reduce<<<(n + 127) / 128, 128, 0, st>>>(a.partials, M, C, Lw, slots, NACC, CE, g_du);
+        GAD_LAUNCH_CHECK();
+    }
     return GAD_OK;
 }

@@ -14,6 +14,8 @@
 //             the input-plane gradient for the next layer down.  Per-mesh parameter gradients go to a workspace and
 //             are summed over the batch in fp64 in a fixed order by a second kernel: no atomics, bit-reproducible.
 // The grid values carry no gradient (f / uu are data), as in the reference's use.
+#include <stdlib.h>
+
 #include "common.cuh"
 
 namespace gad {
@@ -36,6 +38,8 @@ struct CnnArgs {
     float* g_part;           // [B, n_params]       (backward: per-mesh parameter gradients)
     float* act_global;       // [B, L, Cmax, H*W] or null: activation planes in global memory (L2) when they do not
                              // fit the shared memory next to the other buffers
+    float* grad_global;      // [B, 2, Cmax, H*W] or null (backward): the two gradient planes in global memory when
+                             // they do not fit the shared memory either
     int B, H, W, Cm, Co, L, KH;
     int n_params;
 };
@@ -54,13 +58,15 @@ __host__ __device__ inline int cnn_param_offset(const CnnArgs& a, int l) {      
 __host__ __device__ inline int cnn_cmax(const CnnArgs& a) { return a.Cm > a.Co ? a.Cm : a.Co; }
 
 // shared memory: input plane [HW] | L activation planes [Cmax * HW] (unless in global memory) | (backward) two
-// gradient planes | weights | bias
-__host__ __device__ inline size_t cnn_smem_bytes(const CnnArgs& a, bool backward, bool act_in_smem) {
+// gradient planes (unless in global memory) | weights | bias
+__host__ __device__ inline size_t cnn_smem_bytes(const CnnArgs& a, bool backward, bool act_in_smem, bool grad_in_smem) {
     const size_t HW = (size_t)a.H * a.W, C = cnn_cmax(a);
-    size_t fl = HW + (act_in_smem ? (size_t)a.L * C * HW : 0) + (backward ? 2 * C * HW : 0) + C * C * a.KH * 3 + C + 64;
+    size_t fl = HW + (act_in_smem ? (size_t)a.L * C * HW : 0) + (backward && grad_in_smem ? 2 * C * HW : 0) +
+                C * C * a.KH * 3 + C + 64;
     return fl * sizeof(float);
 }
 __host__ __device__ inline size_t cnn_act_floats(const CnnArgs& a) { return (size_t)a.L * cnn_cmax(a) * a.H * a.W; }
+__host__ __device__ inline size_t cnn_grad_floats(const CnnArgs& a) { return (size_t)2 * cnn_cmax(a) * a.H * a.W; }
 
 // layers 0 .. L-1 into the activation planes (all threads; ends with a barrier)
 __device__ void cnn_forward_planes(const CnnArgs& a, int mesh, float* in, float* act, float* wsm, float* bsm) {
@@ -135,9 +141,10 @@ __global__ void __launch_bounds__(CNN_THREADS) k_cnn_bwd(const CnnArgs a) {
     const int mesh = blockIdx.x;
     float* in = cnn_sm;
     float* act = a.act_global ? a.act_global + (size_t)mesh * cnn_act_floats(a) : in + HW;
-    float* gA = in + HW + (a.act_global ? 0 : cnn_act_floats(a));
+    float* gsm = in + HW + (a.act_global ? 0 : cnn_act_floats(a));
+    float* gA = a.grad_global ? a.grad_global + (size_t)mesh * cnn_grad_floats(a) : gsm;
     float* gB = gA + (size_t)C * HW;
-    float* wsm = gB + (size_t)C * HW;
+    float* wsm = a.grad_global ? gsm : gB + (size_t)C * HW;
     float* bsm = wsm + C * C * KH * 3;
     cnn_forward_planes(a, mesh, in, act, wsm, bsm);
     float* gpart = a.g_part + (size_t)mesh * a.n_params;
@@ -251,19 +258,29 @@ extern "C" int64_t gad_cnn_param_count(int H, int Cm, int Co, int L) {
 }
 
 // workspace: [B, n_params] per-mesh parameter gradients (backward), then -- when the activation planes do not fit the
-// shared memory -- [B, L, Cmax, H*W] activations
-static size_t cnn_plan(CnnArgs& a, bool backward, bool* act_in_smem) {
-    *act_in_smem = (int)cnn_smem_bytes(a, backward, true) <= smem_optin_bytes();
-    return cnn_smem_bytes(a, backward, *act_in_smem);
+// shared memory -- [B, L, Cmax, H*W] activations, then -- when the backward's two gradient planes do not fit next to the
+// input plane either (8 channels: grids beyond about 58 x 58) -- [B, 2, Cmax, H*W] gradient planes.  Activations leave
+// shared memory first.  GAD_CNN_GRAD_GLOBAL=1 puts the gradient planes in the workspace whatever fits (read per call;
+// the summation order does not depend on where the planes live, so the results are the same bits).
+static size_t cnn_plan(CnnArgs& a, bool backward, bool* act_in_smem, bool* grad_in_smem) {
+    const char* e = getenv("GAD_CNN_GRAD_GLOBAL");
+    const bool force_grad_global = backward && e && e[0] == '1';
+    *act_in_smem = !force_grad_global && (int)cnn_smem_bytes(a, backward, true, true) <= smem_optin_bytes();
+    *grad_in_smem = !force_grad_global && (int)cnn_smem_bytes(a, backward, *act_in_smem, true) <= smem_optin_bytes();
+    return cnn_smem_bytes(a, backward, *act_in_smem, *grad_in_smem);
+}
+
+static size_t cnn_grads_bytes(const CnnArgs& a) {
+    return ((size_t)a.B * (size_t)gad_cnn_param_count(a.H, a.Cm, a.Co, a.L) * sizeof(float) + 255) & ~(size_t)255;
 }
 
 extern "C" size_t gad_cnn_workspace_bytes(int B, int H, int W, int Cm, int Co, int L) {
     CnnArgs a{};
     a.B = B, a.H = H, a.W = W, a.Cm = Cm, a.Co = Co, a.L = L, a.KH = (H == 1) ? 1 : 3;
-    bool in_smem;
-    cnn_plan(a, true, &in_smem);
-    const size_t grads = (size_t)B * (size_t)gad_cnn_param_count(H, Cm, Co, L) * sizeof(float);
-    return ((grads + 255) & ~(size_t)255) + (in_smem ? 0 : (size_t)B * cnn_act_floats(a) * sizeof(float)) + 256;
+    bool act_in_smem, grad_in_smem;
+    cnn_plan(a, true, &act_in_smem, &grad_in_smem);
+    return cnn_grads_bytes(a) + (act_in_smem ? 0 : (size_t)B * cnn_act_floats(a) * sizeof(float)) +
+           (grad_in_smem ? 0 : (size_t)B * cnn_grad_floats(a) * sizeof(float)) + 256;
 }
 
 extern "C" int gad_cnn_fwd(const float* u, const int32_t* gather, const float* scale, int B, int H, int W, int Cm, int Co,
@@ -274,8 +291,8 @@ extern "C" int gad_cnn_fwd(const float* u, const int32_t* gather, const float* s
     if (rc) return rc;
     GAD_CHECK_ARG(out, "gad_cnn_fwd: null output");
     a.out = out;
-    bool in_smem;
-    const size_t bytes = cnn_plan(a, false, &in_smem);
+    bool in_smem, unused;
+    const size_t bytes = cnn_plan(a, false, &in_smem, &unused);
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "gad_cnn_fwd: a %d x %d grid with %d channels needs %zu B of shared "
                                                     "memory (> %d)", H, W, cnn_cmax(a), bytes, smem_optin_bytes());
     if (!in_smem) {
@@ -299,14 +316,16 @@ extern "C" int gad_cnn_bwd(const float* u, const int32_t* gather, const float* s
     GAD_CHECK_ARG(workspace_bytes >= gad_cnn_workspace_bytes(B, H, W, Cm, Co, L), "gad_cnn_bwd: workspace too small");
     a.g_out = g_out;
     a.g_part = reinterpret_cast<float*>(workspace);
-    bool in_smem;
-    const size_t bytes = cnn_plan(a, true, &in_smem);
+    bool act_in_smem, grad_in_smem;
+    const size_t bytes = cnn_plan(a, true, &act_in_smem, &grad_in_smem);
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "gad_cnn_bwd: a %d x %d grid with %d channels needs %zu B of shared "
                                                     "memory (> %d)", H, W, cnn_cmax(a), bytes, smem_optin_bytes());
-    if (!in_smem) {
-        const size_t grads = ((size_t)B * a.n_params * sizeof(float) + 255) & ~(size_t)255;
-        a.act_global = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + grads);
+    char* next = reinterpret_cast<char*>(workspace) + cnn_grads_bytes(a);
+    if (!act_in_smem) {
+        a.act_global = reinterpret_cast<float*>(next);
+        next += (size_t)B * cnn_act_floats(a) * sizeof(float);
     }
+    if (!grad_in_smem) a.grad_global = reinterpret_cast<float*>(next);
     GAD_CUDA(cudaFuncSetAttribute(k_cnn_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
     cudaStream_t st = as_stream(stream);
     k_cnn_bwd<<<B, CNN_THREADS, bytes, st>>>(a);

@@ -130,6 +130,22 @@ __device__ __forceinline__ Row<CE> ldcg_gplus(const float* g, int64_t i, int gdi
     return r;
 }
 
+// p = M^T y + u with the per-mesh offset of the folded bias (global CNN features, include/gadapt.h): `dui` = the CE
+// floats du[mesh, lw] of the node's mesh, or null.  u + du is rounded before the products are added, as the mesh-resident
+// kernels do when they fold du into their shared copy of u (ell_kernels.cuh: load_mu), so every route rounds alike.
+template <int CE>
+__device__ __forceinline__ Row<CE> project_du(const float* __restrict__ Mu, const float* __restrict__ dui, const Row<CE>& x) {
+    if (!dui) return project<CE>(Mu, x);
+    Row<CE> p;
+#pragma unroll
+    for (int b = 0; b < CE; ++b) p.v[b] = Mu[CE * CE + b] + __ldg(dui + b);
+#pragma unroll
+    for (int a = 0; a < CE; ++a)
+#pragma unroll
+        for (int b = 0; b < CE; ++b) p.v[b] = fmaf(x.v[a], Mu[a * CE + b], p.v[b]);
+    return p;
+}
+
 // ---- wide rows from the (row-sorted) CSR / CSC walk arrays ---------------------------------------
 __global__ void __launch_bounds__(TB) k_build_wide(const int32_t* __restrict__ ptr, const int32_t* __restrict__ idx,
                                                    int64_t N, int4* __restrict__ rows, int32_t* __restrict__ bad) {
@@ -150,10 +166,12 @@ __global__ void __launch_bounds__(TB) k_build_wide(const int32_t* __restrict__ p
 
 // ---- forward stage (same contract as k_stage of stream_kernels.cu) -------------------------------
 //     k = F(y);  v = final ? acc_in + k : k;  out1 = base + c1 v;  out2 = acc_in + c2 k
+// du (or null): the bias offset of this weight set for mesh 0, du + m * du_stride for mesh m = i / nm.
 template <int CE, int W>
 __global__ void __launch_bounds__(TB) k_wide_stage(const int4* __restrict__ rows, int64_t N, const float* __restrict__ y,
                                                    const float* __restrict__ base, const float* __restrict__ acc_in,
-                                                   const float* __restrict__ Mu_g, const float* __restrict__ tau,
+                                                   const float* __restrict__ Mu_g, const float* __restrict__ du,
+                                                   int du_stride, int64_t nm, const float* __restrict__ tau,
                                                    float c1_scale, float c2, int final_stage, float* __restrict__ out1,
                                                    float* __restrict__ out2, float* __restrict__ xphys, int dim) {
     __shared__ float Mu[CE * CE + CE];
@@ -163,12 +181,13 @@ __global__ void __launch_bounds__(TB) k_wide_stage(const int4* __restrict__ rows
     if (i >= N) return;
     const Wide w = load_wide(rows, i);
     const float tau0 = tau ? __ldg(tau) : 1.0f;
+    const float* dui = du ? du + (i / nm) * du_stride : nullptr;
     // everything above is independent of the previous launch; everything below reads what it wrote
     chain_wait();
     chain_release();
     const Row<CE> yi = ldcg_row<CE>(y, i);
     // ---- F(y) at node i: project, gather, softmax, aggregate (ell_math.cuh: ell_feval) ----
-    const Row<CE> p = project<CE>(Mu, yi);
+    const Row<CE> p = project_du<CE>(Mu, dui, yi);
     Row<CE> xj[W];
     float s[W];
     float m = -3.0e38f;
@@ -297,9 +316,9 @@ __device__ __forceinline__ void sts_row(float* sm, int j, const Row<CE>& r) {
 
 // F(y) at one node, neighbours at LOCAL window indices (same expression order as k_wide_stage)
 template <int CE, int W>
-__device__ __forceinline__ Row<CE> window_feval(const float* Mu, const int* nbl, int valid, const float* ysm,
-                                                const Row<CE>& yi) {
-    const Row<CE> p = project<CE>(Mu, yi);
+__device__ __forceinline__ Row<CE> window_feval(const float* Mu, const float* dui, const int* nbl, int valid,
+                                                const float* ysm, const Row<CE>& yi) {
+    const Row<CE> p = project_du<CE>(Mu, dui, yi);
     Row<CE> xj[W];
     float s[W];
     float m = -3.0e38f;
@@ -331,7 +350,8 @@ __device__ __forceinline__ Row<CE> window_feval(const float* Mu, const int* nbl,
 #endif
 template <int CE, int W>
 __global__ void __launch_bounds__(TB, GAD_PERSIST_MINB) k_wide_persist(const int4* __restrict__ rows, int64_t N, int r,
-                                                     const float* __restrict__ x0, const float* __restrict__ Mu_g, int Lw,
+                                                     const float* __restrict__ x0, const float* __restrict__ Mu_g,
+                                                     const float* __restrict__ du, int64_t nm, int Lw,
                                                      const float* __restrict__ tau, int L, int method, float* tbuf0,
                                                      float* tbuf1, float* states, float* __restrict__ xphys, int dim) {
     constexpr int MUSZ = CE * CE + CE;
@@ -450,6 +470,7 @@ __global__ void __launch_bounds__(TB, GAD_PERSIST_MINB) k_wide_persist(const int
     const int per_step = rk4 ? 4 : 1, E = L * per_step;
     Row<CE> y = x, acc = zero_row<CE>();
     float tau0 = 0.f;
+    const float* dui = nullptr;                              // bias offset of this node's mesh and the current weight set
 #pragma unroll 1
     for (int e = 0; e < E; ++e) {
         const int l = rk4 ? (e >> 2) : e, sg = rk4 ? (e & 3) : 3;
@@ -458,10 +479,11 @@ __global__ void __launch_bounds__(TB, GAD_PERSIST_MINB) k_wide_persist(const int
                 __syncthreads();
                 for (int t = threadIdx.x; t < MUSZ; t += blockDim.x) Mu[t] = Mu_g[(size_t)(Lw > 1 ? l : 0) * MUSZ + t];
                 __syncthreads();
+                if (du) dui = du + ((ic / nm) * Lw + (Lw > 1 ? l : 0)) * CE;
             }
             tau0 = __ldg(tau + l);
         }
-        const Row<CE> k = window_feval<CE, W>(Mu, nbl, valid, ysm, y);
+        const Row<CE> k = window_feval<CE, W>(Mu, dui, nbl, valid, ysm, y);
         if (sg < 3) {
             const float c1 = tau0 * (sg == 2 ? 1.0f : 0.5f), c2 = (sg == 0 ? 1.0f : 2.0f);
 #pragma unroll
@@ -493,10 +515,12 @@ __global__ void __launch_bounds__(TB, GAD_PERSIST_MINB) k_wide_persist(const int
 template <int CE, int W>
 __global__ void __launch_bounds__(TB) k_wide_bwd_dst(const int4* __restrict__ rows, int64_t N, const float* __restrict__ x,
                                                      const float* __restrict__ gplus, int gplus_dim,
-                                                     const float* __restrict__ Mu_g, const float* __restrict__ tau,
+                                                     const float* __restrict__ Mu_g, const float* __restrict__ du,
+                                                     int du_stride, int64_t nm, const float* __restrict__ tau,
                                                      float a_coef, float* __restrict__ P, float2* __restrict__ DL,
                                                      float* __restrict__ gself, float* __restrict__ partials,
-                                                     int accumulate, float* __restrict__ tau_part, int tau_stride) {
+                                                     int accumulate, float* __restrict__ tau_part, int tau_stride,
+                                                     float* __restrict__ trows) {
     constexpr int NACC = CE * CE + CE + 1;
     __shared__ float Mu[CE * CE + CE];
     __shared__ float red[NACC * (TB / 32)];
@@ -511,7 +535,7 @@ __global__ void __launch_bounds__(TB) k_wide_bwd_dst(const int4* __restrict__ ro
         const Wide w = load_wide(rows, i);
         const Row<CE> xi = ldg_row<CE>(x, i);
         const bool any = w.nb[7] != 0;
-        const Row<CE> p = project<CE>(Mu, xi);
+        const Row<CE> p = project_du<CE>(Mu, du ? du + (i / nm) * du_stride : nullptr, xi);
         Row<CE> xj[W];
         float s[W];
         float m = -3.0e38f;
@@ -561,6 +585,15 @@ __global__ void __launch_bounds__(TB) k_wide_bwd_dst(const int4* __restrict__ ro
             for (int bb = 0; bb < CE; ++bb) acc[aa * CE + bb] = fmaf(xi.v[aa], t.v[bb], acc[aa * CE + bb]);
 #pragma unroll
         for (int bb = 0; bb < CE; ++bb) acc[CE * CE + bb] += t.v[bb];
+        if (trows) {   // t_i of every pass of the weight set, summed per node: d loss / d du of its mesh (k_wide_du_reduce)
+            Row<CE> tt = t;
+            if (accumulate) {
+                const Row<CE> prev = ldcg_row<CE>(trows, i);
+#pragma unroll
+                for (int c = 0; c < CE; ++c) tt.v[c] = prev.v[c] + t.v[c];
+            }
+            store_row<CE>(trows, i, tt);
+        }
         const Row<CE> Mt = apply_M<CE>(Mu, t);
         Row<CE> gs;
 #pragma unroll
@@ -658,6 +691,33 @@ __global__ void k_wide_reduce(const float* __restrict__ partials, int rows, int 
     if (lane == 0) out[k] = accumulate ? out[k] + (float)s : (float)s;
 }
 
+// d loss / d du[b, lw] = sum of the t rows of mesh b (nodes b nm .. (b + 1) nm - 1): one CTA per mesh, lane-strided fp64
+// sums and a fixed-order tree over the block -- the same bits every run.
+template <int CE>
+__global__ void __launch_bounds__(TB) k_wide_du_reduce(const float* __restrict__ trows, int64_t nm, int Lw, int lw,
+                                                       float* __restrict__ g_du) {
+    __shared__ double red[TB][CE];
+    const int b = blockIdx.x, tid = threadIdx.x;
+    double s[CE];
+#pragma unroll
+    for (int c = 0; c < CE; ++c) s[c] = 0.0;
+    for (int64_t i = tid; i < nm; i += TB) {
+        const Row<CE> t = load_row<CE>(trows, (int64_t)b * nm + i);
+#pragma unroll
+        for (int c = 0; c < CE; ++c) s[c] += (double)t.v[c];
+    }
+#pragma unroll
+    for (int c = 0; c < CE; ++c) red[tid][c] = s[c];
+    __syncthreads();
+    for (int w = TB / 2; w > 0; w >>= 1) {
+        if (tid < w)
+#pragma unroll
+            for (int c = 0; c < CE; ++c) red[tid][c] += red[tid + w][c];
+        __syncthreads();
+    }
+    if (tid < CE) g_du[((size_t)b * Lw + lw) * CE + tid] = (float)red[0][tid];
+}
+
 int grid_for_partials(int64_t N) {
     const int64_t want = (N + TB - 1) / TB;
     const int64_t cap = (int64_t)sm_count() * 8;
@@ -715,8 +775,9 @@ int persist_capacity_t(int64_t reach, int64_t* nodes) {
 int slots_for(int max_deg) { return max_deg <= 2 ? 2 : (max_deg <= 3 ? 3 : (max_deg <= 6 ? 6 : 7)); }
 
 template <int CE, int W>
-int wide_forward_t(const int4* rows, int64_t N, int64_t reach, const float* x0, int dim, const float* Mu, int Lw,
-                   const float* tau, int L, int method, float* x_phys, float* states, float* ws, cudaStream_t st) {
+int wide_forward_t(const int4* rows, int64_t N, int64_t reach, const float* x0, int dim, const float* Mu, const float* du,
+                   int64_t nm, int Lw, const float* tau, int L, int method, float* x_phys, float* states, float* ws,
+                   cudaStream_t st) {
     const size_t row = (size_t)N * CE;
     const int MUSZ = CE * CE + CE;
     const size_t rowa = align_up(row, 64);
@@ -744,31 +805,33 @@ int wide_forward_t(const int4* rows, int64_t N, int64_t reach, const float* x0, 
         attr[0].val.cooperative = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_wide_persist<CE, W>, rows, N, r, x0, Mu, Lw, tau, L, method, tb0, tb1, states,
-                                    x_phys, dim));
+        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_wide_persist<CE, W>, rows, N, r, x0, Mu, du, nm, Lw, tau, L, method, tb0, tb1,
+                                    states, x_phys, dim));
         count_launch(1);
         return GAD_OK;
     }
+    const int dus = Lw * CE;
     for (int l = 0; l < L; ++l) {
         const float* Mul = Mu + (size_t)(Lw > 1 ? l : 0) * MUSZ;
+        const float* dul = du ? du + (size_t)(Lw > 1 ? l : 0) * CE : nullptr;
         const float* tl = tau + l;
         const bool last = (l == L - 1);
         float* nxt = last ? nullptr : (states ? states + (size_t)(l + 1) * row : ping[l & 1]);
         float* xp = last ? x_phys : nullptr;
         if (method == GAD_METHOD_EULER) {
-            GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, l > 0, rows, N, cur, cur, (const float*)nullptr, Mul, tl, 1.0f,
-                                 0.f, 0, nxt, (float*)nullptr, xp, dim));
+            GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, l > 0, rows, N, cur, cur, (const float*)nullptr, Mul, dul, dus, nm,
+                                 tl, 1.0f, 0.f, 0, nxt, (float*)nullptr, xp, dim));
             count_launch(1);
         } else {
             // classical RK4 on F(y) = A(y) y - y (stream_kernels.cu: stream_forward)
-            GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, l > 0, rows, N, cur, cur, (const float*)nullptr, Mul, tl, 0.5f,
-                                 1.0f, 0, ybuf, abuf, (float*)nullptr, dim));
+            GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, l > 0, rows, N, cur, cur, (const float*)nullptr, Mul, dul, dus, nm,
+                                 tl, 0.5f, 1.0f, 0, ybuf, abuf, (float*)nullptr, dim));
             GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, true, rows, N, (const float*)ybuf, cur, (const float*)abuf,
-                                 Mul, tl, 0.5f, 2.0f, 0, y3buf, abuf, (float*)nullptr, dim));
+                                 Mul, dul, dus, nm, tl, 0.5f, 2.0f, 0, y3buf, abuf, (float*)nullptr, dim));
             GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, true, rows, N, (const float*)y3buf, cur, (const float*)abuf,
-                                 Mul, tl, 1.0f, 2.0f, 0, ybuf, abuf, (float*)nullptr, dim));
+                                 Mul, dul, dus, nm, tl, 1.0f, 2.0f, 0, ybuf, abuf, (float*)nullptr, dim));
             GAD_CUDA(launch_link(k_wide_stage<CE, W>, G, st, true, rows, N, (const float*)ybuf, cur, (const float*)abuf,
-                                 Mul, tl, 1.0f / 6.0f, 0.f, 1, nxt, (float*)nullptr, xp, dim));
+                                 Mul, dul, dus, nm, tl, 1.0f / 6.0f, 0.f, 1, nxt, (float*)nullptr, xp, dim));
             count_launch(4);
         }
         cur = nxt;
@@ -778,8 +841,8 @@ int wide_forward_t(const int4* rows, int64_t N, int64_t reach, const float* x0, 
 
 template <int CE, int W>
 int wide_backward_t(const int4* rows_in, const int4* rows_out, int64_t N, const float* states, const float* g_xphys,
-                    int dim, const float* Mu, int Lw, const float* tau, int L, float* gMu, float* g_tau, float* g_x0,
-                    float* ws, cudaStream_t st) {
+                    int dim, const float* Mu, const float* du, int M, int Lw, const float* tau, int L, float* gMu,
+                    float* g_tau, float* g_x0, float* g_du, float* ws, cudaStream_t st) {
     constexpr int NACC = CE * CE + CE + 1;
     const int MUSZ = CE * CE + CE;
     const size_t row = (size_t)N * CE;
@@ -798,15 +861,21 @@ int wide_backward_t(const int4* rows_in, const int4* rows_out, int64_t N, const 
     // dependent launches; the workspace holds WIDE_TAU_LAYERS columns.
     const bool defer_tau = g_tau && L <= WIDE_TAU_LAYERS;
     float* taup = partials + align_up((size_t)G * NACC, 64);
+    // per-node t rows of the passes of one weight set (d loss / d du, reduced per mesh): after the step-size columns
+    float* trows = g_du ? taup + (size_t)G * WIDE_TAU_LAYERS : nullptr;
+    const int64_t nm = N / M;
+    const int dus = Lw * CE;
     bool first = true;
     for (int l = L - 1; l >= 0; --l) {
         const float* Mul = Mu + (size_t)(Lw > 1 ? l : 0) * MUSZ;
+        const float* dul = du ? du + (size_t)(Lw > 1 ? l : 0) * CE : nullptr;
         const float* xl = states + (size_t)l * row;
         const float* tl = tau + l;
         float* gout = (l == 0 && g_x0) ? g_x0 : gping[l & 1];
         const bool shared_w = (Lw == 1);
-        GAD_CUDA(launch_link(k_wide_bwd_dst<CE, W>, (unsigned)G, st, !first, rows_in, N, xl, gcur, gdim, Mul, tl, 1.0f, P, DL,
-                             gself, partials, (shared_w && l < L - 1) ? 1 : 0, defer_tau ? taup + l : (float*)nullptr, L));
+        GAD_CUDA(launch_link(k_wide_bwd_dst<CE, W>, (unsigned)G, st, !first, rows_in, N, xl, gcur, gdim, Mul, dul, dus, nm,
+                             tl, 1.0f, P, DL, gself, partials, (shared_w && l < L - 1) ? 1 : 0,
+                             defer_tau ? taup + l : (float*)nullptr, L, trows));
         count_launch(1);
         first = false;
         if (l > 0 || g_x0) {
@@ -817,6 +886,10 @@ int wide_backward_t(const int4* rows_in, const int4* rows_out, int64_t N, const 
         if (!shared_w || l == 0) {   // shared weights: one reduction of the accumulated partials at the end
             k_wide_reduce<<<(MUSZ + 7) / 8, 256, 0, st>>>(partials, G, MUSZ, NACC, gMu + (size_t)(shared_w ? 0 : l) * MUSZ, 1);
             GAD_LAUNCH_CHECK();
+            if (trows) {
+                k_wide_du_reduce<CE><<<M, TB, 0, st>>>(trows, nm, Lw, shared_w ? 0 : l, g_du);
+                GAD_LAUNCH_CHECK();
+            }
         }
         if (g_tau && !defer_tau) {
             k_wide_reduce<<<1, 32, 0, st>>>(partials + MUSZ, G, 1, NACC, g_tau + l, 0);
@@ -843,7 +916,8 @@ using namespace gad;
 
 size_t wide_bwd_rk4_ws_floats(int64_t N, int CE) {
     const int NACC = CE * CE + CE + 1;
-    return align_up((size_t)N * CE, 64) * 9 + align_up(2 * (size_t)N, 64) +
+    // nine state rows, DL, the per-block partials, the per-node t rows of d loss / d du
+    return align_up((size_t)N * CE, 64) * 10 + align_up(2 * (size_t)N, 64) +
            align_up((size_t)grid_for_partials(N) * NACC, 64) + 64;
 }
 
@@ -856,8 +930,8 @@ size_t wide_bwd_rk4_ws_floats(int64_t N, int CE) {
 // gradient (learn_step is an Euler feature, as in k_ell_bwd_rk4).
 template <int CE, int W>
 int wide_backward_rk4_t(const int4* rows_in, const int4* rows_out, int64_t N, const float* states, const float* g_xphys,
-                        int dim, const float* Mu, int Lw, const float* tau, int L, float* gMu, float* g_x0, float* ws,
-                        cudaStream_t st) {
+                        int dim, const float* Mu, const float* du, int M, int Lw, const float* tau, int L, float* gMu,
+                        float* g_x0, float* g_du, float* ws, cudaStream_t st) {
     constexpr int NACC = CE * CE + CE + 1;
     const int MUSZ = CE * CE + CE;
     const size_t row = (size_t)N * CE;
@@ -872,6 +946,9 @@ int wide_backward_rk4_t(const int4* rows_in, const int4* rows_out, int64_t N, co
     float* yb[3] = {ws + 6 * rowa, ws + 7 * rowa, ws + 8 * rowa};       // y2, y3, y4
     float2* DL = reinterpret_cast<float2*>(ws + 9 * rowa);
     float* partials = ws + 9 * rowa + align_up(2 * (size_t)N, 64);
+    float* trows = g_du ? partials + align_up((size_t)G * NACC, 64) : nullptr;
+    const int64_t nm = N / M;
+    const int dus = Lw * CE;
     GAD_CUDA(cudaMemsetAsync(gMu, 0, (size_t)Lw * MUSZ * sizeof(float), st));
     const float* gcur = g_xphys;
     int gdim = dim;
@@ -880,14 +957,15 @@ int wide_backward_rk4_t(const int4* rows_in, const int4* rows_out, int64_t N, co
     static const float ca_g[4] = {1.0f / 6.0f, 1.0f / 3.0f, 1.0f / 3.0f, 1.0f / 6.0f};      // of a1 .. a4
     for (int l = L - 1; l >= 0; --l) {
         const float* Mul = Mu + (size_t)(Lw > 1 ? l : 0) * MUSZ;
+        const float* dul = du ? du + (size_t)(Lw > 1 ? l : 0) * CE : nullptr;
         const float* xl = states + (size_t)l * row;
         const float* tl = tau + l;
         float* gs = (l == 0 && g_x0) ? g_x0 : gsb[l & 1];
         // stage inputs: y2 = x + tau/2 F(x), y3 = x + tau/2 F(y2), y4 = x + tau F(y3)
         const float* yin = xl;
         for (int sgi = 0; sgi < 3; ++sgi) {
-            GAD_CUDA(launch_link(k_wide_stage<CE, W>, GN, st, false, rows_in, N, yin, xl, (const float*)nullptr, Mul, tl,
-                                 sgi == 2 ? 1.0f : 0.5f, 0.f, 0, yb[sgi], (float*)nullptr, (float*)nullptr, dim));
+            GAD_CUDA(launch_link(k_wide_stage<CE, W>, GN, st, false, rows_in, N, yin, xl, (const float*)nullptr, Mul, dul, dus,
+                                 nm, tl, sgi == 2 ? 1.0f : 0.5f, 0.f, 0, yb[sgi], (float*)nullptr, (float*)nullptr, dim));
             yin = yb[sgi];
         }
         count_launch(3);
@@ -896,8 +974,8 @@ int wide_backward_rk4_t(const int4* rows_in, const int4* rows_out, int64_t N, co
         GAD_LAUNCH_CHECK();
         for (int sgi = 3; sgi >= 0; --sgi) {
             const float* ys = sgi == 0 ? xl : yb[sgi - 1];
-            GAD_CUDA(launch_link(k_wide_bwd_dst<CE, W>, (unsigned)G, st, false, rows_in, N, ys, (const float*)a, CE, Mul, tl,
-                                 0.0f, P, DL, gself, partials, first_of_set ? 0 : 1, (float*)nullptr, 0));
+            GAD_CUDA(launch_link(k_wide_bwd_dst<CE, W>, (unsigned)G, st, false, rows_in, N, ys, (const float*)a, CE, Mul, dul,
+                                 dus, nm, tl, 0.0f, P, DL, gself, partials, first_of_set ? 0 : 1, (float*)nullptr, 0, trows));
             first_of_set = false;
             GAD_CUDA(launch_link(k_wide_bwd_src<CE, W>, GN, st, false, rows_out, N, ys, (const float*)a, CE, tl,
                                  (const float*)P, (const float2*)DL, (const float*)gself, gy));
@@ -910,6 +988,10 @@ int wide_backward_rk4_t(const int4* rows_in, const int4* rows_out, int64_t N, co
         if (!shared_w || l == 0) {
             k_wide_reduce<<<(MUSZ + 7) / 8, 256, 0, st>>>(partials, G, MUSZ, NACC, gMu + (size_t)(shared_w ? 0 : l) * MUSZ, 1);
             GAD_LAUNCH_CHECK();
+            if (trows) {
+                k_wide_du_reduce<CE><<<M, TB, 0, st>>>(trows, nm, Lw, shared_w ? 0 : l, g_du);
+                GAD_LAUNCH_CHECK();
+            }
         }
         gcur = gs;
         gdim = CE;
@@ -941,9 +1023,14 @@ extern "C" int gad_graph_build_wide(const int32_t* ptr, const int32_t* idx, int6
     return GAD_OK;
 }
 
+// The per-mesh bias offset du [M, Lw, CE] (NULL: none) of the streaming entry points: M meshes of N / M nodes each,
+// node i in mesh i / (N / M).
+#define GAD_WIDE_CHECK_DU(FN)                                                                                      \
+    GAD_CHECK_ARG(!du || (M > 0 && N % M == 0), FN ": du needs M > 0 meshes of equal size (N=%lld, M=%d)", (long long)N, M)
+
 extern "C" int gad_deform_fwd_wide(const void* wide_in, int64_t N, int max_deg, int64_t reach, const float* x0, int dim, int CE,
-                                   const float* Mu, int Lw, const float* tau, int L, int method, float* x_phys,
-                                   float* states, void* workspace, size_t workspace_bytes, void* stream) {
+                                   const float* Mu, const float* du, int M, int Lw, const float* tau, int L, int method,
+                                   float* x_phys, float* states, void* workspace, size_t workspace_bytes, void* stream) {
     GAD_CHECK_ARG(wide_in && x0 && Mu && tau && x_phys && workspace, "gad_deform_fwd_wide: null pointer");
     GAD_CHECK_ARG(N > 0 && L > 0 && dim >= 1 && dim <= CE && (Lw == 1 || Lw == L) && max_deg >= 0 && max_deg <= WIDE_SLOTS,
                   "gad_deform_fwd_wide: N=%lld L=%d dim=%d CE=%d Lw=%d max_deg=%d", (long long)N, L, dim, CE, Lw, max_deg);
@@ -951,10 +1038,12 @@ extern "C" int gad_deform_fwd_wide(const void* wide_in, int64_t N, int max_deg, 
     GAD_CHECK_ARG(!states || states == x0, "gad_deform_fwd_wide: when states is given, x0 must alias states[0]");
     GAD_CHECK_ARG(workspace_bytes >= stream_fwd_ws_floats(N, CE, method) * sizeof(float),
                   "gad_deform_fwd_wide: workspace too small");
+    GAD_WIDE_CHECK_DU("gad_deform_fwd_wide");
     const int4* rows = reinterpret_cast<const int4*>(wide_in);
     float* ws = reinterpret_cast<float*>(workspace);
     cudaStream_t st = as_stream(stream);
-    GAD_WIDE_DISPATCH(wide_forward_t, rows, N, reach, x0, dim, Mu, Lw, tau, L, method, x_phys, states, ws, st);
+    const int64_t nm = du ? N / M : N;
+    GAD_WIDE_DISPATCH(wide_forward_t, rows, N, reach, x0, dim, Mu, du, nm, Lw, tau, L, method, x_phys, states, ws, st);
 }
 
 extern "C" size_t gad_deform_bwd_wide_rk4_workspace_bytes(int64_t N, int CE) {
@@ -962,20 +1051,23 @@ extern "C" size_t gad_deform_bwd_wide_rk4_workspace_bytes(int64_t N, int CE) {
 }
 
 extern "C" int gad_deform_bwd_wide_rk4(const void* wide_in, const void* wide_out, int64_t N, int max_deg,
-                                       const float* states, const float* g_xphys, int dim, int CE, const float* Mu, int Lw,
-                                       const float* tau, int L, float* gMu, float* g_x0, void* workspace,
-                                       size_t workspace_bytes, void* stream) {
+                                       const float* states, const float* g_xphys, int dim, int CE, const float* Mu,
+                                       const float* du, int M, int Lw, const float* tau, int L, float* gMu, float* g_x0,
+                                       float* g_du, void* workspace, size_t workspace_bytes, void* stream) {
     GAD_CHECK_ARG(wide_in && wide_out && states && g_xphys && Mu && tau && gMu && workspace,
                   "gad_deform_bwd_wide_rk4: null pointer");
     GAD_CHECK_ARG(N > 0 && L > 0 && dim >= 1 && dim <= CE && (Lw == 1 || Lw == L) && max_deg >= 0 && max_deg <= WIDE_SLOTS,
                   "gad_deform_bwd_wide_rk4: N=%lld L=%d dim=%d CE=%d Lw=%d max_deg=%d", (long long)N, L, dim, CE, Lw, max_deg);
     GAD_CHECK_ARG(workspace_bytes >= wide_bwd_rk4_ws_floats(N, CE) * sizeof(float),
                   "gad_deform_bwd_wide_rk4: workspace too small");
+    GAD_WIDE_CHECK_DU("gad_deform_bwd_wide_rk4");
+    GAD_CHECK_ARG(!g_du || du, "gad_deform_bwd_wide_rk4: g_du needs the bias offset du of the forward");
     const int4* rin = reinterpret_cast<const int4*>(wide_in);
     const int4* rout = reinterpret_cast<const int4*>(wide_out);
     float* ws = reinterpret_cast<float*>(workspace);
     cudaStream_t st = as_stream(stream);
-    GAD_WIDE_DISPATCH(wide_backward_rk4_t, rin, rout, N, states, g_xphys, dim, Mu, Lw, tau, L, gMu, g_x0, ws, st);
+    GAD_WIDE_DISPATCH(wide_backward_rk4_t, rin, rout, N, states, g_xphys, dim, Mu, du, du ? M : 1, Lw, tau, L, gMu, g_x0, g_du,
+                      ws, st);
 }
 
 extern "C" int64_t gad_wide_persist_nodes(int CE, int max_deg, int64_t reach) {
@@ -986,17 +1078,20 @@ extern "C" int64_t gad_wide_persist_nodes(int CE, int max_deg, int64_t reach) {
 }
 
 extern "C" int gad_deform_bwd_wide(const void* wide_in, const void* wide_out, int64_t N, int max_deg,
-                                   const float* states, const float* g_xphys, int dim, int CE, const float* Mu, int Lw,
-                                   const float* tau, int L, float* gMu, float* g_tau, float* g_x0, void* workspace,
-                                   size_t workspace_bytes, void* stream) {
+                                   const float* states, const float* g_xphys, int dim, int CE, const float* Mu,
+                                   const float* du, int M, int Lw, const float* tau, int L, float* gMu, float* g_tau,
+                                   float* g_x0, float* g_du, void* workspace, size_t workspace_bytes, void* stream) {
     GAD_CHECK_ARG(wide_in && wide_out && states && g_xphys && Mu && tau && gMu && workspace,
                   "gad_deform_bwd_wide: null pointer");
     GAD_CHECK_ARG(N > 0 && L > 0 && dim >= 1 && dim <= CE && (Lw == 1 || Lw == L) && max_deg >= 0 && max_deg <= WIDE_SLOTS,
                   "gad_deform_bwd_wide: N=%lld L=%d dim=%d CE=%d Lw=%d max_deg=%d", (long long)N, L, dim, CE, Lw, max_deg);
     GAD_CHECK_ARG(workspace_bytes >= stream_bwd_ws_floats(N, CE) * sizeof(float), "gad_deform_bwd_wide: workspace too small");
+    GAD_WIDE_CHECK_DU("gad_deform_bwd_wide");
+    GAD_CHECK_ARG(!g_du || du, "gad_deform_bwd_wide: g_du needs the bias offset du of the forward");
     const int4* rin = reinterpret_cast<const int4*>(wide_in);
     const int4* rout = reinterpret_cast<const int4*>(wide_out);
     float* ws = reinterpret_cast<float*>(workspace);
     cudaStream_t st = as_stream(stream);
-    GAD_WIDE_DISPATCH(wide_backward_t, rin, rout, N, states, g_xphys, dim, Mu, Lw, tau, L, gMu, g_tau, g_x0, ws, st);
+    GAD_WIDE_DISPATCH(wide_backward_t, rin, rout, N, states, g_xphys, dim, Mu, du, du ? M : 1, Lw, tau, L, gMu, g_tau, g_x0,
+                      g_du, ws, st);
 }

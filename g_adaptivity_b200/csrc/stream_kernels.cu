@@ -365,9 +365,10 @@ size_t stream_fwd_ws_floats(int64_t N, int CE, int method) {
 
 size_t stream_bwd_ws_floats(int64_t N, int CE) {
     const int NACC = CE * CE + CE + 1;
-    // last term: per-layer step-size partials of the streaming ELL backward (stream_ell.cu: WIDE_TAU_LAYERS = 64)
+    // last terms: per-layer step-size partials of the streaming ELL backward (stream_ell.cu: WIDE_TAU_LAYERS = 64), then
+    // its per-node t rows of d loss / d du
     const size_t G = (size_t)stream_grid_for_partials(N);
-    return align_up((size_t)N * CE, 64) * 4 + align_up(2 * (size_t)N, 64) + align_up(G * NACC, 64) + 64 + G * 64;
+    return align_up((size_t)N * CE, 64) * 5 + align_up(2 * (size_t)N, 64) + align_up(G * NACC, 64) + 64 + G * 64;
 }
 
 }  // namespace gad

@@ -126,9 +126,9 @@ def pack_features(x_comp, f, uu, f_scale, uu_scale, CE: int, out: Optional[torch
 
 def deform_forward(graph: MeshGraph, x0: torch.Tensor, dim: int, Mu: torch.Tensor, tau: torch.Tensor,
                    method: int = METHOD_EULER, states: Optional[torch.Tensor] = None,
-                   force_stream: bool = False) -> torch.Tensor:
+                   force_stream: bool = False, du: Optional[torch.Tensor] = None) -> torch.Tensor:
     """x0 [N, CE] -> x_phys [N, dim].  `states` ([L, N, CE], states[0] aliasing x0) receives the
-    layer inputs x^0..x^{L-1} for the backward."""
+    layer inputs x^0..x^{L-1} for the backward.  `du` [meshes, Lw, CE]: per-mesh bias offset (see _check_du)."""
     _need_cuda(x0, Mu, tau)
     lib = _lib.load()
     N, CE = x0.shape
@@ -136,6 +136,11 @@ def deform_forward(graph: MeshGraph, x0: torch.Tensor, dim: int, Mu: torch.Tenso
     assert graph.N == N
     x_phys = torch.empty((N, dim), dtype=torch.float32, device=x0.device)
     use_tiles = graph.tile_ptr is not None and not force_stream
+    if du is not None:
+        _check_du(graph, du, CE, Lw, force_stream)
+        if use_tiles:
+            raise NotImplementedError("deform_forward takes the bias offset on the streaming kernels only; "
+                                      "use deform_forward_raw on mesh-resident graphs")
     if use_tiles and use_ell(graph, CE):
         with _on_device(x0.device):
             _lib.check(lib.gad_deform_fwd_ell(
@@ -146,13 +151,15 @@ def deform_forward(graph: MeshGraph, x0: torch.Tensor, dim: int, Mu: torch.Tenso
     ws = None
     ws_bytes = 0
     if not use_tiles:
+        _need_wide(graph, CE, du)
         ws_bytes = lib.gad_deform_workspace_bytes(N, CE, method)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x0.device)
         if graph.ensure_wide(CE):      # streaming ELL kernels (csrc/stream_ell.cu)
             with _on_device(x0.device):
                 _lib.check(lib.gad_deform_fwd_wide(
-                    _lib.ptr(graph.wide_in), N, graph.wide_deg, graph.wide_reach, _lib.ptr(x0), dim, CE, _lib.ptr(Mu), Lw,
-                    _lib.ptr(tau), L, method, _lib.ptr(x_phys), _lib.ptr(states), _lib.ptr(ws), ws_bytes, _stream(x0)), "gad_deform_fwd_wide")
+                    _lib.ptr(graph.wide_in), N, graph.wide_deg, graph.wide_reach, _lib.ptr(x0), dim, CE, _lib.ptr(Mu),
+                    _lib.ptr(du), _n_meshes(graph, du), Lw, _lib.ptr(tau), L, method, _lib.ptr(x_phys), _lib.ptr(states),
+                    _lib.ptr(ws), ws_bytes, _stream(x0)), "gad_deform_fwd_wide")
             return x_phys
     with _on_device(x0.device):
         _lib.check(lib.gad_deform_fwd(
@@ -170,13 +177,35 @@ def fold_scale(inv_temp: float, C: int) -> float:
 
 
 def _check_du(graph: MeshGraph, du: torch.Tensor, CE: int, Lw: int, force_stream: bool):
-    """Per-tile bias offsets (global CNN features) need the mesh-resident ELL kernels with one mesh per tile."""
-    if force_stream or graph.tile_ptr is None or not use_ell(graph, CE):
-        raise NotImplementedError("global CNN features (per-mesh bias offset) run on the mesh-resident ELL kernels only")
-    if graph.mesh_sizes is None or graph.T != len(graph.mesh_sizes):
-        raise NotImplementedError("global CNN features need one mesh per tile (the module plans tiles that way)")
-    if tuple(du.shape) != (graph.T, Lw, CE) or du.dtype != torch.float32 or not du.is_contiguous():
-        raise ValueError(f"du must be a contiguous float32 [{graph.T}, {Lw}, {CE}] tensor, got {tuple(du.shape)}")
+    """Per-mesh bias offsets du [meshes, Lw, CE] (global CNN features, include/gadapt.h) run on the mesh-resident ELL
+    kernels with one mesh per tile, on the cluster kernels and on the streaming ELL kernels (meshes of one size); the
+    CSR kernels take none."""
+    if graph.mesh_sizes is None:
+        raise NotImplementedError("global CNN features need the batch's mesh sizes")
+    M = len(graph.mesh_sizes)
+    if graph.tile_ptr is not None and not force_stream:
+        if not use_ell(graph, CE):
+            raise NotImplementedError("global CNN features (per-mesh bias offset) do not run on the CSR mesh-resident "
+                                      "kernels (degree > 7 or CE = 8)")
+        if graph.T != M:
+            raise NotImplementedError("global CNN features need one mesh per tile (the module plans tiles that way)")
+    elif any(n != graph.mesh_sizes[0] for n in graph.mesh_sizes) or CE not in (2, 4) or max(graph.max_in_deg, graph.max_out_deg) > 7:
+        raise NotImplementedError("global CNN features on meshes beyond one CTA need meshes of equal size, degree <= 7 and "
+                                  "CE in {2, 4} (the CSR streaming kernels take no bias offset)")
+    if tuple(du.shape) != (M, Lw, CE) or du.dtype != torch.float32 or not du.is_contiguous():
+        raise ValueError(f"du must be a contiguous float32 [{M}, {Lw}, {CE}] tensor, got {tuple(du.shape)}")
+
+
+def _n_meshes(graph: MeshGraph, du: Optional[torch.Tensor]) -> int:
+    """The mesh count the streaming entry points take with `du` (0 without)."""
+    return len(graph.mesh_sizes) if du is not None else 0
+
+
+def _need_wide(graph: MeshGraph, CE: int, du: Optional[torch.Tensor]):
+    """With `du`, the streaming route must be the wide-row one: the CSR streaming kernels take no offset."""
+    if du is not None and not graph.ensure_wide(CE):
+        raise NotImplementedError("global CNN features (per-mesh bias offset) need the streaming ELL kernels "
+                                  "(degree <= 7, CE in {2, 4}); the CSR streaming kernels take none")
 
 
 def deform_forward_raw(graph: MeshGraph, x_comp, f, uu, f_scale, uu_scale, dim: int, CE: int, Mu: torch.Tensor,
@@ -207,13 +236,13 @@ def deform_forward_raw(graph: MeshGraph, x_comp, f, uu, f_scale, uu_scale, dim: 
             _lib.check(lib.gad_deform_fwd_cluster(
                 _lib.ptr(graph.clf_in), _lib.ptr(graph.clf_mesh_ptr), len(graph.mesh_sizes), max(graph.mesh_sizes),
                 graph.clf_deg, graph.clf_C, N, _lib.ptr(x_comp), _lib.ptr(f), _lib.ptr(uu), _lib.ptr(f_scale),
-                _lib.ptr(uu_scale), dim, CE, _lib.ptr(Mu), Lw, _lib.ptr(tau), L, method, _lib.ptr(x_phys), _lib.ptr(states),
-                _stream(x_comp)), "gad_deform_fwd_cluster")
+                _lib.ptr(uu_scale), dim, CE, _lib.ptr(Mu), _lib.ptr(du), Lw, _lib.ptr(tau), L, method, _lib.ptr(x_phys),
+                _lib.ptr(states), _stream(x_comp)), "gad_deform_fwd_cluster")
         return x_phys
     if not (graph.tile_ptr is not None and not force_stream and use_ell(graph, CE)):
         x0 = states[0] if states is not None else torch.empty((N, CE), dtype=torch.float32, device=x_comp.device)
         pack_features(x_comp, f, uu, f_scale, uu_scale, CE, out=x0)
-        return deform_forward(graph, x0, dim, Mu, tau, method, states=states, force_stream=force_stream)
+        return deform_forward(graph, x0, dim, Mu, tau, method, states=states, force_stream=force_stream, du=du)
     lib = _lib.load()
     # identity encoder with hidden < in_dim truncates (src/GNN.py:84-90): features beyond CE are dropped
     if f is not None and dim >= CE:
@@ -274,17 +303,15 @@ def deform_backward_rk4(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.T
     gMu = torch.empty_like(Mu)
     g_x0 = torch.empty((N, CE), dtype=torch.float32, device=dev) if want_gx0 else None
     if not rk4_backward_resident(graph, CE, force_stream):
-        if du is not None:
-            raise NotImplementedError("global CNN features reach the kernels as a per-tile bias offset: meshes that fit "
-                                      "a CTA only (backward through ode_method='rk4' on the streaming kernels has none)")
         ws_bytes = lib.gad_deform_bwd_wide_rk4_workspace_bytes(N, CE)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        g_du = torch.empty_like(du) if du is not None else None
         with _on_device(dev):
             _lib.check(lib.gad_deform_bwd_wide_rk4(
                 _lib.ptr(graph.wide_in), _lib.ptr(graph.wide_out), N, graph.wide_deg, _lib.ptr(states), _lib.ptr(g_xphys),
-                dim, CE, _lib.ptr(Mu), Lw, _lib.ptr(tau), L, _lib.ptr(gMu), _lib.ptr(g_x0), _lib.ptr(ws), ws_bytes,
-                _stream(states)), "gad_deform_bwd_wide_rk4")
-        return gMu, g_x0, None
+                dim, CE, _lib.ptr(Mu), _lib.ptr(du), _n_meshes(graph, du), Lw, _lib.ptr(tau), L, _lib.ptr(gMu),
+                _lib.ptr(g_x0), _lib.ptr(g_du), _lib.ptr(ws), ws_bytes, _stream(states)), "gad_deform_bwd_wide_rk4")
+        return gMu, g_x0, g_du
     ws_bytes = lib.gad_ell_workspace_bytes(CE, graph.T, L)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     with _on_device(dev):
@@ -300,7 +327,7 @@ def deform_backward_rk4(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.T
 def deform_backward(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.Tensor, dim: int, Mu: torch.Tensor,
                     tau: torch.Tensor, want_gtau: bool = False, want_gx0: bool = False, force_stream: bool = False,
                     du: Optional[torch.Tensor] = None):
-    """Cotangent of x_phys -> (gMu [Lw, CE*CE+CE], g_tau [L] | None, g_x0 [N, CE] | None[, g_du [T, Lw, CE]])."""
+    """Cotangent of x_phys -> (gMu [Lw, CE*CE+CE], g_tau [L] | None, g_x0 [N, CE] | None[, g_du [meshes, Lw, CE]])."""
     _need_cuda(states, g_xphys, Mu, tau)
     lib = _lib.load()
     L, N, CE = states.shape
@@ -324,8 +351,8 @@ def deform_backward(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.Tenso
         if du is not None:
             return gMu, g_tau, g_x0, _tile_bias_grads(ws, T, Lw, L, CE)
         return gMu, g_tau, g_x0
-    if du is not None:
-        raise NotImplementedError("global CNN features (per-mesh bias offset) run on the mesh-resident ELL kernels only")
+    g_du = torch.empty_like(du) if du is not None else None
+    done = (gMu, g_tau, g_x0) if du is None else (gMu, g_tau, g_x0, g_du)
     if (graph.tile_ptr is None and not force_stream and not getattr(graph, "_no_cluster", False)
             and graph.ensure_cluster(CE)):
         # meshes beyond one CTA (up to 4 slabs): cluster-resident backward, one launch + the reduction
@@ -335,19 +362,24 @@ def deform_backward(graph: MeshGraph, states: torch.Tensor, g_xphys: torch.Tenso
         with _on_device(dev):
             _lib.check(lib.gad_deform_bwd_cluster(
                 _lib.ptr(graph.cl_in), _lib.ptr(graph.cl_out), _lib.ptr(graph.mesh_ptr), M, max(graph.mesh_sizes),
-                graph.cl_deg, graph.cl_C, N, _lib.ptr(states), _lib.ptr(g_xphys), dim, CE, _lib.ptr(Mu), Lw, _lib.ptr(tau),
-                L, _lib.ptr(gMu), _lib.ptr(g_tau), _lib.ptr(g_x0), _lib.ptr(ws), ws_bytes, _stream(states)),
-                "gad_deform_bwd_cluster")
-        return gMu, g_tau, g_x0
+                graph.cl_deg, graph.cl_C, N, _lib.ptr(states), _lib.ptr(g_xphys), dim, CE, _lib.ptr(Mu), _lib.ptr(du), Lw,
+                _lib.ptr(tau), L, _lib.ptr(gMu), _lib.ptr(g_tau), _lib.ptr(g_x0), _lib.ptr(g_du), _lib.ptr(ws), ws_bytes,
+                _stream(states)), "gad_deform_bwd_cluster")
+        return done
     ws_bytes = lib.gad_deform_bwd_workspace_bytes(N, CE, T, L)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    if not use_tiles:
+        _need_wide(graph, CE, du)
     if not use_tiles and graph.ensure_wide(CE):
         with _on_device(dev):
             _lib.check(lib.gad_deform_bwd_wide(
                 _lib.ptr(graph.wide_in), _lib.ptr(graph.wide_out), N, graph.wide_deg, _lib.ptr(states), _lib.ptr(g_xphys),
-                dim, CE, _lib.ptr(Mu), Lw, _lib.ptr(tau), L, _lib.ptr(gMu), _lib.ptr(g_tau), _lib.ptr(g_x0), _lib.ptr(ws),
-                ws_bytes, _stream(states)), "gad_deform_bwd_wide")
-        return gMu, g_tau, g_x0
+                dim, CE, _lib.ptr(Mu), _lib.ptr(du), _n_meshes(graph, du), Lw, _lib.ptr(tau), L, _lib.ptr(gMu),
+                _lib.ptr(g_tau), _lib.ptr(g_x0), _lib.ptr(g_du), _lib.ptr(ws), ws_bytes, _stream(states)),
+                "gad_deform_bwd_wide")
+        return done
+    if du is not None:
+        raise NotImplementedError("global CNN features (per-mesh bias offset) do not run on the CSR kernels")
     with _on_device(dev):
         _lib.check(lib.gad_deform_bwd(
             _lib.ptr(graph.rowptr), _lib.ptr(graph.col_walk), _lib.ptr(graph.t_rowptr), _lib.ptr(graph.t_dst_walk), N, graph.E,

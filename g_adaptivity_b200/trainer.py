@@ -410,10 +410,12 @@ class DeformerTrainer:
         planning); anything else raises as the module path does."""
         if (self.opt.get("gad_force_stream", False) or not GF.use_ell(g, self.CE) or g.mesh_sizes is None
                 or g.T != len(g.mesh_sizes)):
-            raise NotImplementedError("global CNN features (per-mesh bias offset) run on the mesh-resident ELL kernels only")
+            raise NotImplementedError("DeformerTrainer trains global CNN features on the mesh-resident ELL kernels only "
+                                      "(meshes that fit a CTA); train larger batches through GNN.forward + autograd")
         if self.method == GF.METHOD_RK4 and not GF.rk4_backward_resident(g, self.CE):
-            raise NotImplementedError("global CNN features reach the kernels as a per-tile bias offset: meshes that fit "
-                                      "a CTA only (backward through ode_method='rk4' on the streaming kernels has none)")
+            raise NotImplementedError("DeformerTrainer trains global CNN features with ode_method='rk4' on meshes that fit "
+                                      "the mesh-resident RK4 backward only; train larger batches through GNN.forward + "
+                                      "autograd")
 
     def _pde_setup(self, s: "_Slot", data):
         """Refusals, FEM tables and buffers of a pde slot (loss_type='pde_loss'), from the helpers GNN.forward uses."""
@@ -576,8 +578,8 @@ class DeformerTrainer:
                                       P(s.states), stream_ptr), "gad_pack_features")
             wide = (not tiles) and g.ensure_wide(CE)      # streaming ELL kernels (csrc/stream_ell.cu)
             if wide:
-                chk(lib.gad_deform_fwd_wide(P(g.wide_in), s.N, g.wide_deg, g.wide_reach, P(s.states), dim, CE, P(self.Mu), Lw, P(self.tau), L,
-                                            self.method, P(s.x_phys), P(s.states), P(s.fwd_ws), s.fwd_ws_bytes, stream_ptr),
+                chk(lib.gad_deform_fwd_wide(P(g.wide_in), s.N, g.wide_deg, g.wide_reach, P(s.states), dim, CE, P(self.Mu), None, 0, Lw,
+                                            P(self.tau), L, self.method, P(s.x_phys), P(s.states), P(s.fwd_ws), s.fwd_ws_bytes, stream_ptr),
                     "gad_deform_fwd_wide")
             else:
                 chk(lib.gad_deform_fwd(P(g.rowptr), P(g.col_walk), s.N, g.E, P(g.tile_ptr) if tiles else None,
@@ -597,12 +599,12 @@ class DeformerTrainer:
                     "gad_deform_bwd_ell_rk4")
             elif self.method == GF.METHOD_RK4:
                 chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
-                                                dim, CE, P(self.Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
-                                                s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
+                                                dim, CE, P(self.Mu), None, 0, Lw, P(self.tau), L, P(self.gMu), None, None,
+                                                P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
             elif wide:
                 chk(lib.gad_deform_bwd_wide(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out), dim, CE,
-                                            P(self.Mu), Lw, P(self.tau), L, P(self.gMu), P(self.gtau), None, P(s.bwd_ws),
-                                            s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide")
+                                            P(self.Mu), None, 0, Lw, P(self.tau), L, P(self.gMu), P(self.gtau), None, None,
+                                            P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide")
             else:
                 chk(lib.gad_deform_bwd(P(g.rowptr), P(g.col_walk), P(g.t_rowptr), P(g.t_dst_walk), s.N, g.E,
                                        P(g.tile_ptr) if tiles else None, g.T if tiles else 0, g.max_tile_nodes,
@@ -667,8 +669,8 @@ class DeformerTrainer:
                                       P(s.g_out), P(s.loss_ws), stream_ptr), "gad_mesh_loss")
             if self.method == GF.METHOD_RK4 and not s.rk4_resident:
                 chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
-                                                dim, CE, P(Mu), Lw, P(self.tau), L, P(self.gMu), None, P(s.bwd_ws),
-                                                s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
+                                                dim, CE, P(Mu), None, 0, Lw, P(self.tau), L, P(self.gMu), None, None,
+                                                P(s.bwd_ws), s.bwd_ws_bytes, stream_ptr), "gad_deform_bwd_wide_rk4")
             elif self.method == GF.METHOD_RK4:
                 chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
                                                g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(Mu), P(s.du), Lw,

@@ -164,18 +164,19 @@ int gad_graph_build_wide(const int32_t* ptr, const int32_t* idx, int64_t N, void
  * RK4 step (north_star item 3; template classical_meshing/ma_mesh_1d.py:65-70). */
 size_t gad_deform_bwd_wide_rk4_workspace_bytes(int64_t N, int CE);
 int gad_deform_bwd_wide_rk4(const void* wide_in, const void* wide_out, int64_t N, int max_deg, const float* states,
-                            const float* g_xphys, int dim, int CE, const float* Mu, int Lw, const float* tau, int L,
-                            float* gMu, float* g_x0, void* workspace, size_t workspace_bytes, void* stream);
+                            const float* g_xphys, int dim, int CE, const float* Mu, const float* du, int M, int Lw,
+                            const float* tau, int L, float* gMu, float* g_x0, float* g_du, void* workspace,
+                            size_t workspace_bytes, void* stream);
 /* Largest node count the one-launch persistent forward takes on the current device for rows of this shape
  * (0: never -- reach unknown, window beyond 96 KB of shared memory, no cooperative launch). */
 int64_t gad_wide_persist_nodes(int CE, int max_deg, int64_t reach);
 int gad_deform_fwd_wide(const void* wide_in, int64_t N, int max_deg, int64_t reach, const float* x0, int dim, int CE,
-                        const float* Mu, int Lw, const float* tau, int L, int method, float* x_phys,
-                        float* states, void* workspace, size_t workspace_bytes, void* stream);
+                        const float* Mu, const float* du, int M, int Lw, const float* tau, int L, int method,
+                        float* x_phys, float* states, void* workspace, size_t workspace_bytes, void* stream);
 int gad_deform_bwd_wide(const void* wide_in, const void* wide_out, int64_t N, int max_deg, const float* states,
-                        const float* g_xphys, int dim, int CE, const float* Mu, int Lw, const float* tau, int L,
-                        float* gMu, float* g_tau, float* g_x0, void* workspace, size_t workspace_bytes,
-                        void* stream);
+                        const float* g_xphys, int dim, int CE, const float* Mu, const float* du, int M, int Lw,
+                        const float* tau, int L, float* gMu, float* g_tau, float* g_x0, float* g_du, void* workspace,
+                        size_t workspace_bytes, void* stream);
 
 /* ---- mesh-resident ELL path -------------------------------------------------------------------
  * The fast path for batches of bounded-degree meshes (every 1-D / 2-D mesh of the reference: in-
@@ -198,14 +199,23 @@ int gad_deform_bwd_wide(const void* wide_in, const void* wide_out, int64_t N, in
  * with the cotangent grad_scale * d(sum)/d(out).  `states` [L, N, CE] is scratch (layer inputs),
  * x_phys [N, dim] is optional.  workspace: gad_ell_workspace_bytes(CE, T, L).
  *
- * PER-TILE BIAS OFFSET `du` [T, Lw, CE] (gad_deform_fwd_ell_raw, gad_deform_bwd_ell, gad_deform_bwd_ell_rk4; NULL =
- * none): added to the folded bias u of every node of the tile.  This is all the global CNN features of the
- * reference (src/GNN.py:242-268: a per-mesh constant vector appended to every node's features) do to the deformer:
- * constant channels stay constant under A(x) x - x, and in the logits x_i^T M x_j + u^T x_j every term they enter is
- * constant over the in-edges of i -- and cancels in the softmax -- except g^T M_gz z_j, a shift of u by M_gz^T g.
- * One mesh per tile is required (the caller plans tiles that way).  d loss / d du is read from the backward's
- * workspace, which begins with the per-tile partials [T, slots, CE*CE + CE + 1] (slots = L if Lw > 1 else 1):
- * entries CE*CE .. CE*CE + CE - 1 of a row are sum_i t_i = d loss / d u restricted to the tile.
+ * PER-MESH BIAS OFFSET `du` [M, Lw, CE] (NULL = none): added to the folded bias u of weight set lw for every node of
+ * mesh b.  This is all the global CNN features of the reference (src/GNN.py:242-268: a per-mesh constant vector
+ * appended to every node's features) do to the deformer: constant channels stay constant under A(x) x - x, and in the
+ * logits x_i^T M x_j + u^T x_j every term they enter is constant over the in-edges of i -- and cancels in the softmax --
+ * except g^T M_gz z_j, a shift of u by M_gz^T g.  u + du is rounded to fp32 before the products are added on every
+ * route, and NULL gives the same bits as before the offset existed.  Taken by
+ *   - the mesh-resident ELL kernels (gad_deform_fwd_ell_raw, gad_deform_bwd_ell, gad_deform_bwd_ell_rk4): one mesh per
+ *     tile is required (the caller plans tiles that way), M = T.  d loss / d du is read from the backward's workspace,
+ *     which begins with the per-tile partials [T, slots, CE*CE + CE + 1] (slots = L if Lw > 1 else 1): entries
+ *     CE*CE .. CE*CE + CE - 1 of a row are sum_i t_i = d loss / d u restricted to the tile;
+ *   - the cluster kernels (gad_deform_fwd_cluster, gad_deform_bwd_cluster): one mesh per cluster, M = meshes;
+ *   - the streaming ELL kernels (gad_deform_fwd_wide, gad_deform_bwd_wide, gad_deform_bwd_wide_rk4): M meshes of N / M
+ *     nodes each, node i in mesh i / (N / M).
+ * The cluster and streaming backward entry points write d loss / d du into the explicit output g_du [M, Lw, CE]
+ * (may be NULL; needs du): the cluster backward sums the G_u entries of a cluster's CTA partials in rank order, the
+ * streaming backward keeps t_i per node over the passes of a weight set and sums each mesh's rows in a fixed order.
+ * No floating-point atomics: deterministic.  The CSR kernels (gad_deform_fwd / gad_deform_bwd) take no offset.
  *
  * SHARED TOPOLOGY (tile_ptr == NULL, in every gad_*_ell entry point and in gad_train_desc): the batch is
  * T = ceil(N / max_tile_nodes) equal tiles of max_tile_nodes nodes (the last one may be shorter) and ell_in /
@@ -370,15 +380,16 @@ int gad_train_step_cluster(const gad_train_desc* desc, int cluster_size, void* s
  * contract over cluster rows; workspace of gad_cluster_workspace_bytes. */
 int gad_deform_bwd_cluster(const void* crows_in, const void* crows_out, const int32_t* mesh_ptr, int M,
                            int max_mesh_nodes, int max_deg, int cluster_size, int64_t N, const float* states,
-                           const float* g_xphys, int dim, int CE, const float* Mu, int Lw, const float* tau, int L,
-                           float* gMu, float* g_tau, float* g_x0, void* workspace, size_t workspace_bytes,
-                           void* stream);
+                           const float* g_xphys, int dim, int CE, const float* Mu, const float* du, int Lw,
+                           const float* tau, int L, float* gMu, float* g_tau, float* g_x0, float* g_du, void* workspace,
+                           size_t workspace_bytes, void* stream);
 /* Forward only (module seam / inference), all L Euler layers or RK4 steps in ONE launch with the state
  * resident in the cluster's shared memory: gad_deform_fwd_ell_raw's contract over cluster rows. */
 int gad_deform_fwd_cluster(const void* crows_in, const int32_t* mesh_ptr, int M, int max_mesh_nodes, int max_deg,
                            int cluster_size, int64_t N, const float* x_comp, const float* f, const float* uu,
-                           const float* f_scale, const float* uu_scale, int dim, int CE, const float* Mu, int Lw,
-                           const float* tau, int L, int method, float* x_phys, float* states, void* stream);
+                           const float* f_scale, const float* uu_scale, int dim, int CE, const float* Mu,
+                           const float* du, int Lw, const float* tau, int L, int method, float* x_phys, float* states,
+                           void* stream);
 
 /* ---- operator seam: one GRAND_plusConv / GRAND_conv layer (src/GRAND_plus.py:204-267,380-382) --
  * res = A(x) x - x  for x [N, CE];  alpha (optional) [E] in filtered edge-list order.
@@ -473,7 +484,9 @@ int gad_peer_free(void* dev_ptr);
  * the forward is recomputed, per-mesh parts are summed over the batch in fp64 in a fixed order (workspace of
  * gad_cnn_workspace_bytes; the same workspace size serves the forward).  When the L activation planes do not fit
  * the shared memory next to the other buffers (16 channels on a 30 x 30 grid) they live in the workspace instead
- * (L2-resident).  The grid values get no gradient.  Limits: L <= 8, channels <= 16. */
+ * (L2-resident), and when the backward's two gradient planes do not fit next to the input plane either (8 channels:
+ * grids beyond about 58 x 58, 1-D meshes beyond about 3300 nodes) so do they; the results are the same bits.  The grid
+ * values get no gradient.  Limits: L <= 8, channels <= 16, the input plane in shared memory (about 240 x 240). */
 int64_t gad_cnn_param_count(int H, int Cm, int Co, int L);
 size_t gad_cnn_workspace_bytes(int B, int H, int W, int Cm, int Co, int L);
 int gad_cnn_fwd(const float* u, const int32_t* gather, const float* scale, int B, int H, int W, int Cm, int Co, int L,
