@@ -263,8 +263,9 @@ __device__ __forceinline__ void cl_backward(const Args& a, const Layout& lay, in
 }
 
 // a.tile_ptr = mesh_ptr [M + 1]; a.T = number of per-CTA partial rows (= grid); a.cap_nodes = slab capacity;
-// a.ell_in / a.ell_out = cluster rows (2 x uint4 per node)
-template <int CE, int W>
+// a.ell_in / a.ell_out = cluster rows (2 x uint4 per node).  COT: loss_kind 2, the target rows hold the caller's
+// cotangent of x_phys (ell_kernels.cuh: k_ell_train).
+template <int CE, int W, bool COT = false>
 __global__ void __launch_bounds__(MAXT, 1) k_cl_train(const Args a) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
@@ -399,13 +400,19 @@ __global__ void __launch_bounds__(MAXT, 1) k_cl_train(const Args a) {
                 Row<CE> g;
 #pragma unroll
                 for (int c = 0; c < CE; ++c) {
-                    const float d = (c < a.dim) ? xn.v[c] - tg.v[c] : 0.f;
-                    if (a.loss_kind == 0) {
-                        loss_acc += fabsf(d);
-                        g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);
+                    if constexpr (COT) {
+                        const float cc = (c < a.dim) ? tg.v[c] : 0.f;
+                        loss_acc = fmaf(xn.v[c], cc, loss_acc);
+                        g.v[c] = a.grad_scale * cc;
                     } else {
-                        loss_acc = fmaf(d, d, loss_acc);
-                        g.v[c] = 2.0f * a.grad_scale * d;
+                        const float d = (c < a.dim) ? xn.v[c] - tg.v[c] : 0.f;
+                        if (a.loss_kind == 0) {
+                            loss_acc += fabsf(d);
+                            g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);
+                        } else {
+                            loss_acc = fmaf(d, d, loss_acc);
+                            g.v[c] = 2.0f * a.grad_scale * d;
+                        }
                     }
                 }
                 sts_row<CE>(GS, i * RB, g);
@@ -685,11 +692,12 @@ int slab_cap(int CE) {
 
 template <int CE, int W>
 int launch_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
+    auto kern = a.loss_kind == 2 ? k_cl_train<CE, W, true> : k_cl_train<CE, W, false>;
     const size_t bytes = make_layout(CE, a.cap_nodes, (threads + 31) / 32).total;
     GAD_CHECK_ARG((int)bytes <= smem_optin_bytes(), "cluster kernel: slab of %d nodes needs %zu B of shared memory",
                   a.cap_nodes, bytes);
-    GAD_CUDA(cudaFuncSetAttribute(k_cl_train<CE, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(k_cl_train<CE, W>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    if (C > 8) GAD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3((unsigned)threads);
@@ -708,7 +716,7 @@ int launch_t(const Args& a, int C, int grid, int threads, cudaStream_t st) {
     }
     cfg.attrs = attr;
     cfg.numAttrs = na;
-    GAD_CUDA(cudaLaunchKernelEx(&cfg, k_cl_train<CE, W>, a));
+    GAD_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
     count_launch(1);
     return GAD_OK;
 }
@@ -793,6 +801,7 @@ extern "C" int gad_train_step_cluster(const gad_train_desc* d, int cluster_size,
                   d->Lw);
     GAD_CHECK_ARG(d->dim + (d->f ? 1 : 0) + (d->uu ? 1 : 0) <= d->CE, "gad_train_step_cluster: input features exceed CE=%d",
                   d->CE);
+    GAD_CHECK_ARG(d->loss_kind >= 0 && d->loss_kind <= 2, "gad_train_step_cluster: unknown loss kind %d", d->loss_kind);
     GAD_CHECK_ARG(d->tail == 1 || d->tail == 2, "gad_train_step_cluster: tail must be 1 or 2");
     GAD_CHECK_ARG(d->Wq && d->bq && d->Wk && d->gWq && d->gbq && d->gWk && d->gbk && d->C > 0,
                   "gad_train_step_cluster: the tail needs the Linear parameters and their gradient buffers");

@@ -396,7 +396,7 @@ extern "C" int gad_deform_train_ell(const void* ell_in, const void* ell_out, int
                   "gad_deform_train_ell: N=%lld T=%d L=%d dim=%d CE=%d Lw=%d", (long long)N, T, L, dim, CE, Lw);
     GAD_CHECK_ARG(dim + (f ? 1 : 0) + (uu ? 1 : 0) <= CE, "gad_deform_train_ell: %d input features exceed CE=%d",
                   dim + (f ? 1 : 0) + (uu ? 1 : 0), CE);
-    GAD_CHECK_ARG(loss_kind == 0 || loss_kind == 1, "gad_deform_train_ell: unknown loss kind %d", loss_kind);
+    GAD_CHECK_ARG(loss_kind >= 0 && loss_kind <= 2, "gad_deform_train_ell: unknown loss kind %d", loss_kind);
     GAD_CHECK_ARG(workspace_bytes >= ws_floats(CE, T, L) * sizeof(float), "gad_deform_train_ell: workspace too small");
     Plan p;
     int rc = make_plan(CE, KIND_BWD, max_tile_nodes, max_deg, &p);
@@ -447,7 +447,7 @@ static int train_step(const gad_train_desc* d, int method, const char* who, void
     GAD_CHECK_ARG(d->N > 0 && d->T > 0 && d->L > 0 && d->dim >= 1 && d->dim <= d->CE && (d->Lw == 1 || d->Lw == d->L),
                   "%s: N=%lld T=%d L=%d dim=%d CE=%d Lw=%d", who, (long long)d->N, d->T, d->L, d->dim, d->CE, d->Lw);
     GAD_CHECK_ARG(d->dim + (d->f ? 1 : 0) + (d->uu ? 1 : 0) <= d->CE, "%s: input features exceed CE=%d", who, d->CE);
-    GAD_CHECK_ARG(d->loss_kind == 0 || d->loss_kind == 1, "%s: unknown loss kind %d", who, d->loss_kind);
+    GAD_CHECK_ARG(d->loss_kind >= 0 && d->loss_kind <= 2, "%s: unknown loss kind %d", who, d->loss_kind);
     GAD_CHECK_ARG(d->tail == 1 || d->tail == 2, "%s: tail must be 1 or 2 (got %d)", who, d->tail);
     GAD_CHECK_ARG(d->Wq && d->bq && d->Wk && d->gWq && d->gbq && d->gWk && d->gbk && d->C > 0,
                   "%s: the tail needs the Linear parameters and their gradient buffers", who);

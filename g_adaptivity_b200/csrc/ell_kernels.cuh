@@ -114,9 +114,9 @@ struct Args {
     const float* f_scale;
     const float* uu_scale;
     const float* target;    // [N, dim]
-    int loss_kind;          // 0: L1, 1: MSE
-    float grad_scale;       // cotangent = grad_scale * d|out - target| (or d(out - target)^2)
-    float* loss_partials;   // [T] sum over the tile of |d| or d^2
+    int loss_kind;          // 0: L1, 1: MSE, 2: target holds the caller's cotangent c of x_phys
+    float grad_scale;       // cotangent = grad_scale * d|out - target| (or d(out - target)^2, or c)
+    float* loss_partials;   // [T] sum over the tile of |d|, d^2 or out * c
     // train tail, run by the last CTA to finish (tail = 0: none, the host launches the reduction;
     // 1: reduction + weight gradients; 2: + Adam + the folded weights of the NEXT step)
     int tail;
@@ -1171,7 +1171,10 @@ __device__ __forceinline__ void tail_finish(const Args& a, unsigned char* scratc
 // expressions), the loss fused into stage 4 of the last step, then tile_backward_rk4.  The inputs are
 // staged into the Y2 rows (untouched until the backward recomputes the stages) and the target into DL;
 // the cotangent goes to the G rows, which tile_backward_rk4 reads as dL/dx^L.
-template <int CE, int W, bool ELLS, int METHOD>
+// COT (loss_kind 2): the target rows hold a cotangent c of x_phys computed outside the model; the loss stage sets
+// dL/dx^L = grad_scale * c and sums the pseudo-loss <x_phys, c>.  A template flag, so that the mesh-loss kernels
+// compile to what they were before it existed.
+template <int CE, int W, bool ELLS, int METHOD, bool COT = false>
 __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const Args a) {
     constexpr uint32_t RB = CE * sizeof(float);
     constexpr int MUSZ = CE * CE + CE;
@@ -1348,6 +1351,10 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
                         loss_acc = fmaf(d, d, loss_acc);
                         return 2.0f * a.grad_scale * d;
                     };
+                    auto cterm = [&](float x, float c) {   // COT: adds x * c, returns the scaled cotangent entry
+                        loss_acc = fmaf(x, c, loss_acc);
+                        return a.grad_scale * c;
+                    };
                     Row<CE> g = zero_row<CE>();
                     if (a.dim == 2) {
                         // 2-D meshes: float2 rows, no per-channel tests; the channels beyond dim have d = 0, whose
@@ -1355,14 +1362,24 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
                         if (a.x_phys) *reinterpret_cast<float2*>(a.x_phys + gi * 2) = make_float2(xn.v[0], xn.v[1]);
                         const float2 tg = stage ? *reinterpret_cast<const float2*>(DL + (size_t)i * 8)
                                                 : *reinterpret_cast<const float2*>(a.target + gi * 2);
-                        g.v[0] = term(xn.v[0] - tg.x);
-                        g.v[1] = term(xn.v[1] - tg.y);
+                        if constexpr (COT) {
+                            g.v[0] = cterm(xn.v[0], tg.x);
+                            g.v[1] = cterm(xn.v[1], tg.y);
+                        } else {
+                            g.v[0] = term(xn.v[0] - tg.x);
+                            g.v[1] = term(xn.v[1] - tg.y);
+                        }
                     } else {
                         if (a.x_phys) store_dims<CE>(a.x_phys, gi, a.dim, xn);
                         const Row<CE> tg = stage ? load_dims<CE>(reinterpret_cast<const float*>(TG + i * tg_rb), 0, a.dim)
                                                  : load_dims<CE>(a.target, gi, a.dim);
+                        if constexpr (COT) {
 #pragma unroll
-                        for (int c = 0; c < CE; ++c) g.v[c] = term((c < a.dim) ? xn.v[c] - tg.v[c] : 0.f);
+                            for (int c = 0; c < CE; ++c) g.v[c] = cterm(xn.v[c], tg.v[c]);   // load_dims: 0 beyond dim
+                        } else {
+#pragma unroll
+                            for (int c = 0; c < CE; ++c) g.v[c] = term((c < a.dim) ? xn.v[c] - tg.v[c] : 0.f);
+                        }
                     }
                     return g;
                 };
@@ -1460,13 +1477,19 @@ __global__ void __launch_bounds__(GAD_ELL_MAXT, GAD_ELL_MINB) k_ell_train(const 
                             Row<CE> g;
 #pragma unroll
                             for (int c = 0; c < CE; ++c) {
-                                const float d = (c < a.dim) ? out.v[c] - tg.v[c] : 0.f;
-                                if (a.loss_kind == 0) {
-                                    loss_acc += fabsf(d);
-                                    g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);   // torch sign()
+                                if constexpr (COT) {
+                                    const float cc = (c < a.dim) ? tg.v[c] : 0.f;
+                                    loss_acc = fmaf(out.v[c], cc, loss_acc);
+                                    g.v[c] = a.grad_scale * cc;
                                 } else {
-                                    loss_acc = fmaf(d, d, loss_acc);
-                                    g.v[c] = 2.0f * a.grad_scale * d;
+                                    const float d = (c < a.dim) ? out.v[c] - tg.v[c] : 0.f;
+                                    if (a.loss_kind == 0) {
+                                        loss_acc += fabsf(d);
+                                        g.v[c] = (d > 0.f) ? a.grad_scale : ((d < 0.f) ? -a.grad_scale : 0.f);   // torch sign()
+                                    } else {
+                                        loss_acc = fmaf(d, d, loss_acc);
+                                        g.v[c] = 2.0f * a.grad_scale * d;
+                                    }
                                 }
                             }
                             sts_row<CE>(G, i * RB, g);
@@ -1588,12 +1611,12 @@ int launch_bwd_rk4_t(const Args& a, int threads, cudaStream_t st) {
     return GAD_OK;
 }
 
-template <int CE, int W, bool ELLS, int METHOD>
+template <int CE, int W, bool ELLS, int METHOD, bool COT>
 int launch_train_m(const Args& a_in, int threads, cudaStream_t st) {
     int grid = 0, rc;
     const int kind = METHOD == GAD_METHOD_RK4 ? KIND_TRAIN_RK4 : KIND_BWD;
     const size_t bytes = make_layout(CE, kind, a_in.cap_nodes, ELLS, (threads + 31) / 32).total;
-    if ((rc = prepare_launch(k_ell_train<CE, W, ELLS, METHOD>, threads, bytes, a_in.T + 1, &grid))) return rc;
+    if ((rc = prepare_launch(k_ell_train<CE, W, ELLS, METHOD, COT>, threads, bytes, a_in.T + 1, &grid))) return rc;
     Args a = a_in;
     // grid == T + 1: every tile has its own CTA and one more fits -> that one is the reducer
     static const bool allow_reducer = !(getenv("GAD_TAIL_CTA") && atoi(getenv("GAD_TAIL_CTA")) == 0);
@@ -1612,19 +1635,23 @@ int launch_train_m(const Args& a_in, int threads, cudaStream_t st) {
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_ell_train<CE, W, ELLS, METHOD>, a));
+        GAD_CUDA(cudaLaunchKernelEx(&cfg, k_ell_train<CE, W, ELLS, METHOD, COT>, a));
         count_launch(1);
         return GAD_OK;
     }
-    k_ell_train<CE, W, ELLS, METHOD><<<grid, threads, bytes, st>>>(a);
+    k_ell_train<CE, W, ELLS, METHOD, COT><<<grid, threads, bytes, st>>>(a);
     GAD_LAUNCH_CHECK();
     return GAD_OK;
 }
 
 template <int CE, int W, bool ELLS>
 int launch_train_t(const Args& a, int method, int threads, cudaStream_t st) {
-    if (method == GAD_METHOD_RK4) return launch_train_m<CE, W, ELLS, GAD_METHOD_RK4>(a, threads, st);
-    return launch_train_m<CE, W, ELLS, GAD_METHOD_EULER>(a, threads, st);
+    if (a.loss_kind == 2) {
+        if (method == GAD_METHOD_RK4) return launch_train_m<CE, W, ELLS, GAD_METHOD_RK4, true>(a, threads, st);
+        return launch_train_m<CE, W, ELLS, GAD_METHOD_EULER, true>(a, threads, st);
+    }
+    if (method == GAD_METHOD_RK4) return launch_train_m<CE, W, ELLS, GAD_METHOD_RK4, false>(a, threads, st);
+    return launch_train_m<CE, W, ELLS, GAD_METHOD_EULER, false>(a, threads, st);
 }
 
 // which: 0 forward, 1 backward, 2 train (Euler or RK4 by `method`), 3 backward through RK4 steps

@@ -200,7 +200,8 @@ __global__ void k_reduce_partials(const float* __restrict__ partials, int rows, 
 // Per-block partial sums of |d| or d^2, d = out[j] - target[i], and the cotangent at out[j].  Without an index map
 // j = i.  With one (kOrder, the pde loss) entry i = b * Q + q of `target` pairs with j = b * Q + order[q]: the FEM
 // solution stays in evaluation-grid order and the target is in the fine mesh's node order (src/GNN.py:333).
-template <bool kOrder>
+// kCot (gad_mesh_loss kind 2): target[i] is a cotangent c of out[i]; partial sums of out * c, g_out = grad_scale * c.
+template <bool kOrder, bool kCot = false>
 __device__ __forceinline__ void loss_partials(const float* __restrict__ out, const float* __restrict__ target,
                                               int64_t count, int kind, float grad_scale, float* __restrict__ g_out,
                                               float* __restrict__ partials, const int32_t* __restrict__ order,
@@ -212,6 +213,11 @@ __device__ __forceinline__ void loss_partials(const float* __restrict__ out, con
         if (kOrder) {
             const int64_t b = i / Q;
             j = b * Q + order[i - b * Q];
+        }
+        if constexpr (kCot) {
+            acc[0] = fmaf(out[j], target[i], acc[0]);
+            if (g_out) g_out[j] = grad_scale * target[i];
+            continue;
         }
         const float d = out[j] - target[i];
         if (kind == 0) {
@@ -229,6 +235,12 @@ __global__ void __launch_bounds__(TB) k_loss(const float* __restrict__ out, cons
                                              int64_t count, int kind, float grad_scale, float* __restrict__ g_out,
                                              float* __restrict__ partials) {
     loss_partials<false>(out, target, count, kind, grad_scale, g_out, partials, nullptr, 1);
+}
+
+__global__ void __launch_bounds__(TB) k_loss_cot(const float* __restrict__ out, const float* __restrict__ cot,
+                                                 int64_t count, float grad_scale, float* __restrict__ g_out,
+                                                 float* __restrict__ partials) {
+    loss_partials<false, true>(out, cot, count, 2, grad_scale, g_out, partials, nullptr, 1);
 }
 
 // squared error through the index map (gad_pde_loss)
@@ -441,14 +453,17 @@ extern "C" size_t gad_mesh_loss_workspace_bytes(int64_t count) {
 
 extern "C" int gad_mesh_loss(const float* out, const float* target, int64_t count, int kind, float grad_scale,
                              float* loss, float* g_out, void* workspace, void* stream) {
-    GAD_CHECK_ARG(out && target && loss && workspace && count > 0 && (kind == 0 || kind == 1), "gad_mesh_loss: bad arguments");
+    GAD_CHECK_ARG(out && target && loss && workspace && count > 0 && kind >= 0 && kind <= 2, "gad_mesh_loss: bad arguments");
     cudaStream_t st = as_stream(stream);
     const int64_t want = (count + TB - 1) / TB;
     const int G = (int)(want < (int64_t)sm_count() * 8 ? want : (int64_t)sm_count() * 8);
     float* partials = reinterpret_cast<float*>(workspace);
-    k_loss<<<G, TB, 0, st>>>(out, target, count, kind, grad_scale, g_out, partials);
+    if (kind == 2)   // the pseudo-loss <out, c> is a sum, not a mean
+        k_loss_cot<<<G, TB, 0, st>>>(out, target, count, grad_scale, g_out, partials);
+    else
+        k_loss<<<G, TB, 0, st>>>(out, target, count, kind, grad_scale, g_out, partials);
     GAD_LAUNCH_CHECK();
-    k_loss_final<<<1, 32, 0, st>>>(partials, G, 1.0f / (float)count, loss);
+    k_loss_final<<<1, 32, 0, st>>>(partials, G, kind == 2 ? 1.0f : 1.0f / (float)count, loss);
     GAD_LAUNCH_CHECK();
     return GAD_OK;
 }

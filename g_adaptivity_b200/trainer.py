@@ -44,6 +44,14 @@ cannot: its tail refolds (M, u) with a constant temperature.  Such slots need th
 Neither option is trained together with global CNN features, and gnn_dont_train is refused: those raise
 NotImplementedError and train through GNN.forward + autograd.
 
+`loss_type='modular'` (the reference's Burgers preset, src/run_GNN.py:111-131: an outside function returns (loss,
+x_grads) for the detached x_phys and the loop back-propagates sum(x_phys * x_grads)) is the cotangent mode:
+`forward(sid)` runs the step's forward and returns the slot's x_phys, the caller computes x_grads, and
+`step(sid, cotangent=x_grads)` copies it into the slot's target segment and replays the step, whose loss stage (loss
+kind 2, include/gadapt.h) back-propagates exactly that cotangent on every route; `train_batch(data, grad_fn)` is the
+loop body.  Steps cannot be issued ahead of the caller (run_epoch, run_from_host raise).  An explicit `loss_fn` trains
+the mesh loss instead.
+
 Sharding (SURVEY 8e): a batch is a disjoint union of meshes, so ranks take contiguous shards of
 whole meshes with no data-path collective; the only exchange is the all-reduce of the flat
 gradient (144 + L floats).  The mesh loss is a mean over ALL nodes of the global batch
@@ -92,13 +100,16 @@ class DeformerTrainer:
         # Options GNN.forward and the reference training loop honour but this fused step does not implement
         # raise instead of silently training something else (src/run_GNN.py:80-88,109-131; src/GNN.py:231-237).
         loss_type = opt.get("loss_type", "mesh_loss")
-        if loss_fn is None and loss_type not in ("mesh_loss", "pde_loss"):
+        if loss_fn is None and loss_type not in ("mesh_loss", "pde_loss", "modular"):
             raise NotImplementedError(
-                f"DeformerTrainer trains the mesh loss and the pde loss (src/run_GNN.py:105-110); opt['loss_type']="
-                f"{opt['loss_type']!r} trains through GNN.forward + autograd instead.  Pass loss_fn='l1' / 'mse' explicitly "
-                "to train the mesh loss on such a preset")
+                f"DeformerTrainer trains the mesh loss, the pde loss and the modular loss (src/run_GNN.py:105-131); "
+                f"opt['loss_type']={opt['loss_type']!r} trains through GNN.forward + autograd instead.  Pass loss_fn='l1' / "
+                "'mse' explicitly to train the mesh loss on such a preset")
         # loss_type='pde_loss': mse(FEM solution on the deformed mesh, u_true_fine), unless loss_fn asks for the mesh loss
         self.pde = loss_fn is None and loss_type == "pde_loss"
+        # loss_type='modular': the caller's cotangent of x_phys (src/run_GNN.py:111-131), unless loss_fn asks for the
+        # mesh loss
+        self.cot = loss_fn is None and loss_type == "modular"
         # softmax_temp_type='learnable_a': one trainable temperature per weight set (src/GRAND_plus.py:152-154,328-329)
         self.learn_temp = opt.get("softmax_temp_type") == "learnable_a"
         # gnn_normalize: f / torch.max(f) and uu / torch.max(uu) over the batch (src/GNN.py:231-237)
@@ -109,8 +120,8 @@ class DeformerTrainer:
         if opt.get("gnn_dont_train", False):
             raise NotImplementedError("DeformerTrainer: gnn_dont_train=True skips the optimizer step (src/run_GNN.py:122-131); "
                                       "evaluate with GNN.forward instead")
-        self.loss_kind = "pde" if self.pde else (opt.get("loss_fn", "l1") if loss_fn is None else loss_fn)
-        if not self.pde and self.loss_kind not in ("l1", "mse"):
+        self.loss_kind = "pde" if self.pde else "cot" if self.cot else (opt.get("loss_fn", "l1") if loss_fn is None else loss_fn)
+        if not (self.pde or self.cot) and self.loss_kind not in ("l1", "mse"):
             raise NotImplementedError(f"DeformerTrainer: loss_fn={self.loss_kind!r} (the reference has 'l1' and 'mse', "
                                       "src/run_GNN.py:80-84)")
         self.pg = process_group
@@ -130,6 +141,7 @@ class DeformerTrainer:
         self._flatten_parameters()
         self.slots: List[_Slot] = []
         self.graphs: Dict[int, torch.cuda.CUDAGraph] = {}
+        self.fwd_graphs: Dict[int, torch.cuda.CUDAGraph] = {}
         self.epoch_graphs: Dict[tuple, torch.cuda.CUDAGraph] = {}
         self.lib = _lib.load()
         # data parallel on one NVLink node: the training kernel all-reduces the gradient itself over
@@ -245,10 +257,18 @@ class DeformerTrainer:
                                                         self.C, self.CE, self.model.inv_temp, _lib.ptr(self.Mu),
                                                         self.stream.cuda_stream), "gad_prepare_weights")
 
+    def _loss_args(self, s: "_Slot") -> tuple:
+        """(loss kind, cotangent scale, loss scale) of the slot's mesh-loss stage (include/gadapt.h: loss_kind).  The
+        cotangent mode's loss is the pseudo-loss sum <x_phys, c>: every rank passes the cotangent of its own shard
+        unscaled, and the all-reduce sums to the gradient of the union batch's pseudo-loss."""
+        if self.cot:
+            return 2, 1.0, 1.0
+        count = s.N * self.dim
+        return (0 if self.loss_kind == "l1" else 1), dp.local_grad_scale(count, s.count_global, world=self.world), 1.0 / count
+
     def _train_desc(self, s: "_Slot", tail: int) -> "_lib.TrainDesc":
         """Descriptor of one `gad_train_step_ell` launch on slot `s` (include/gadapt.h: gad_train_desc)."""
         P, g = _lib.ptr, s.graph
-        count = s.N * self.dim
         b1, b2 = self.betas
         d = _lib.TrainDesc()
         if g.tile_ptr is None:      # cluster-resident meshes (gad_train_step_cluster)
@@ -261,8 +281,7 @@ class DeformerTrainer:
         d.f_scale, d.uu_scale = P(s.f_scale), P(s.uu_scale)
         d.dim, d.CE = self.dim, self.CE
         d.Mu, d.tau, d.Lw, d.L, d.C, d.inv_temp = P(self.Mu), P(self.tau), self.Lw, self.L, self.C, self.model.inv_temp
-        d.loss_kind = 0 if self.loss_kind == "l1" else 1
-        d.grad_scale, d.loss_scale = dp.local_grad_scale(count, s.count_global, world=self.world), 1.0 / count
+        d.loss_kind, d.grad_scale, d.loss_scale = self._loss_args(s)
         d.states, d.gMu, d.g_tau, d.loss, d.x_phys = P(s.states), P(self.gMu), P(self.gtau), P(s.loss), P(s.x_phys)
         d.workspace, d.workspace_bytes = P(s.bwd_ws), s.bwd_ws_bytes
         d.tail, d.counter = tail, P(self.counter)
@@ -273,8 +292,10 @@ class DeformerTrainer:
         d.lr, d.beta1, d.beta2, d.eps, d.weight_decay, d.adam_grad_scale = self.lr, b1, b2, self.eps, self.wd, 1.0
         d.step = P(self.step_count)
         # GAD_TRAIN_PDL.  Not on a normalised slot: the kernel reads f_scale / uu_scale while staging its inputs, before
-        # it waits on its predecessor, which there is gad_batch_max (or the all-reduce of its result)
-        d.flags = 1 if (self.use_pdl and tail == 2 and not s.norm) else 0
+        # it waits on its predecessor, which there is gad_batch_max (or the all-reduce of its result).  Nor in the
+        # cotangent mode: the staged target is the cotangent the caller has just written, and no train kernel
+        # precedes the step there (forward and the caller's loss come between)
+        d.flags = 1 if (self.use_pdl and tail == 2 and not s.norm and not self.cot) else 0
         d.peer_timeout_ms = 0
         if self.fused_dp and tail == 2:
             d.rank, d.world, d.peers, d.peer_seq = self.rank, self.world, P(self.peer.ptrs), P(self.peer.seq)
@@ -488,6 +509,8 @@ class DeformerTrainer:
         xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
         if s.pde:
             first = [data.u_true_fine_tensor, *self.model._pde_params_to_tensors(data.pde_params, s.B, "cpu")]
+        elif self.cot:          # the target segment takes the caller's cotangent (step(sid, cotangent=...))
+            first = [None]
         else:
             first = [data.x_phys if data.x_phys.dim() == 2 else data.x_phys.unsqueeze(-1)]
         return first + [data.f_tensor if s.f is not None else None, data.uu_tensor if s.uu is not None else None,
@@ -537,8 +560,10 @@ class DeformerTrainer:
 
     # ------------------------------------------------------------------------------------
     def _issue(self, s: _Slot, stream_ptr: int, with_optimizer: bool = True, stage: str = "all"):
-        """Enqueue the kernels of one training step on `stream_ptr` (captured or eager)."""
-        if s.norm and stage in ("all", "pre"):
+        """Enqueue the kernels of one training step on `stream_ptr` (captured or eager).  stage 'fwd': the step's
+        forward only (cotangent mode: what `forward(sid)` runs) -- the work before the deformer and the deformer
+        forward on the same kernels and arithmetic, so its x_phys is the step's bit for bit."""
+        if s.norm and stage in ("all", "pre", "fwd"):
             self._issue_batch_max(s, stream_ptr)
         if s.chain:
             return self._issue_chain(s, stream_ptr, with_optimizer, stage)
@@ -549,6 +574,19 @@ class DeformerTrainer:
         inv_temp = self.model.inv_temp
         ell = self._fused_ell(s)
         cluster = (not ell) and self._cluster(s)
+        if stage == "fwd" and (ell or cluster):
+            # the forward of the one-launch kernel: same rows, inputs and folded weights (the step keeps Mu == fold(params))
+            if cluster:
+                chk(lib.gad_deform_fwd_cluster(P(g.cl_in), P(g.mesh_ptr), len(g.mesh_sizes), max(g.mesh_sizes), g.cl_deg,
+                                               g.cl_C, s.N, P(s.x_comp), P(s.f), P(s.uu), P(s.f_scale), P(s.uu_scale), dim,
+                                               CE, P(self.Mu), None, Lw, P(self.tau), L, self.method, P(s.x_phys),
+                                               P(s.states), stream_ptr), "gad_deform_fwd_cluster")
+            else:
+                chk(lib.gad_deform_fwd_ell_raw(P(g.ell_in), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes, g.ell_deg,
+                                               P(s.x_comp), P(s.f), P(s.uu), P(s.f_scale), P(s.uu_scale), dim, CE,
+                                               P(self.Mu), None, Lw, P(self.tau), L, self.method, P(s.x_phys),
+                                               P(s.states), stream_ptr), "gad_deform_fwd_ell_raw")
+            return
         if ell or cluster:
             # ONE launch per step (csrc/ell_kernels.cuh: k_ell_train): pack + forward + loss + backward per
             # tile, then the last CTA reduces, applies the chain rule and -- single GPU -- takes the Adam step
@@ -571,7 +609,7 @@ class DeformerTrainer:
                 chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu),
                                             stream_ptr), "gad_prepare_weights")
             return
-        if stage in ("all", "pre"):
+        if stage in ("all", "pre", "fwd"):
             chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
                 "gad_prepare_weights")
             chk(lib.gad_pack_features(P(s.x_comp), P(s.f), P(s.uu), P(s.f_scale), P(s.uu_scale), s.N, dim, CE,
@@ -587,11 +625,11 @@ class DeformerTrainer:
                                        P(self.Mu), Lw, P(self.tau), L, self.method, P(s.x_phys), P(s.states), P(s.fwd_ws),
                                        s.fwd_ws_bytes, stream_ptr),
                     "gad_deform_fwd")
-            chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, 0 if self.loss_kind == "l1" else 1,
-                                  dp.local_grad_scale(s.N * dim, s.count_global, world=self.world), P(s.loss), P(s.g_out),
-                                  P(s.loss_ws),
-                                  stream_ptr),
-                "gad_mesh_loss")
+            if stage == "fwd":
+                return
+            kind, grad_scale, _ = self._loss_args(s)
+            chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, kind, grad_scale, P(s.loss), P(s.g_out),
+                                  P(s.loss_ws), stream_ptr), "gad_mesh_loss")
             if self.method == GF.METHOD_RK4 and s.rk4_resident:
                 chk(lib.gad_deform_bwd_ell_rk4(P(g.ell_in), P(g.ell_out), s.N, P(g.ell_tile_ptr), g.T, g.max_tile_nodes,
                                                g.ell_deg, P(s.states), P(s.g_out), dim, CE, P(self.Mu), None, Lw,
@@ -639,7 +677,7 @@ class DeformerTrainer:
             H, W = s.cnn_hw
             g_f, g_uu = s.cnn_out.get("f"), s.cnn_out.get("uu")
             glob = (B, used[0]["Co"], self.n_g, P(self.Wq), P(self.Wk), Lw, C_, m.z_dim, m.live, CE, inv_temp)
-        if stage in ("all", "pre"):
+        if stage in ("all", "pre", "fwd"):
             chk(lib.gad_prepare_weights(P(self.Wq), P(self.bq), P(self.Wk), Lw, C_, CE, inv_temp, P(self.Mu), stream_ptr),
                 "gad_prepare_weights")
             if s.temp:
@@ -661,12 +699,14 @@ class DeformerTrainer:
                                            P(s.x_comp), P(f), P(uu), P(s.f_scale), P(s.uu_scale), dim, CE, P(Mu),
                                            P(s.du), Lw, P(self.tau), L, self.method, P(s.x_phys), P(s.states), stream_ptr),
                 "gad_deform_fwd_ell_raw")
+            if stage == "fwd":
+                return
             if s.pde:
                 self._issue_pde_loss(s, stream_ptr)
             else:
-                chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, 0 if self.loss_kind == "l1" else 1,
-                                      dp.local_grad_scale(s.N * dim, s.count_global, world=self.world), P(s.loss),
-                                      P(s.g_out), P(s.loss_ws), stream_ptr), "gad_mesh_loss")
+                kind, grad_scale, _ = self._loss_args(s)
+                chk(lib.gad_mesh_loss(P(s.x_phys), P(s.target), s.N * dim, kind, grad_scale, P(s.loss), P(s.g_out),
+                                      P(s.loss_ws), stream_ptr), "gad_mesh_loss")
             if self.method == GF.METHOD_RK4 and not s.rk4_resident:
                 chk(lib.gad_deform_bwd_wide_rk4(P(g.wide_in), P(g.wide_out), s.N, g.wide_deg, P(s.states), P(s.g_out),
                                                 dim, CE, P(Mu), None, 0, Lw, P(self.tau), L, P(self.gMu), None, None,
@@ -772,6 +812,7 @@ class DeformerTrainer:
         """Drop the captured graphs and the peer mappings (call on every rank, after the last step)."""
         self.stream.synchronize()
         self.graphs.clear()
+        self.fwd_graphs.clear()
         self.epoch_graphs.clear()
         for p in self.__dict__.pop("_host_allocs", []):
             self.lib.gad_host_free(p)
@@ -817,6 +858,7 @@ class DeformerTrainer:
         spin, an event record, the steps, an event record (external events = event-record NODES of the graph).
         `run_epoch(sids, timed=True)` replays it and `epoch_elapsed_ms(sids)` reads the device time between the two
         records: the steps' own time, without the latency of getting a graph launch from the host to the device."""
+        self._refuse_cotangent_mode("capture_epoch")
         key = tuple(int(s) for s in sids)
         if timed:
             key = ("timed",) + key
@@ -862,9 +904,16 @@ class DeformerTrainer:
         # the kernels update the parameters in place without bumping tensor version counters
         self.model._param_epoch = getattr(self.model, "_param_epoch", 0) + 1
 
+    def _refuse_cotangent_mode(self, what: str):
+        if self.cot:
+            raise ValueError(f"{what}: with loss_type='modular' every step takes the cotangent of the x_phys of the current "
+                             "parameters, so steps cannot be issued ahead of the caller's loss; use train_batch(data, "
+                             "grad_fn) or forward(sid) -> step(sid, cotangent=x_grads)")
+
     def run_epoch(self, sids, timed: bool = False):
         """One pass over the resident batches `sids` (one training step each) as a single graph replay.
         Returns the per-slot loss tensors (device; each holds the loss of that slot's LAST step)."""
+        self._refuse_cotangent_mode("run_epoch")
         if not self.use_graph:
             return [self.step(sid) for sid in sids]
         key = self.capture_epoch(sids, timed=timed)
@@ -873,8 +922,67 @@ class DeformerTrainer:
             self.epoch_graphs[key].replay()
         return [self.slots[sid].loss for sid in (key[1:] if timed else key)]
 
-    def step(self, sid: int):
-        """One training step on the resident batch `sid` (asynchronous; loss stays on the device)."""
+    def forward(self, sid: int) -> torch.Tensor:
+        """Cotangent mode (loss_type='modular'): the forward of slot `sid`'s training step -- batch maxima, CNN
+        features and bias offset, temperature fold where the slot has them, then the deformer -- on the step's kernels
+        and arithmetic, so the step recomputes this x_phys bit for bit.  Returns the slot's static x_phys [N, dim]
+        (device; valid until the next forward or step on the slot), ordered before later work on the caller's
+        stream.  Captured as its own CUDA graph under use_cuda_graph."""
+        if not self.cot:
+            raise ValueError("forward(sid) is the cotangent mode of loss_type='modular'")
+        s = self.slots[sid]
+        with torch.cuda.device(self.dev):
+            cur = torch.cuda.current_stream(self.dev)
+            self.stream.wait_stream(cur)      # the caller is done with the previous x_phys
+            if self.use_graph and sid not in self.fwd_graphs:
+                with torch.cuda.stream(self.stream):      # warm-up: first-call attribute setting, communicators
+                    self._issue(s, self.stream.cuda_stream, stage="fwd")
+                self.stream.synchronize()
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g, stream=self.stream):
+                    self._issue(s, torch.cuda.current_stream(self.dev).cuda_stream, stage="fwd")
+                self.fwd_graphs[sid] = g
+            with torch.cuda.stream(self.stream):
+                if self.use_graph:
+                    self.fwd_graphs[sid].replay()
+                else:
+                    self._issue(s, self.stream.cuda_stream, stage="fwd")
+            cur.wait_stream(self.stream)
+        return s.x_phys
+
+    def _load_cotangent(self, s: _Slot, cot):
+        """Copy the caller's cotangent of x_phys into the slot's target segment, on the trainer stream after the
+        caller's current stream (where it was computed)."""
+        if cot is None:
+            raise ValueError("loss_type='modular': step(sid, cotangent=x_grads) needs the cotangent of forward(sid)'s x_phys")
+        if not torch.is_tensor(cot) or cot.dtype != torch.float32 or tuple(cot.shape) != tuple(s.x_phys.shape):
+            raise ValueError(f"the cotangent must be a float32 tensor of shape {tuple(s.x_phys.shape)}, got "
+                             f"{(cot.dtype, tuple(cot.shape)) if torch.is_tensor(cot) else type(cot).__name__}")
+        if cot.device.type == "cpu":
+            if not cot.is_pinned():
+                raise ValueError("a host cotangent must be in pinned memory")
+        elif cot.device != s.x_phys.device:
+            raise ValueError(f"the cotangent is on {cot.device}; the trainer runs on {s.x_phys.device}")
+        with torch.cuda.device(self.dev):
+            self.stream.wait_stream(torch.cuda.current_stream(self.dev))
+            with torch.cuda.stream(self.stream):
+                s.target.copy_(cot, non_blocking=True)
+            if cot.is_cuda:
+                cot.record_stream(self.stream)
+
+    def step(self, sid: int, cotangent: Optional[torch.Tensor] = None):
+        """One training step on the resident batch `sid` (asynchronous; loss stays on the device).
+
+        Cotangent mode (loss_type='modular', no loss_fn): `cotangent` is required, the caller's x_grads for
+        `forward(sid)`'s x_phys -- a float32 [N, dim] tensor on the trainer's device or pinned on the host.  It is
+        copied into the slot, and the step recomputes its forward, back-propagates exactly that cotangent (the
+        gradient of the pseudo-loss sum(x_phys * x_grads), src/run_GNN.py:111-131) and takes the Adam step; the loss
+        it leaves is that pseudo-loss."""
+        if self.cot:
+            self._load_cotangent(self.slots[sid], cotangent)
+        elif cotangent is not None:
+            raise ValueError(f"step(cotangent=...) is the cotangent mode of loss_type='modular'; this trainer trains the "
+                             f"{self.loss_kind!r} loss")
         self._touch_params()
         if self.use_graph:
             if sid not in self.graphs:
@@ -891,13 +999,14 @@ class DeformerTrainer:
 
     def step_from_host(self, sid: int, data) -> float:
         """End-to-end step: host (pinned) inputs -> device, train step, loss back to the host."""
+        self._refuse_cotangent_mode("step_from_host")
         self.load_inputs(sid, data)
         loss = self.step(sid)
         with torch.cuda.stream(self.stream):
             out = loss.to("cpu", non_blocking=False)
         return float(out)
 
-    def train_batch(self, data, ring: int = 3) -> torch.Tensor:
+    def train_batch(self, data, ring: int = 3, grad_fn=None):
         """The body of the reference's training loop on the batch the loader just yielded --
         `optimizer.zero_grad(); out = model(data); loss = loss_fn(out, data.x_phys); loss.backward();
         optimizer.step()` (src/run_GNN.py:99-131, mesh loss) -- as: copy this batch's node inputs to a resident slot
@@ -909,8 +1018,14 @@ class DeformerTrainer:
 
         Slots are found by topology: batches of a dataset on one mesh (`opt['gad_shared_topology']`, the reference's
         `randg` data) share `ring` slots -- the graph is built once, no topology tensor crosses PCIe again; any other
-        batch gets slots keyed on the identity of its `edge_index` (re-used when the same Batch object returns)."""
-        m = self.model
+        batch gets slots keyed on the identity of its `edge_index` (re-used when the same Batch object returns).
+
+        Cotangent mode (loss_type='modular'): `grad_fn(x_phys) -> (loss, x_grads)` is the reference's outside loss
+        (src/run_GNN.py:111-131); the body is `forward(sid)` -> `grad_fn` -> `step(sid, cotangent=x_grads)`, and the
+        return value is grad_fn's loss."""
+        if self.cot != (grad_fn is not None):
+            raise ValueError("train_batch(data, grad_fn) is the cotangent mode of loss_type='modular'" if self.cot else
+                             "grad_fn is taken with loss_type='modular' only")
         if bool(self.opt.get("gad_shared_topology", False)):
             ei = data.edge_index
             key = ("shared", tuple(ei.shape), int(data.x_comp.shape[0]), tuple(getattr(data, "mesh_sizes", ()) or ())[:4])
@@ -941,7 +1056,11 @@ class DeformerTrainer:
             with torch.cuda.stream(self.stream):
                 self.stream.wait_event(s._ready)
         entry["next"] += 1
-        loss = self.step(sid)
+        if self.cot:
+            loss, x_grads = grad_fn(self.forward(sid))
+            self.step(sid, cotangent=x_grads)
+        else:
+            loss = self.step(sid)
         with torch.cuda.stream(self.stream):
             self.slots[sid]._free.record(self.stream)
         return loss
@@ -982,6 +1101,7 @@ class DeformerTrainer:
         `relay=(device, fraction)` (native loop only): that fraction of every batch reaches this GPU through another
         visible GPU -- host -> staging there over ITS path to host memory, then NVLink -- for boxes whose GPUs do not
         have equal host paths (gad_pipeline_run_relay; `dp.balance_host_paths` picks partner and fraction)."""
+        self._refuse_cotangent_mode("run_from_host")
         R = len(self.slots)
         if R < 2:
             raise ValueError("run_from_host needs at least two resident slots (double buffering)")

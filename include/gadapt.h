@@ -302,7 +302,10 @@ typedef struct gad_train_desc {
     const float* tau;    /* [L] */
     int32_t Lw, L, C;
     float inv_temp;
-    /* loss: loss[0] = loss_scale * sum, cotangent = grad_scale * d(sum)/d(out) */
+    /* loss: loss[0] = loss_scale * sum, cotangent = grad_scale * d(sum)/d(out).  loss_kind 0: sum |out - target|,
+     * 1: sum (out - target)^2, 2: `target` holds a cotangent c [N, dim] of x_phys computed outside the model (the
+     * reference's loss_type = modular): sum = <out, c>, the pseudo-loss whose gradient is c, and the cotangent handed
+     * to the backward is grad_scale * c.  Any other kind is an argument error. */
     int32_t loss_kind;
     float grad_scale, loss_scale;
     /* scratch and outputs */
@@ -402,8 +405,10 @@ int gad_conv_bwd(const int32_t* rowptr, const int32_t* col, const int32_t* t_row
                  size_t workspace_bytes, void* stream);
 
 /* ---- loss seam used by the training step (run_GNN.py:80-84,103-106): mean |out - target| or
- * mean (out - target)^2 over N*dim entries; writes the cotangent and a per-call loss scalar. */
-int gad_mesh_loss(const float* out, const float* target, int64_t count, int kind /*0 l1, 1 mse*/,
+ * mean (out - target)^2 over N*dim entries; writes the cotangent and a per-call loss scalar.
+ * kind 2 (loss_type = modular, run_GNN.py:111-131): `target` is a cotangent c of `out` computed outside the model;
+ * loss = sum out * c (not a mean) and g_out = grad_scale * c. */
+int gad_mesh_loss(const float* out, const float* target, int64_t count, int kind /*0 l1, 1 mse, 2 cotangent*/,
                   float grad_scale, float* loss, float* g_out, void* workspace, void* stream);
 size_t gad_mesh_loss_workspace_bytes(int64_t count);
 
