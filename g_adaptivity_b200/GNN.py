@@ -23,6 +23,7 @@ Options the reference supports but this path does not (see SURVEY 8a) raise
 """
 from __future__ import annotations
 
+import copy
 import time
 from typing import List, Optional
 
@@ -242,6 +243,29 @@ class GNN(nn.Module):
             self._graphs._d[skey] = g
         return g
 
+    def _plan_graph(self, data, dev, allow_uniform: bool) -> MeshGraph:
+        """The graph a call runs on (the module and InferenceSession both plan here).  With global CNN features the bias
+        offset is per tile, so tiles hold one mesh each; a mesh too large for the mesh-resident ELL kernels gets the graph
+        a model without global features builds, which runs on the cluster / streaming kernels (they take the offset per
+        mesh), not on CSR tiles."""
+        tile_nodes = None
+        if self.n_glob_used:
+            sizes = self._mesh_sizes(data)
+            if any(n != sizes[0] for n in sizes):
+                raise NotImplementedError("global CNN features need meshes of equal size in a batch")
+            tile_nodes = int(sizes[0])
+        graph = self._graph(data, dev, allow_uniform=allow_uniform, tile_nodes=tile_nodes)
+        if tile_nodes is not None and graph.tile_ptr is not None and not GF.use_ell(graph, self.CE):
+            graph = self._graph(data, dev, allow_uniform=allow_uniform)
+        return graph
+
+    def _softmax_temps(self) -> Optional[torch.Tensor]:
+        """[Lw] learnable temperatures of `softmax_temp_type='learnable_a'` (src/GRAND_plus.py:152-154,328-329), or None."""
+        if self.opt.get("softmax_temp_type") != "learnable_a":
+            return None
+        convs = [self.conv_layers[0]] if self.opt["share_conv"] else list(self.conv_layers)
+        return torch.cat([c.sm_temp_a.reshape(1) for c in convs])
+
     def _folded_weights(self, dev):
         """(M, u) of the current Linear parameters (csrc/weights.cu), cached until a parameter changes:
         keyed on storage and version counter of every parameter plus `_param_epoch`, which the
@@ -280,18 +304,8 @@ class GNN(nn.Module):
         opt = self.opt
         dev = self._device()
         keep_alpha = isinstance(opt.get("show_mesh_evol_plots"), bool) or opt["conv_type"] == "GRAND"
-        keep_alpha = keep_alpha and bool(opt.get("gad_store_alpha", True)) and self.n_glob_used == 0
-        tile_nodes = None
-        if self.n_glob_used:
-            sizes = self._mesh_sizes(data)
-            if any(n != sizes[0] for n in sizes):
-                raise NotImplementedError("global CNN features need meshes of equal size in a batch")
-            tile_nodes = int(sizes[0])              # one mesh per tile: the bias offset is per tile
-        graph = self._graph(data, dev, allow_uniform=not keep_alpha, tile_nodes=tile_nodes)
-        if tile_nodes is not None and graph.tile_ptr is not None and not GF.use_ell(graph, self.CE):
-            # a mesh too large for the mesh-resident ELL kernels: the graph a model without global features builds, which
-            # runs on the cluster / streaming kernels (they take the offset per mesh), not on CSR tiles
-            graph = self._graph(data, dev, allow_uniform=not keep_alpha)
+        keep_alpha = keep_alpha and bool(opt.get("gad_store_alpha", True))
+        graph = self._plan_graph(data, dev, allow_uniform=not keep_alpha)
         x_comp = data.x_comp.to(dev, non_blocking=True)
         f = data.f_tensor.to(dev, non_blocking=True) if opt["gnn_inc_feat_f"] else None
         uu = data.uu_tensor.to(dev, non_blocking=True) if opt["gnn_inc_feat_uu"] else None
@@ -305,12 +319,9 @@ class GNN(nn.Module):
         Mu_in = self._folded_weights(dev)
         aux = {"keep_states": keep_alpha, "Mu_in": Mu_in}
         du = self._global_bias_offsets(data, graph, f, uu, f_scale, uu_scale, dev) if self.n_glob_used else None
-        temp = None
-        if opt.get("softmax_temp_type") == "learnable_a":      # per weight set, src/GRAND_plus.py:152-154,328-329
-            convs = [self.conv_layers[0]] if opt["share_conv"] else list(self.conv_layers)
-            temp = torch.cat([c.sm_temp_a.reshape(1) for c in convs])
-            if du is not None:
-                du = du / temp.reshape(1, -1, 1)                 # the bias offset is a logit term too
+        temp = self._softmax_temps()                            # per weight set
+        if temp is not None and du is not None:
+            du = du / temp.reshape(1, -1, 1)                     # the bias offset is a logit term too
         method = GF.METHODS[opt.get("ode_method", "euler")]
         force_stream = bool(opt.get("gad_force_stream", False))
         if not torch.is_grad_enabled():
@@ -330,12 +341,13 @@ class GNN(nn.Module):
                 method, force_stream, aux, du, temp)
         if keep_alpha and aux.get("states") is not None:
             states, Mu = aux["states"], aux["Mu"]
+            du_a = None if du is None else du.detach()          # the offset the deformer ran with (temperature included)
             L = opt["num_layers"]
             if opt["share_conv"]:
-                self.conv_layers[0]._set_alpha_source(graph, states[L - 1], Mu[0:1])
+                self.conv_layers[0]._set_alpha_source(graph, states[L - 1], Mu[0:1], None if du_a is None else du_a[:, 0])
             else:
                 for l, conv in enumerate(self.conv_layers):
-                    conv._set_alpha_source(graph, states[l], Mu[l:l + 1])
+                    conv._set_alpha_source(graph, states[l], Mu[l:l + 1], None if du_a is None else du_a[:, l])
         object.__setattr__(self, "last_graph", graph)      # plain attributes: nn.Module.__setattr__ costs 2 us each
         # `end_MLmodel` is read by the reference's evaluation code as the end of the model's run time
         # (src/utils_eval.py:193-201): in eval mode the stamp is taken after the stream has drained; the training
@@ -419,23 +431,36 @@ class GNN(nn.Module):
         parameters (hand-written backward, csrc/glob_cnn.cu) and to Wq / Wk (a [n_g x z] matrix product per
         weight set, left to autograd)."""
         opt = self.opt
-        lib_c = GF.fold_scale(self.inv_temp, int(opt["hidden_dim"]))
         sizes = self._mesh_sizes(data)
         B, N1 = len(sizes), int(sizes[0])
         gather = self._cnn_grid_map(data, N1, dev)
+        if opt["gnn_inc_glob_feat_f"] and f is None:
+            f = data.f_tensor.to(dev, non_blocking=True)
+        if opt["gnn_inc_glob_feat_uu"] and uu is None:
+            uu = data.uu_tensor.to(dev, non_blocking=True)
+        Wq, _, Wk, _ = self._weights()
+        return self._bias_offsets(B, N1, gather, f, uu, f_scale, uu_scale, Wq, Wk,
+                                  getattr(self, "global_feature_extractor_cnn_f", None),
+                                  getattr(self, "global_feature_extractor_cnn_uu", None))
+
+    def _bias_offsets(self, B: int, N1: int, gather, f, uu, f_scale, uu_scale, Wq, Wk, cnn_f, cnn_uu) -> torch.Tensor:
+        """du [B, Lw, CE] of `_global_bias_offsets` from device tensors only (no host synchronisation, so that
+        InferenceSession can capture it): B meshes of N1 nodes, the CNNs' inputs f / uu [B * N1], the deformer's
+        gnn_normalize maxima, Wq / Wk [Lw, C, C] and the two CNN modules (None where the option is off)."""
+        opt = self.opt
+        lib_c = GF.fold_scale(self.inv_temp, int(opt["hidden_dim"]))
         feats = []
         if opt["gnn_inc_glob_feat_f"]:
-            src = data.f_tensor.to(dev, non_blocking=True) if f is None else f
+            src = f
             if opt["gnn_inc_feat_f"] and f_scale is not None:
                 src = src / f_scale                      # the reference normalises f in place before the CNN sees it (:231-233)
-            feats.append(self.global_feature_extractor_cnn_f(src.reshape(B, N1), gather=gather))
+            feats.append(cnn_f(src.reshape(B, N1), gather=gather))
         if opt["gnn_inc_glob_feat_uu"]:
-            src = data.uu_tensor.to(dev, non_blocking=True) if uu is None else uu
+            src = uu
             if opt["gnn_inc_feat_uu"] and uu_scale is not None:
                 src = src / uu_scale
-            feats.append(self.global_feature_extractor_cnn_uu(src.reshape(B, N1), gather=gather))
+            feats.append(cnn_uu(src.reshape(B, N1), gather=gather))
         g = torch.cat(feats, dim=1)[:, :self.n_glob_used]                 # what the encoder's truncation keeps
-        Wq, _, Wk, _ = self._weights()
         z0, z1 = self.z_dim, self.z_dim + self.n_glob_used
         M = lib_c * torch.matmul(Wq.transpose(1, 2), Wk)                  # [Lw, C, C], log2-domain scale of the kernels
         du = torch.einsum("bg,lgz->blz", g, M[:, z0:z1, :self.live])      # [B, Lw, live]
@@ -513,32 +538,44 @@ class GNN(nn.Module):
 class InferenceSession:
     """`GNN.forward(data)` in inference mode as one CUDA-graph replay (see GNN.inference_session).
 
-    The output tensor is static: it is overwritten by the next call.  Parameters are read when the
-    session is created (and again by `refresh_weights()`)."""
+    The output tensor is static: it is overwritten by the next call.  Parameters are read when the session is created
+    (and again by `refresh_weights()`): the folded weights, the step sizes, the learnable temperatures and, with global
+    CNN features, the CNN parameters and the Wq / Wk the bias offset is formed from.  What depends on the node inputs
+    -- the gnn_normalize maxima, the CNN features with their abs-max scale, the bias offset -- is recomputed inside the
+    graph on every replay by the module's own arithmetic, so a replay gives the bits of `model(data)` under no_grad."""
 
     def __init__(self, model: GNN, data):
         opt = model.opt
         self.model, self.dev = model, model._device()
         dev = self.dev
-        if opt["gnn_normalize"]:
-            raise NotImplementedError("inference_session with gnn_normalize=True is not implemented")
-        if model.n_glob_used:
-            raise NotImplementedError("inference_session with global CNN features is not implemented (call the module)")
-        if opt.get("softmax_temp_type") == "learnable_a":
-            raise NotImplementedError("inference_session with a learnable temperature is not implemented (call the module)")
-        self.graph = model._graph(data, dev, allow_uniform=True)
+        self.graph = model._plan_graph(data, dev, allow_uniform=True)
         f32 = dict(dtype=torch.float32, device=dev)
         xc = data.x_comp if data.x_comp.dim() == 2 else data.x_comp.unsqueeze(-1)
         self.x_comp = xc.to(**f32).contiguous().clone()
-        self.f = data.f_tensor.to(**f32).contiguous().clone() if opt["gnn_inc_feat_f"] else None
-        self.uu = data.uu_tensor.to(**f32).contiguous().clone() if opt["gnn_inc_feat_uu"] else None
+        glob = model.n_glob_used > 0
+        # f / uu are kept when the deformer or a CNN reads them
+        need_f = opt["gnn_inc_feat_f"] or (glob and opt["gnn_inc_glob_feat_f"])
+        need_uu = opt["gnn_inc_feat_uu"] or (glob and opt["gnn_inc_glob_feat_uu"])
+        self.f = data.f_tensor.to(**f32).contiguous().clone() if need_f else None
+        self.uu = data.uu_tensor.to(**f32).contiguous().clone() if need_uu else None
         self.tau = GF._f32(model._tau(dev).detach().reshape(-1)).clone()
-        self.Mu = model._folded_weights(dev).clone()
+        temp = model._softmax_temps()
+        self.temp = None if temp is None else temp.detach().float().clone()
+        self.Mu = self._read_mu()
+        self.cnns = None
+        if glob:
+            sizes = model._mesh_sizes(data)
+            self.B, self.N1 = len(sizes), int(sizes[0])
+            self.gather = model._cnn_grid_map(data, self.N1, dev)
+            Wq, _, Wk, _ = model._weights()
+            self.Wq, self.Wk = Wq.detach().clone(), Wk.detach().clone()
+            self.cnns = {k: copy.deepcopy(getattr(model, "global_feature_extractor_cnn_" + k)).requires_grad_(False)
+                         for k in ("f", "uu") if opt["gnn_inc_glob_feat_" + k]}
         self.method = GF.METHODS[opt.get("ode_method", "euler")]
         self.force_stream = bool(opt.get("gad_force_stream", False))
         self.stream = torch.cuda.Stream(device=dev)
         self.out = None
-        with torch.cuda.device(dev):
+        with torch.cuda.device(dev), torch.no_grad():
             self.stream.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(self.stream):
                 self._call()                       # warm-up: attribute set-up, allocations
@@ -548,15 +585,45 @@ class InferenceSession:
                 self.out = self._call()
             torch.cuda.current_stream(dev).wait_stream(self.stream)
 
+    def _read_mu(self) -> torch.Tensor:
+        """The folded weights the module's no_grad call runs on: (M, u) / T with a learnable temperature."""
+        Mu = self.model._folded_weights(self.dev)
+        if self.temp is not None:
+            Mu = (Mu / self.temp.reshape(-1, 1)).contiguous()
+        return Mu.clone()
+
     def _call(self):
-        m = self.model
-        return GF.deform_forward_raw(self.graph, self.x_comp, self.f, self.uu, None, None, m.dim, m.CE, self.Mu, self.tau,
-                                     self.method, states=None, force_stream=self.force_stream)
+        m, opt = self.model, self.model.opt
+        f = self.f if opt["gnn_inc_feat_f"] else None
+        uu = self.uu if opt["gnn_inc_feat_uu"] else None
+        f_scale = uu_scale = None
+        if opt["gnn_normalize"]:                   # GNN.forward: signed batch-wide max of the current inputs
+            f_scale = torch.max(f).reshape(1).float() if f is not None else None
+            uu_scale = torch.max(uu).reshape(1).float() if uu is not None else None
+        du = None
+        if self.cnns is not None:
+            du = m._bias_offsets(self.B, self.N1, self.gather, self.f, self.uu, f_scale, uu_scale, self.Wq, self.Wk,
+                                 self.cnns.get("f"), self.cnns.get("uu"))
+            if self.temp is not None:
+                du = du / self.temp.reshape(1, -1, 1)
+        return GF.deform_forward_raw(self.graph, self.x_comp, f, uu, f_scale, uu_scale, m.dim, m.CE, self.Mu, self.tau,
+                                     self.method, states=None, force_stream=self.force_stream, du=du)
 
     def refresh_weights(self):
         """Re-read the model's parameters (on the caller's current stream, like the replays)."""
-        self.Mu.copy_(self.model._folded_weights(self.dev))
-        self.tau.copy_(GF._f32(self.model._tau(self.dev).detach().reshape(-1)))
+        m = self.model
+        with torch.no_grad():
+            if self.temp is not None:
+                self.temp.copy_(m._softmax_temps())
+            self.Mu.copy_(self._read_mu())
+            self.tau.copy_(GF._f32(m._tau(self.dev).detach().reshape(-1)))
+            if self.cnns is not None:
+                Wq, _, Wk, _ = m._weights()
+                self.Wq.copy_(Wq)
+                self.Wk.copy_(Wk)
+                for k, cnn in self.cnns.items():
+                    for mine, theirs in zip(cnn.parameters(), getattr(m, "global_feature_extractor_cnn_" + k).parameters()):
+                        mine.copy_(theirs)
 
     def __call__(self, x_comp=None, f=None, uu=None) -> torch.Tensor:
         """Replay with (optionally) new node inputs; returns the static output tensor [N, dim].  The input copies

@@ -43,10 +43,11 @@ def inv_temperature(opt: dict) -> float:
 
 class _AlphaSource:
     """Everything needed to materialise `stored_alpha` on demand (it costs an [E] write, so it is
-    not produced on every call the way the reference does, `src/GRAND_plus.py:253-256`)."""
+    not produced on every call the way the reference does, `src/GRAND_plus.py:253-256`).  `du` [meshes, CE]: the
+    per-mesh bias offset of the layer's weight set (global CNN features), or None."""
 
-    def __init__(self, graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor):
-        self.graph, self.x, self.Mu = graph, x, Mu
+    def __init__(self, graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor, du: Optional[torch.Tensor] = None):
+        self.graph, self.x, self.Mu, self.du = graph, x, Mu, du
 
 
 class GRAND_plusConv(nn.Module):
@@ -96,9 +97,9 @@ class GRAND_plusConv(nn.Module):
         self.lin_skip.reset_parameters()
 
     # ---- attention read-out -------------------------------------------------------------
-    def _set_alpha_source(self, graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor):
+    def _set_alpha_source(self, graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor, du: Optional[torch.Tensor] = None):
         self.stored_ei = graph.edge_index
-        self._alpha_src = _AlphaSource(graph, x, Mu)
+        self._alpha_src = _AlphaSource(graph, x, Mu, du)
         self._alpha_cache = None
 
     @property
@@ -106,8 +107,7 @@ class GRAND_plusConv(nn.Module):
         """Attention weights [E, 1] of the last call, in `stored_ei` order (`src/GRAND_plus.py:253-256`)."""
         if self._alpha_cache is None and self._alpha_src is not None:
             s = self._alpha_src
-            _, alpha = GF.conv_forward(s.graph, s.x, s.Mu, want_res=False, want_alpha=True)
-            self._alpha_cache = alpha.view(-1, 1)
+            self._alpha_cache = GF.conv_alpha(s.graph, s.x, s.Mu, s.du).view(-1, 1)
         return self._alpha_cache
 
     @stored_alpha.setter

@@ -107,6 +107,7 @@ SIGNATURES = {
     "gad_cluster_occupancy": (_i, [_i, _i, _i, _i, C.POINTER(_i)]),
     "gad_train_step_cluster": (_i, [C.POINTER(TrainDesc), _i, _p]),
     "gad_conv_fwd": (_i, [_p, _p, _p, _i64, _i64, _p, _i, _p, _p, _p, _p]),
+    "gad_conv_alpha_du": (_i, [_p, _p, _p, _i64, _i64, _p, _i, _p, _p, _i, _p, _p]),
     "gad_conv_bwd": (_i, [_p, _p, _p, _p, _i64, _i64, _p, _p, _i, _p, _p, _p, _p, _sz, _p]),
     "gad_mesh_loss": (_i, [_p, _p, _i64, _i, _f, _p, _p, _p, _p]),
     "gad_mesh_loss_workspace_bytes": (_sz, [_i64]),

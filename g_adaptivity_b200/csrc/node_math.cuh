@@ -137,6 +137,22 @@ __device__ __forceinline__ Row<CE> project(const float* __restrict__ Mu, const R
     return p;
 }
 
+// p = M^T y + u with the per-mesh offset of the folded bias (global CNN features, include/gadapt.h): `dui` = the CE
+// floats du[mesh, lw] of the node's mesh, or null.  u + du is rounded before the products are added, as the mesh-resident
+// kernels do when they fold du into their shared copy of u (ell_kernels.cuh: load_mu), so every route rounds alike.
+template <int CE>
+__device__ __forceinline__ Row<CE> project_du(const float* __restrict__ Mu, const float* __restrict__ dui, const Row<CE>& x) {
+    if (!dui) return project<CE>(Mu, x);
+    Row<CE> p;
+#pragma unroll
+    for (int b = 0; b < CE; ++b) p.v[b] = Mu[CE * CE + b] + __ldg(dui + b);
+#pragma unroll
+    for (int a = 0; a < CE; ++a)
+#pragma unroll
+        for (int b = 0; b < CE; ++b) p.v[b] = fmaf(x.v[a], Mu[a * CE + b], p.v[b]);
+    return p;
+}
+
 // y = M t
 template <int CE>
 __device__ __forceinline__ Row<CE> apply_M(const float* __restrict__ Mu, const Row<CE>& t) {
@@ -165,12 +181,14 @@ struct RowCache {
 
 // One F-evaluation at node i.  X: state rows (global or shared), indexed by the entries of `col`
 // (already relative to X).  Returns k_i = o_i - x_i; o_i, the softmax stats and p_i on request.
+// dui: the bias offset of node i's mesh (project_du), or null.
 template <int CE, typename ColT>
 __device__ __forceinline__ Row<CE> node_feval(const float* __restrict__ X, const ColT* __restrict__ col,
                                               int e_begin, int e_end, const Row<CE>& xi,
                                               const float* __restrict__ Mu, Row<CE>* o_out = nullptr,
-                                              SoftmaxStats* st_out = nullptr, Row<CE>* p_out = nullptr) {
-    const Row<CE> p = project<CE>(Mu, xi);
+                                              SoftmaxStats* st_out = nullptr, Row<CE>* p_out = nullptr,
+                                              const float* __restrict__ dui = nullptr) {
+    const Row<CE> p = project_du<CE>(Mu, dui, xi);
     const int deg = e_end - e_begin;
     float m = -CUDART_INF_F, Z = 0.f;
     Row<CE> o = zero_row<CE>();

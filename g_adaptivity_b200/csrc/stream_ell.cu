@@ -130,22 +130,6 @@ __device__ __forceinline__ Row<CE> ldcg_gplus(const float* g, int64_t i, int gdi
     return r;
 }
 
-// p = M^T y + u with the per-mesh offset of the folded bias (global CNN features, include/gadapt.h): `dui` = the CE
-// floats du[mesh, lw] of the node's mesh, or null.  u + du is rounded before the products are added, as the mesh-resident
-// kernels do when they fold du into their shared copy of u (ell_kernels.cuh: load_mu), so every route rounds alike.
-template <int CE>
-__device__ __forceinline__ Row<CE> project_du(const float* __restrict__ Mu, const float* __restrict__ dui, const Row<CE>& x) {
-    if (!dui) return project<CE>(Mu, x);
-    Row<CE> p;
-#pragma unroll
-    for (int b = 0; b < CE; ++b) p.v[b] = Mu[CE * CE + b] + __ldg(dui + b);
-#pragma unroll
-    for (int a = 0; a < CE; ++a)
-#pragma unroll
-        for (int b = 0; b < CE; ++b) p.v[b] = fmaf(x.v[a], Mu[a * CE + b], p.v[b]);
-    return p;
-}
-
 // ---- wide rows from the (row-sorted) CSR / CSC walk arrays ---------------------------------------
 __global__ void __launch_bounds__(TB) k_build_wide(const int32_t* __restrict__ ptr, const int32_t* __restrict__ idx,
                                                    int64_t N, int4* __restrict__ rows, int32_t* __restrict__ bad) {

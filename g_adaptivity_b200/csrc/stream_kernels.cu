@@ -106,6 +106,29 @@ __global__ void __launch_bounds__(TB) k_alpha(const int32_t* __restrict__ rowptr
     }
 }
 
+// k_alpha of a model with global CNN features: du [M, CE] is the bias offset of each mesh for this layer's weight set,
+// node i lies in mesh i / nm.  The logits are those of the deformer kernels that took du (project_du).
+template <int CE>
+__global__ void __launch_bounds__(TB) k_alpha_du(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                                                 const int32_t* __restrict__ eid, int64_t N, const float* __restrict__ x,
+                                                 const float* __restrict__ Mu_g, const float* __restrict__ du, int64_t nm,
+                                                 float* __restrict__ alpha) {
+    __shared__ float Mu[CE * CE + CE];
+    for (int t = threadIdx.x; t < CE * CE + CE; t += blockDim.x) Mu[t] = Mu_g[t];
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const Row<CE> xi = load_row<CE>(x, i);
+    Row<CE> p;
+    SoftmaxStats st;
+    const int b = rowptr[i], e_end = rowptr[i + 1];
+    node_feval<CE, int32_t>(x, col, b, e_end, xi, Mu, nullptr, &st, &p, du + (i / nm) * CE);
+    for (int e = b; e < e_end; ++e) {
+        const Row<CE> xj = load_row<CE>(x, (int64_t)col[e]);
+        alpha[eid[e]] = gexp(dot<CE>(p, xj) - st.m) * st.rZ;
+    }
+}
+
 // ---- backward, destination pass -----------------------------------------------------------
 // grid-stride over nodes so that the number of weight-gradient partials is bounded.
 template <int CE>
@@ -422,6 +445,20 @@ extern "C" int gad_conv_fwd(const int32_t* rowptr, const int32_t* col, const int
         GAD_DISPATCH_CE(CE, k_alpha, <<<nblocks(N), TB, 0, st>>>(rowptr, col, eid, N, x, Mu, alpha));
         GAD_LAUNCH_CHECK();
     }
+    (void)E;
+    return GAD_OK;
+}
+
+extern "C" int gad_conv_alpha_du(const int32_t* rowptr, const int32_t* col, const int32_t* eid, int64_t N, int64_t E,
+                                 const float* x, int CE, const float* Mu, const float* du, int M, float* alpha,
+                                 void* stream) {
+    GAD_CHECK_ARG(rowptr && col && eid && x && Mu && du && alpha && N > 0, "gad_conv_alpha_du: bad arguments");
+    GAD_CHECK_ARG(M > 0 && N % M == 0, "gad_conv_alpha_du: du needs M > 0 meshes of equal size (N=%lld, M=%d)",
+                  (long long)N, M);
+    cudaStream_t st = as_stream(stream);
+    const int64_t nm = N / M;
+    GAD_DISPATCH_CE(CE, k_alpha_du, <<<nblocks(N), TB, 0, st>>>(rowptr, col, eid, N, x, Mu, du, nm, alpha));
+    GAD_LAUNCH_CHECK();
     (void)E;
     return GAD_OK;
 }

@@ -404,6 +404,25 @@ def conv_forward(graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor, want_res: 
     return res, alpha
 
 
+def conv_alpha(graph: MeshGraph, x: torch.Tensor, Mu: torch.Tensor, du: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Attention weights alpha [E] of one layer in filtered edge-list order.  `du` [meshes, CE] (or None): the per-mesh
+    bias offset of this layer's weight set that the deformer ran with (global CNN features, meshes of equal size)."""
+    if du is None:
+        return conv_forward(graph, x, Mu, want_res=False, want_alpha=True)[1]
+    _need_cuda(x, Mu, du)
+    lib = _lib.load()
+    N, CE = x.shape
+    du = _f32(du)
+    if graph.mesh_sizes is None or du.shape != (len(graph.mesh_sizes), CE):
+        raise ValueError(f"du must be [meshes, {CE}], got {tuple(du.shape)}")
+    alpha = torch.empty(graph.E, dtype=torch.float32, device=x.device)
+    with _on_device(x.device):
+        _lib.check(lib.gad_conv_alpha_du(_lib.ptr(graph.rowptr), _lib.ptr(graph.col), _lib.ptr(graph.eid), N, graph.E,
+                                         _lib.ptr(x), CE, _lib.ptr(Mu), _lib.ptr(du), int(du.shape[0]), _lib.ptr(alpha),
+                                         _stream(x)), "gad_conv_alpha_du")
+    return alpha
+
+
 def conv_backward(graph: MeshGraph, x: torch.Tensor, g_res: torch.Tensor, Mu: torch.Tensor):
     lib = _lib.load()
     N, CE = x.shape

@@ -399,6 +399,11 @@ int gad_deform_fwd_cluster(const void* crows_in, const int32_t* mesh_ptr, int M,
  */
 int gad_conv_fwd(const int32_t* rowptr, const int32_t* col, const int32_t* eid, int64_t N, int64_t E,
                  const float* x, int CE, const float* Mu, float* res, float* alpha, void* stream);
+/* alpha [E] of one layer of a model with global CNN features: the logits take the per-mesh bias offset the deformer
+ * kernels took, u + du[m] for node i of mesh m = i / (N / M).  du [M, CE]: the offset of this layer's weight set
+ * (du[:, lw] of the deformer's [M, Lw, CE]); the M meshes are of equal size. */
+int gad_conv_alpha_du(const int32_t* rowptr, const int32_t* col, const int32_t* eid, int64_t N, int64_t E,
+                      const float* x, int CE, const float* Mu, const float* du, int M, float* alpha, void* stream);
 int gad_conv_bwd(const int32_t* rowptr, const int32_t* col, const int32_t* t_rowptr,
                  const int32_t* t_dst, int64_t N, int64_t E, const float* x, const float* g_res,
                  int CE, const float* Mu, float* gMu, float* g_x, void* workspace,
